@@ -24,7 +24,8 @@ per-sketch reduction, identity/p-value, and the rows mash would print (shared > 
   value  : device-resident (packed query already in HBM), whole job, CUDA-event timed, max over ranks.
   e2e    : same screen through the public API from FASTA TEXT in pinned host memory: host->device
            copies, FASTA parsing + 2-bit packing, kernels and the result copy inside the timed region.
-One JSON line on stdout (rank 0).
+One JSON line on stdout (rank 0).  --dump-outputs DIR also writes the last timed step's result columns
+as DIR/*.npy; the inputs are generated from fixed seeds, so two builds can be compared output for output.
 """
 from __future__ import annotations
 
@@ -71,7 +72,15 @@ def parse_args():
     ap.add_argument("--s", type=int, default=1000)
     ap.add_argument("--clusters", type=int, default=0,
                     help="config 4: make this many of the real genomes 1-5 %% diverged copies of the others")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the result of the last timed step as DIR/<column>.npy (float64), so that two builds "
+                         "can be compared output for output on the same seeded inputs")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the CUDA arm's result")
+    return args
 
 
 def pick_workload(args) -> str:
@@ -148,6 +157,25 @@ class ClockSampler:
         if not sm:
             return {"sm_mhz": None, "sm_max_mhz": None, "reasons": [], "samples": 0}
         return {"sm_mhz": statistics.median(sm), "sm_max_mhz": max(mx), "reasons": sorted(reasons), "samples": len(sm)}
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, res) -> None:
+    """The columns a caller of the timed step receives (ScreenHits: the references with shared > 0,
+    ascending), as float64 .npy files; every count is below 2^53, so the conversion is exact.  Above
+    DUMP_LIMIT_BYTES in all, a fixed seeded sample of the rows is written instead."""
+    import numpy as np
+    cols = {"ref": res.ref, "shared": res.shared, "median": res.median, "identity": res.identity, "pvalue": res.pvalue}
+    rows = np.arange(len(res.ref))
+    max_rows = (DUMP_LIMIT_BYTES - 4096) // (8 * len(cols))     # 4 KB: set_size and the .npy headers
+    if len(rows) > max_rows:
+        rows = np.sort(np.random.default_rng(0).choice(len(rows), max_rows, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, col in cols.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(col, dtype=np.float64)[rows])
+    np.save(os.path.join(out_dir, "set_size.npy"), np.array([res.set_size], dtype=np.float64))
 
 
 def n_host_threads() -> int:
@@ -411,6 +439,8 @@ def run_b200(args):
 
     total_bases = all_sum(wl.n_bases)
     ms, wall, stats, res, clocks = timed(step_resident, args.steps, args.warmup, sample_clocks=True)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, res)
     value = args.steps * total_bases / (ms * 1e-3) / 1e6
     st = stats[-1]
     launches = sum(s["n_launches"] for s in stats)

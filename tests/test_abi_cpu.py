@@ -36,21 +36,33 @@ def test_library_exports_every_declared_symbol():
 
 
 def test_no_gpu_means_error_not_fallback():
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
-    lib = _abi.load()
-    assert lib.hs_init(0) == -2  # HS_ENODEV
-    assert b"no CPU fallback" in lib.hs_last_error()
-    h = C.c_void_p()
-    off = np.array([0, 1], np.uint64); hh = np.array([5], np.uint64)
-    rc = lib.hs_db_from_arrays(21, 1000, 42, 1, off.ctypes.data_as(_abi.u64p), hh.ctypes.data_as(_abi.u64p), None,
-                               C.byref(h))
-    assert rc == -2 and not h.value
-    with pytest.raises(_abi.HsError):
-        hs.hash_packed(21, 42, np.zeros(256, np.uint64), np.zeros(256, np.uint32), 100)
-    with pytest.raises(_abi.HsError):
-        hs.Database.from_arrays(21, 1000, 42, off, hh)
+    """Run in a child process that sees no device (CUDA_VISIBLE_DEVICES empty), so that the check also
+    holds on a box with a B200."""
+    import subprocess
+    code = r'''
+import ctypes as C, sys
+sys.path.insert(0, %r)
+import numpy as np
+import pytest
+from hymet_b200 import _abi
+from hymet_b200 import screen as hs
+lib = _abi.load()
+assert lib.hs_init(0) == -2  # HS_ENODEV
+assert b"no CPU fallback" in lib.hs_last_error()
+h = C.c_void_p()
+off = np.array([0, 1], np.uint64); hh = np.array([5], np.uint64)
+rc = lib.hs_db_from_arrays(21, 1000, 42, 1, off.ctypes.data_as(_abi.u64p), hh.ctypes.data_as(_abi.u64p), None,
+                           C.byref(h))
+assert rc == -2 and not h.value
+with pytest.raises(_abi.HsError):
+    hs.hash_packed(21, 42, np.zeros(256, np.uint64), np.zeros(256, np.uint32), 100)
+with pytest.raises(_abi.HsError):
+    hs.Database.from_arrays(21, 1000, 42, off, hh)
+print("ok")
+''' % ROOT
+    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=300,
+                       env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
+    assert r.returncode == 0 and r.stdout.strip() == "ok", (r.returncode, r.stdout, r.stderr[-2000:])
 
 
 def test_host_packer_layout():

@@ -19,6 +19,7 @@ from hymet_b200 import synth
 from hymet_b200.tsv import screen_lines
 from oracle import py_micro_oracle as po
 from tests import _oracle as orc
+from tests.test_stage_cpu import reference_mash_sh
 
 pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -415,19 +416,6 @@ def test_cli_tsv_byte_identical_to_oracle_cli(tmp_path):
     r = subprocess.run([sys.executable, os.path.join(ROOT, "bin", "mash"), "screen", dbp, str(tmp_path / "none.fna")],
                        capture_output=True)
     assert r.returncode == 1 and b"ERROR" in r.stderr and r.stdout == b""
-
-
-def reference_mash_sh(tmp_path, golden_dir):
-    """The reference's scripts/mash.sh, byte for byte, from the compressed fixture."""
-    import base64
-    import gzip
-    import hashlib
-    fx = json.load(open(os.path.join(golden_dir, "mash_sh_fixture.json")))
-    raw = gzip.decompress(base64.b64decode(fx["gzip_base64"]))
-    assert hashlib.sha256(raw).hexdigest() == fx["sha256"]
-    sh = tmp_path / "mash.sh"
-    sh.write_bytes(raw)
-    return str(sh)
 
 
 def run_mash_sh(tmp_path, script, mash_exe, tag, indir, dbp, thr):
