@@ -132,9 +132,7 @@ def load(rebuild: bool = False) -> C.CDLL:
     if _lib is not None and not rebuild:
         return _lib
     path = _build.LIB
-    if os.environ.get("HYMET_SCREEN_LIB"):        # kernel experiments: an alternative build of the same sources
-        path = os.environ["HYMET_SCREEN_LIB"]
-    elif rebuild or not os.path.exists(path) or (os.path.exists(_build.CSRC) and _build.stale()
+    if rebuild or not os.path.exists(path) or (os.path.exists(_build.CSRC) and _build.stale()
                                                 and os.path.exists(os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc"))):
         path = _build.build(force=rebuild)
     if not os.path.exists(path):

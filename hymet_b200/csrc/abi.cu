@@ -130,7 +130,6 @@ struct Ingest {
     struct Slot { uint8_t *raw = nullptr, *codes = nullptr; size_t cap = 0; cudaEvent_t done = nullptr, copied = nullptr; };
     Slot slots[kSlots];
     int next = 0;
-    int n_slots = kSlots;   // how many of them rotate (option "ingest_slots")
     FaScratch sc{};
     size_t tile_cap = 0;
     std::vector<unsigned long long *> counter_blocks;   // per-chunk position counters (512 per block)
@@ -172,7 +171,7 @@ struct Ingest {
     int slot_for(size_t bytes, Slot **out)
     {
         Slot &sl = slots[next];
-        next = (next + 1) % n_slots;
+        next = (next + 1) % kSlots;
         CU(cudaEventSynchronize(sl.done));  // throttle: at most kSlots chunks of raw text in flight
         if (sl.cap < bytes) {
             cudaFree(sl.raw); cudaFree(sl.codes);
@@ -344,11 +343,9 @@ struct hs_screen {
     cudaStream_t copy_stream = nullptr;      // H2D of query chunks overlaps the kernels of earlier chunks
     std::vector<cudaEvent_t> copy_evs;
     size_t copy_ev_used = 0;
-    uint64_t piece_positions = (uint64_t)32 << 20;  // packed host feeds are uploaded + launched in pieces
     Ingest ingest;
     int ingest_mode = 2;   // 0 = host packer only, 1 = device parser only, 2 = both compete for chunks (pinned text)
     uint64_t text_chunk = (uint64_t)256 << 20;   // gzip / stdin input: bytes inflated per hand-over to the packers
-    int ingest_batch = 0;  // spans per device-ingest submission (0 = 2 next to packer threads, 4 alone)
     FileRing ring;
     // plain FASTA files: nominal bytes per reader block and reader threads.  Pinning the ring costs
     // ~0.5 ms per MB once per handle (measured), which a one-shot `mash screen` pays in full: the
@@ -395,7 +392,6 @@ struct hs_screen {
     std::vector<Staging> staging;
     std::mutex mu;  // serialises arena + launches when packer threads feed concurrently
     bool filter = true;
-    int batch_bloom = 1, coop_probe = 1;
     uint64_t chunk_text = (uint64_t)16 << 20;
     hs_stats_t st;
     std::vector<std::pair<cudaEvent_t, cudaEvent_t>> ev_pool;
@@ -502,15 +498,10 @@ int db_build(hs_db *db, const uint64_t *hashes)
     db->dense_max = db->max_key;
     {
         // Second tier: worth it when the range test lets more than ~1 % of uniformly distributed query
-        // hashes through.  HYMET_SCREEN_BLOOM=0/1 overrides.
+        // hashes through.
         const double pass = (double)db->max_key / 18446744073709551615.0;
-        FilterPlan plan = plan_filter(db, hashes);
-        bool want = pass > 0.01 && plan.bloom;
-        if (const char *e = getenv("HYMET_SCREEN_BLOOM")) {
-            want = atoi(e) != 0 && E > 0;
-            if (want && !plan.bloom) plan = FilterPlan{0, std::min<uint64_t>((uint64_t)1 << 24, std::max<uint64_t>(4096, E)), (double)E, true};
-        }
-        if (want && E) {
+        const FilterPlan plan = plan_filter(db, hashes);
+        if (pass > 0.01 && plan.bloom && E) {
             uint64_t words = 4096;
             while (words < plan.words) words <<= 1;
             CU(cudaMalloc((void **)&db->d_bloom, words * 4));
@@ -564,11 +555,10 @@ int launch_chunk(hs_screen *s, const Chunk &c, bool count, bool mix, uint64_t ti
     a.tile_begin = (uint32_t)tile_begin; a.n_tiles = (uint32_t)tile_end;
     a.do_count = count; a.do_filter = s->filter; a.do_mix = mix;
     a.tab = s->db->view(); a.counts = s->d_counts;
-    a.batch_bloom = s->batch_bloom;
     // the range test removes probes only when the keys are confined to a sliver of the hash range; a db
     // whose keys cover a quarter of it or more and has no Bloom tier probes for most k-mers: that is
     // the warp-cooperative kernel's job, as is "filter" = 0
-    a.probe_all = s->coop_probe && (!s->filter || (!s->db->d_bloom && s->db->max_key >= ((uint64_t)1 << 62)));
+    a.probe_all = !s->filter || (!s->db->d_bloom && s->db->max_key >= ((uint64_t)1 << 62));
     if (count && s->sparse_enabled) a.sparse = SparseView{s->d_touched, s->touched_cap, s->d_sparse};
     const uint64_t launch_positions = (tile_end - tile_begin) * kTileWords * 32;
     a.mix = s->mix.view(mix ? s->mix.launch_cap(launch_positions) : ~0ull);
@@ -816,7 +806,6 @@ HS_API int hs_init(int device)
     g_device = device;
     g_sm = p.multiProcessorCount;
     g_debug_timing = getenv("HYMET_SCREEN_DEBUG_TIMING") != nullptr;
-    if (const char *e = getenv("HYMET_PACK_STREAMING")) set_pack_streaming(atoi(e) != 0);
     return HS_OK;
 }
 
@@ -1001,7 +990,6 @@ HS_API int hs_screen_new(hs_db *db, hs_screen **out)
     s->pair_cap = (uint32_t)std::min<uint64_t>(E, std::max<uint64_t>((uint64_t)1 << 23, E / 4));
     if (const char *e = getenv("HYMET_SCREEN_TOUCHED_CAP")) s->touched_cap = (uint32_t)std::max(1ll, atoll(e));   // tests: force the fallbacks
     if (const char *e = getenv("HYMET_SCREEN_PAIR_CAP")) s->pair_cap = (uint32_t)std::max(1ll, atoll(e));
-    if (const char *e = getenv("HYMET_SCREEN_SPARSE")) s->sparse_enabled = atoi(e) != 0;
     if (const char *e = getenv("HYMET_SCREEN_FORCE_UNSETTLED")) s->force_unsettled = atoi(e);
     CUB(cudaMalloc((void **)&s->d_sparse, sizeof(SparseState)));
     CUB(cudaMemsetAsync(s->d_sparse, 0, sizeof(SparseState), s->stream));
@@ -1049,18 +1037,12 @@ HS_API int hs_screen_set_option(hs_screen *s, const char *key, int64_t value)
     if (!s || !key) return fail(HS_EINVAL, "null argument");
     if (!strcmp(key, "filter")) s->filter = value != 0;
     else if (!strcmp(key, "chunk_bases")) s->chunk_text = value > 4096 ? (uint64_t)value : 4096;
-    else if (!strcmp(key, "piece_bases")) s->piece_positions = value > 8192 ? (uint64_t)value : 8192;
     else if (!strcmp(key, "ingest")) s->ingest_mode = (int)value;
-    else if (!strcmp(key, "ingest_slots")) s->ingest.n_slots = value < 1 ? 1 : (value > Ingest::kSlots ? Ingest::kSlots : (int)value);
-    else if (!strcmp(key, "ingest_batch")) s->ingest_batch = value < 1 ? 1 : (value > 8 ? 8 : (int)value);
     else if (!strcmp(key, "text_chunk_bytes")) s->text_chunk = value > 4096 ? (uint64_t)value : 4096;
     else if (!strcmp(key, "file_block_bytes")) s->file_block = value > 65536 ? (uint64_t)value : 65536;
     else if (!strcmp(key, "file_mode")) s->file_mode = value < 0 ? -1 : (value ? 1 : 0);
     else if (!strcmp(key, "file_readers")) s->file_readers = value < 1 ? 1 : (value > 16 ? 16 : (int)value);
-    else if (!strcmp(key, "batch_bloom")) s->batch_bloom = value != 0;
-    else if (!strcmp(key, "coop_probe")) s->coop_probe = value != 0;
     else if (!strcmp(key, "sparse")) { s->sparse_enabled = value != 0; s->touched_valid = false; }
-    else if (!strcmp(key, "keep_query")) { if (!value) return fail(HS_EUNSUPPORTED, "keep_query=0 is not implemented: chunks stay resident until reset"); }
     else return fail(HS_EINVAL, std::string("unknown option ") + key);
     return HS_OK;
 }
@@ -1081,6 +1063,9 @@ HS_API int hs_pack_text(const char *text, size_t n, uint64_t *seq2, uint32_t *in
 
 namespace {
 
+constexpr uint64_t kPieceWords = ((uint64_t)32 << 20) / 32;   // 32 Mi positions per piece, a whole number of tiles
+static_assert(kPieceWords % kTileWords == 0, "pieces must be whole tiles");
+
 // copy a packed host chunk into the arena (padding flagged invalid) and launch it, in
 // pieces: the copy of piece i+1 (copy stream) overlaps the kernel of piece i (compute stream)
 int feed_host_chunk(hs_screen *s, const uint64_t *seq, const uint32_t *inv, uint64_t n_bases, cudaEvent_t done_ev)
@@ -1093,9 +1078,8 @@ int feed_host_chunk(hs_screen *s, const uint64_t *seq, const uint32_t *inv, uint
     Chunk c{(const uint64_t *)dseq, (const uint32_t *)dinv, n_bases};
     s->chunks.push_back(c);
     s->st.h2d_bytes += words * 12;
-    const uint64_t piece_words = std::max<uint64_t>(kTileWords, s->piece_positions / 32 / kTileWords * kTileWords);
-    for (uint64_t w0 = 0; w0 < alloc; w0 += piece_words) {
-        const uint64_t w1 = std::min(alloc, w0 + piece_words);      // tile aligned
+    for (uint64_t w0 = 0; w0 < alloc; w0 += kPieceWords) {
+        const uint64_t w1 = std::min(alloc, w0 + kPieceWords);      // tile aligned
         const uint64_t cw1 = std::min(words, w1);                   // words that exist in the host buffer
         if (cw1 > w0) {
             CU(cudaMemcpyAsync((char *)dseq + w0 * 8, seq + w0, (cw1 - w0) * 8, cudaMemcpyHostToDevice, s->copy_stream));
@@ -1273,7 +1257,7 @@ int feed_text_impl(hs_screen *s, const char *text, size_t n, int threads)
         cudaSetDevice(s->db->device);
         // consecutive spans are contiguous text: take a few at a time so that the parser and
         // stream kernels run on >= 48 MB launches (fewer, fuller waves; fewer host wake-ups)
-        const size_t batch = s->ingest_batch ? (size_t)s->ingest_batch : (threads > 0 ? 2 : 4);
+        const size_t batch = threads > 0 ? 2 : 4;
         for (;;) {
             if (threads > 0) {
                 // The mirror image of the packers' rule: a batch taken now completes after everything already
@@ -1284,7 +1268,7 @@ int feed_text_impl(hs_screen *s, const char *text, size_t n, int threads)
                 const size_t nx = next.load();
                 if (nx >= spans.size()) break;
                 int busy = 0;
-                for (int q = 0; q < s->ingest.n_slots; q++)
+                for (int q = 0; q < Ingest::kSlots; q++)
                     if (s->ingest.slots[q].done && cudaEventQuery(s->ingest.slots[q].done) == cudaErrorNotReady) busy++;
                 cudaGetLastError();
                 const int alive = packers_alive.load();

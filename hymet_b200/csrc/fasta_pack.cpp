@@ -29,7 +29,6 @@ struct Lut {
     }
 };
 const Lut kLut;
-bool g_pack_streaming = true;   // measured on the 16-vCPU B200 host: e2e 13.6 -> 12.7 ms per Gbp (HYMET_PACK_STREAMING=0 turns it off)
 
 // Left-aligned accumulator: base i of the pending word sits at bits [62-2i, 63-2i],
 // its invalid flag at bit (31-i).
@@ -219,7 +218,6 @@ HS_AVX512_TARGET size_t run_avx512(Writer &wr, const unsigned char *p, size_t n,
     size_t off = 0, fill = 0;
     uint64_t kept = 0;
     bool stop = false, aligned = wr.cnt == 0;
-    const bool nt = g_pack_streaming;
     while (!stop && off + 64 <= n) {
         while (off + 64 <= n && fill <= kScratch) {
             _mm_prefetch((const char *)(p + off + 4096), _MM_HINT_T0);   // measured: 4.5 -> 6.4 GB/s per thread out of cache
@@ -246,17 +244,13 @@ HS_AVX512_TARGET size_t run_avx512(Writer &wr, const unsigned char *p, size_t n,
             __m128i codes;
             uint64_t bad;
             convert64(_mm512_permutexvar_epi8(rev, _mm512_loadu_si512((const void *)(tmp + q))), codes, bad);
-            if (nt) {
-                // staging buffers are written once and read by the DMA engine only: streaming stores skip the
-                // read-for-ownership of lines the CPU never looks at again (option, see set_pack_streaming)
-                _mm_stream_si64((long long *)(seq + words), _mm_extract_epi64(codes, 0));
-                _mm_stream_si64((long long *)(seq + words + 1), _mm_extract_epi64(codes, 1));
-                _mm_stream_si32((int *)(inv + words), (int)(uint32_t)bad);
-                _mm_stream_si32((int *)(inv + words + 1), (int)(uint32_t)(bad >> 32));
-            } else {
-                _mm_storeu_si128((__m128i *)(seq + words), codes);
-                memcpy(inv + words, &bad, 8);
-            }
+            // staging buffers are written once and read by the DMA engine only: streaming stores skip the
+            // read-for-ownership of lines the CPU never looks at again (measured on the 16-vCPU B200 host:
+            // e2e 13.6 -> 12.7 ms per Gbp)
+            _mm_stream_si64((long long *)(seq + words), _mm_extract_epi64(codes, 0));
+            _mm_stream_si64((long long *)(seq + words + 1), _mm_extract_epi64(codes, 1));
+            _mm_stream_si32((int *)(inv + words), (int)(uint32_t)bad);
+            _mm_stream_si32((int *)(inv + words + 1), (int)(uint32_t)(bad >> 32));
         }
         wr.w += words;
         kept += q;
@@ -273,7 +267,7 @@ HS_AVX512_TARGET size_t run_avx512(Writer &wr, const unsigned char *p, size_t n,
         wr.positions -= fill;
         kept += fill;
     }
-    if (nt) _mm_sfence();
+    _mm_sfence();
     wr.positions += kept;
     kept_out = kept;
     return off;
@@ -285,7 +279,6 @@ int g_pack_level = -1;   // -1: best the host has; 0 scalar, 1 AVX2 lines, 2 AVX
 }  // namespace
 
 void set_pack_level(int level) { g_pack_level = level; }
-void set_pack_streaming(bool on) { g_pack_streaming = on; }
 
 int pack_level()
 {

@@ -31,8 +31,6 @@ uint64_t pack_text_span(const char *text, size_t n, uint64_t *seq, uint32_t *inv
 // compare them bit for bit.
 void set_pack_level(int level);
 int pack_level();
-// AVX-512 path: write the packed words with non-temporal stores (output that only a DMA engine reads next)
-void set_pack_streaming(bool on);
 
 // Offsets of the header lines as pack_text_span sees them ('>' / '@' at a line start outside a FASTQ
 // quality block), thinned to >= min_gap bytes apart.  The text may be cut in front of any of them.

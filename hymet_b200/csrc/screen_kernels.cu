@@ -53,9 +53,7 @@ __device__ __forceinline__ void mbar_arrive(uint64_t *bar)
 {
     asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
-#ifndef HS_WAIT_SLEEP
-#define HS_WAIT_SLEEP 100   // ns between tries of a warp that is ahead of its CTA (0: spin)
-#endif
+constexpr unsigned kWaitSleepNs = 100;   // between tries of a warp that is ahead of its CTA
 __device__ __forceinline__ bool mbar_try(uint64_t *bar, uint32_t phase)
 {
     uint32_t ok;
@@ -76,9 +74,7 @@ __device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t phase)
     // with a clock read per trip was 3.9 % of all issued warp instructions of the kernel (ncu r02, 13 trips per
     // wait), taken from the issue slots of the very warps it was waiting for.
     for (uint32_t spins = 1;; spins++) {
-#if HS_WAIT_SLEEP
-        __nanosleep(HS_WAIT_SLEEP);
-#endif
+        __nanosleep(kWaitSleepNs);
         if (mbar_try(bar, phase)) return;
         // a tile that never lands means a broken launch contract: fail loudly, never hang the GPU
         if (spins > (1u << 24)) __trap();
@@ -374,39 +370,21 @@ struct SmemPremul {
     }
 };
 
-#ifndef HS_ILP
-#define HS_ILP 4
-#endif
-#ifndef HS_MIN_CTAS
-#define HS_MIN_CTAS 4   // 48 KB of shared memory per CTA
-#endif
-#ifndef HS_BLOOM_LD
-#define HS_BLOOM_LD __ldcg    // the Bloom tier's filter words are read through L2 only: with them out of L1 the
-                              // tail-term table pays in that instantiation too (tiny-genome DB: 6.30 -> 6.18 ms; with __ldg 6.50)
-#endif
-#ifndef HS_BLOOM_HI_GATE
-#define HS_BLOOM_HI_GATE 1
-#endif
-#ifndef HS_TAIL_TABLE
-#define HS_TAIL_TABLE 1
-#endif
-// compile-time k with a 1..5 letter tail (k = 21): the tail term comes from its own table
-#ifndef HS_TAIL_MODES
-#define HS_TAIL_MODES 0x7   // bit m: instantiation MODE m uses the table (it takes 8 KB from the L1 of every CTA: not the
-                            // probe-everything kernel, which lives on L1/L2 traffic)
-#endif
+constexpr int kMinCtas = 4;   // 48 KB of shared memory per CTA
+// compile-time k with a 1..5 letter tail (k = 21): the tail term comes from its own table.  It takes 8 KB
+// from the L1 of every CTA, so the probe-everything kernel (MODE 3), which lives on L1/L2 traffic, goes without
 __host__ __device__ constexpr bool stream_tail_table(int kt, int mode)
 {
-    return HS_TAIL_TABLE && ((HS_TAIL_MODES >> mode) & 1) && kt > 0 && (kt & 15) >= 1 && (kt & 15) <= 5;
+    return mode != 3 && kt > 0 && (kt & 15) >= 1 && (kt & 15) <= 5;
 }
-constexpr int kIlp = HS_ILP;   // k-mers hashed side by side per thread (measured, ms per Gbp: 1: 5.33, 2: 5.02, 4: 4.83, 8: 6.47)
+constexpr int kIlp = 4;   // k-mers hashed side by side per thread (measured, ms per Gbp: 1: 5.33, 2: 5.02, 4: 4.83, 8: 6.47)
 
 // MODE: 0 = screen, 1 = K1 parity (emit every hash), 2 = screen with the Bloom reads of a group of
 // kIlp k-mers issued together (databases with keys above the dense range), 3 = screen that probes for
 // (nearly) every k-mer: the warp looks its hashes up cooperatively (coop_probe), control flow stays
 // warp-uniform and the CTA may use twice the registers (the kernel waits on HBM, not on issue slots)
 template <int KT, int MODE>
-__global__ void __launch_bounds__(kCtaThreads, MODE == 3 ? 3 : HS_MIN_CTAS) k_stream(const StreamArgs a)
+__global__ void __launch_bounds__(kCtaThreads, MODE == 3 ? 3 : kMinCtas) k_stream(const StreamArgs a)
 {
     constexpr bool EMIT = MODE == 1, BLOOMB = MODE == 2, COOP = MODE == 3;
     constexpr bool kTailTab = stream_tail_table(KT, MODE);
@@ -548,10 +526,10 @@ __global__ void __launch_bounds__(kCtaThreads, MODE == 3 ? 3 : HS_MIN_CTAS) k_st
                 mix_insert(a.mix, mix_set, h);
             }
             if (a.do_count && (!a.do_filter || h <= a.tab.max_key)) {
-                if (a.do_filter && a.tab.bloom && h > a.tab.dense_max) {  // second tier (exact: no false negatives)
+                // second tier (exact: no false negatives); only MODE 2 runs with one, its words read in word()
+                if (BLOOMB && a.do_filter && a.tab.bloom && h > a.tab.dense_max) {
                     uint32_t bw, bb;
                     bloom_slot(h, a.tab.bloom_mask, use64, bw, bb);
-                    if (!BLOOMB) bloom_word = __ldg(a.tab.bloom + bw);
                     if ((bloom_word & bb) != bb) return;
                 }
                 n_probe++;
@@ -594,12 +572,10 @@ __global__ void __launch_bounds__(kCtaThreads, MODE == 3 ? 3 : HS_MIN_CTAS) k_st
                             uint32_t bw;
                             bloom_slot(h[u], a.tab.bloom_mask, use64, bw, bbits[u]);
                             pre[u] = 0u;                               // fails the test below: bbits is never 0
-                            // (high words only: a superset of h <= max_key, and the word index is masked into range)
-#if HS_BLOOM_HI_GATE
-                            if ((uint32_t)(h[u] >> 32) <= max_hi) pre[u] = HS_BLOOM_LD(a.tab.bloom + bw);
-#else
-                            if (h[u] <= a.tab.max_key) pre[u] = HS_BLOOM_LD(a.tab.bloom + bw);
-#endif
+                            // (high words only: a superset of h <= max_key, and the word index is masked into range).
+                            // Read through L2 only: with the filter words out of L1 the tail-term table pays in
+                            // this instantiation too (tiny-genome DB: 6.30 -> 6.18 ms; with __ldg 6.50)
+                            if ((uint32_t)(h[u] >> 32) <= max_hi) pre[u] = __ldcg(a.tab.bloom + bw);
                         }
                     }
                     if (COOP) {
@@ -644,11 +620,7 @@ __global__ void __launch_bounds__(kCtaThreads, MODE == 3 ? 3 : HS_MIN_CTAS) k_st
                         for (int u = 0; u < kIlp; u++) {
                             const int j = half * 16 + q + u;
                             // (high word of the low gate: a superset; the sink repeats every test exactly)
-#if HS_BLOOM_HI_GATE
                             const bool enter = (uint32_t)(h[u] >> 32) <= lowgate_hi || (pre[u] & bbits[u]) == bbits[u];
-#else
-                            const bool enter = h[u] <= lowgate || (pre[u] & bbits[u]) == bbits[u];
-#endif
                             if (enter && (!decltype(check)::value || ((ok >> (31 - j)) & 1u))) sink(j, h[u], pre[u]);
                         }
                     } else {
@@ -729,7 +701,7 @@ cudaError_t launch_stream(const StreamArgs &a, int sm_count, cudaStream_t st)
         default: return launch_stream_t<0, 3>(a, sm_count, st);
         }
     }
-    if (a.batch_bloom && a.do_count && a.do_filter && a.tab.bloom) {
+    if (a.do_count && a.do_filter && a.tab.bloom) {
         switch (a.k) {
         case 21: return launch_stream_t<21, 2>(a, sm_count, st);
         case 31: return launch_stream_t<31, 2>(a, sm_count, st);

@@ -95,7 +95,6 @@ struct StreamArgs {
     unsigned long long *stats;  // ST_COUNT slots
     uint64_t *emit_hash;    // optional: per position hash (K1 parity), n_bases entries
     uint8_t *emit_valid;
-    int batch_bloom;        // use the instantiation that issues the Bloom reads of a group of k-mers together
     int probe_all;          // (nearly) every k-mer probes: use the warp-cooperative instantiation
 };
 

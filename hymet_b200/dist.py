@@ -177,9 +177,6 @@ class DistributedScreen:
         if self.exchange_mode == "sparse":      # forced: room for every entry, never falls back
             self.cap = int(max(4096, db.n_entries))
         self._rec = self._all = self._mix = self._mix_all = None
-        # one host synchronisation per screen (hs_screen_flush_async): the host enqueues the whole exchange and
-        # the reduction while the stream kernel still runs.  HYMET_SCREEN_SYNC_FREE=0 restores the round trip.
-        self.sync_free = os.environ.get("HYMET_SCREEN_SYNC_FREE", "1") != "0"
         self.n_unsettled = 0
 
     def __getattr__(self, name):      # feed_*, reset, stats, set_option ...
@@ -214,8 +211,10 @@ class DistributedScreen:
                 self._all = torch.empty(self.world * n_rec, dtype=torch.int64, device=dev)
             self.scr.counts_compact_async(self._rec[1:].data_ptr(), cap, self._rec.data_ptr())
             work = dist.all_gather_into_tensor(self._all, self._rec, async_op=True)
-        if sparse and self.sync_free:
-            self.scr.flush_async()                        # bottom-s selection enqueued; its verdict travels inside the record
+        if sparse:
+            # one host synchronisation per screen: the host enqueues the whole exchange and the reduction while
+            # the stream kernel still runs; the bottom-s selection's verdict travels inside the record
+            self.scr.flush_async()
         else:
             self.scr.flush()                              # host round trips of the mixture finaliser: the collective runs underneath
         self.scr.mixture_record(self._mix.data_ptr())

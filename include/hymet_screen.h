@@ -137,11 +137,8 @@ int hs_screen_new(hs_db *db, hs_screen **out);
 /* Run on a caller-owned CUDA stream (cudaStream_t as void*; NULL = library's own). */
 int hs_screen_set_stream(hs_screen *s, void *cuda_stream);
 /* Options: "filter" 1/0 = skip probes for hashes above the db's largest key (exact;
- * default 1); "batch_bloom" 1/0 = issue the Bloom-tier reads of four k-mers together (default 1);
- * "sparse" 1/0 = O(present hashes) reduction and reset (default 1; 0 = always the dense kernels); "keep_query" 1 = keep packed chunks in HBM until finish
- * (needed if the mixture threshold must be revisited; 0 is refused with HS_EUNSUPPORTED: one screen holds 3/8 byte per query
- * base in HBM, i.e. ~480 Gbp fit a 180 GB B200 -- split larger read sets across screens and GPUs); "chunk_bases" = host packer
- * chunk size; "piece_bases" = positions per upload+launch piece of packed host feeds;
+ * default 1); "sparse" 1/0 = O(present hashes) reduction and reset (default 1; 0 = always the dense kernels);
+ * "chunk_bases" = host packer chunk size;
  * "ingest" 0/1/2 = host packer only / device parser only / both compete (default; packer
  * threads join when at least six were asked for); "file_readers", "file_block_bytes" = reader
  * threads and nominal block size of the pinned ring that streams plain FASTA files (defaults
@@ -150,8 +147,10 @@ int hs_screen_set_stream(hs_screen *s, void *cuda_stream);
  * where the page cache holds them / chosen by host capability (default: mapped when the packer has
  * its AVX-512 path and at least four threads); "text_chunk_bytes" =
  * bytes of gzip / stdin FASTA inflated per hand-over to the packer threads (default 256 MiB;
- * cut at record starts -- FASTQ too, where the packer's own walk tells a header from a quality line that starts with '@'); "ingest_slots" (1-4), "ingest_batch" (1-8) = depth
- * and granularity of the device parser's raw-text queue. */
+ * cut at record starts -- FASTQ too, where the packer's own walk tells a header from a quality line that starts with '@').
+ * Any other key is refused with HS_EINVAL.  Packed query chunks stay in HBM until reset (the mixture
+ * threshold may have to be revisited): one screen holds 3/8 byte per query base, i.e. ~480 Gbp fit a
+ * 180 GB B200 -- split larger read sets across screens and GPUs. */
 int hs_screen_set_option(hs_screen *s, const char *key, int64_t value);
 
 /* rows a6/a7: stream FASTA/FASTQ (plain or gzip; "-" = stdin).  A plain FASTA file is read by

@@ -41,11 +41,6 @@ for mode, name in ((0, "host"), (2, "hybrid"), (1, "device")):
         if mode == 1:
             break
 scr.set_option("ingest", 2); scr.set_option("chunk_bases", 16 << 20)
-for slots in (2, 4):
-    for batch in (1, 2, 3):
-        scr.set_option("ingest_slots", slots); scr.set_option("ingest_batch", batch)
-        run("hybrid 16 MB slots %d batch %d" % (slots, batch), nthreads)
-scr.set_option("ingest_slots", 4); scr.set_option("ingest_batch", 3)
 
 # the same text as a FILE in the page cache
 import tempfile

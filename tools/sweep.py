@@ -12,7 +12,6 @@ runs = [
     ("c4_wta_clusters", ["--wta", "--clusters", "250"]),
     ("c4_plain_clusters", ["--clusters", "250"]),
     ("c2_tiny10k_bloom", ["--tiny", "10000"]),
-    ("c2_tiny10k_nobloom", ["--tiny", "10000"]),
     ("c5_k21_s5000", ["--s", "5000"]),
     ("c5_k21_s10000", ["--s", "10000"]),
     ("c5_k31_s1000", ["--k", "31"]),
@@ -25,8 +24,7 @@ with open(out, "a") as fh:
         if only and name not in only:
             continue
         cmd = [sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "3", "--warmup", "3", "--no-e2e", "--no-extras", "--workload", "c2"] + extra + (["--no-cpu"] if os.environ.get("SWEEP_NO_CPU") else [])
-        env = dict(os.environ, HYMET_SCREEN_BLOOM="0") if name.endswith("nobloom") else dict(os.environ)
-        r = subprocess.run(cmd, capture_output=True, text=True, timeout=1200, env=env)
+        r = subprocess.run(cmd, capture_output=True, text=True, timeout=1200)
         line = r.stdout.strip().splitlines()[-1] if r.stdout.strip() else ""
         try:
             d = json.loads(line)
