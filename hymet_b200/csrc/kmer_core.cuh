@@ -127,6 +127,22 @@ HS_HD uint64_t fmix64(uint64_t k)
     return k;
 }
 
+// High word of fmix64(k).  Its last xorshift33 changes only the low word, and the high word of the
+// last product is mul.hi(lo, c_lo) + lo * c_hi + hi * c_lo: three multiply-adds, no low-word product.
+HS_HD uint32_t fmix64_hi(uint64_t k)
+{
+    k = xorshift33(k); k *= 0xff51afd7ed558ccdull;
+    k = xorshift33(k);
+    const uint32_t lo = (uint32_t)k, hi = (uint32_t)(k >> 32);
+    const uint32_t c_lo = 0x1a85ec53u, c_hi = 0xc4ceb9feu;
+#if defined(__CUDA_ARCH__)
+    const uint32_t mh = __umulhi(lo, c_lo);
+#else
+    const uint32_t mh = (uint32_t)(((uint64_t)lo * c_lo) >> 32);
+#endif
+    return mh + lo * c_hi + hi * c_lo;
+}
+
 HS_HD uint64_t mul5_add(uint64_t h, uint32_t c)  // h * 5 + c
 {
 #if defined(__CUDA_ARCH__)
@@ -227,10 +243,35 @@ HS_HD uint64_t tail_entry(uint32_t x, int r)
     return k1 * kMurmurC2;
 }
 
+// h1 and h2 of MurmurHash3_x64_128 right before the finalizer: h1 of the hash is fmix64(x) + fmix64(y).
+struct MurmurState { uint64_t x, y; };
+
+HS_HD uint64_t murmur_finish(const MurmurState &s) { return fmix64(s.x) + fmix64(s.y); }
+
+// ---- range gate on the high word ---------------------------------------------------------------
+// The kernels' pre-filter keeps a 64-bit hash h only when h <= gate, and turns away all but a few
+// k-mers in a thousand.  Deciding that from the high words alone saves most of the finalizer:
+// with  s = fmix64_hi(x) + fmix64_hi(y)  (mod 2^32), the true high word of h is s or s + 1, the
+// carry out of the low-word add.  The test  (u32)(s + 1) <= gate_hi + 1  accepts every s in
+// [0, gate_hi] and also s = 0xFFFFFFFF (whose carry wraps the high word to 0), so it accepts every
+// h <= gate: no false negatives.  It also accepts h > gate when hi32(h) == gate_hi (as a compare of
+// high words would), when s == gate_hi carried into gate_hi + 1, and when s == 0xFFFFFFFF did not
+// carry -- a few in 2^32 beyond that.  Callers finish the hash exactly for the k-mers that pass and
+// repeat the exact 64-bit test.  gate_hi + 1 must not wrap: for gate_hi == 0xFFFFFFFF the bound
+// saturates and every k-mer takes the exact test (then every k-mer is let through by the gate
+// anyway).
+HS_HD uint32_t murmur_finish_hi_floor(const MurmurState &s) { return fmix64_hi(s.x) + fmix64_hi(s.y); }
+HS_HD uint32_t hi_gate_bound(uint64_t gate)
+{
+    const uint32_t gate_hi = (uint32_t)(gate >> 32);
+    return gate_hi == 0xFFFFFFFFu ? gate_hi : gate_hi + 1u;
+}
+HS_HD bool hi_gate_may_pass(uint32_t s_hi, uint32_t bound) { return (uint32_t)(s_hi + 1u) <= bound; }
+
 // `Pre::full(cl, i, second)`: 64-bit product of word i's letters; `Pre::low`: its low 32 bits;
 // `Pre::kTail` / `Pre::tail(cl, k)`: the finished tail term when a table of it exists.
 template <class Pre>
-HS_HD uint64_t hash_canonical_premul(uint64_t cl, int k, uint32_t seed, bool use64, const Pre &pre)
+HS_HD MurmurState murmur_state_premul(uint64_t cl, int k, uint32_t seed, const Pre &pre)
 {
     const bool tail_tab = Pre::kTail && tail_table_applies(k);
     uint64_t m[4];
@@ -272,9 +313,14 @@ HS_HD uint64_t hash_canonical_premul(uint64_t cl, int k, uint32_t seed, bool use
     }
     h1 ^= (uint64_t)k; h2 ^= (uint64_t)k;
     h1 += h2; h2 += h1;
-    h1 = fmix64(h1); h2 = fmix64(h2);
-    h1 += h2;
-    return use64 ? h1 : (h1 & 0xFFFFFFFFull);
+    return MurmurState{h1, h2};
+}
+
+template <class Pre>
+HS_HD uint64_t hash_canonical_premul(uint64_t cl, int k, uint32_t seed, bool use64, const Pre &pre)
+{
+    const uint64_t h = murmur_finish(murmur_state_premul(cl, k, seed, pre));
+    return use64 ? h : (h & 0xFFFFFFFFull);
 }
 
 struct PremulArith {  // host-side stand-in for the shared-memory tables (tests)
@@ -372,6 +418,12 @@ template <class Pre>
 HS_HD uint64_t hash_canonical_premul_top(uint64_t ct, int k, uint32_t seed, bool use64, const Pre &pre)
 {
     return hash_canonical_premul(ct, k, seed, use64, TopAdapter<Pre>{pre, k});
+}
+
+template <class Pre>
+HS_HD MurmurState murmur_state_premul_top(uint64_t ct, int k, uint32_t seed, const Pre &pre)
+{
+    return murmur_state_premul(ct, k, seed, TopAdapter<Pre>{pre, k});
 }
 
 // the tail's letters inside a TOP-aligned k-mer: letters 16*(k>>4) .. k-1 end at bit 64-2k, and start at

@@ -53,7 +53,14 @@ __device__ __forceinline__ void mbar_arrive(uint64_t *bar)
 {
     asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
-constexpr unsigned kWaitSleepNs = 100;   // between tries of a warp that is ahead of its CTA
+constexpr unsigned kWaitSuspendNs = 1000000;   // longest a waiting warp stays parked per try
+constexpr uint64_t kWaitTrapNs = 2000000000ull;  // a wait this long is a fault
+__device__ __forceinline__ uint64_t globaltimer_ns()
+{
+    uint64_t t;
+    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
+    return t;
+}
 __device__ __forceinline__ bool mbar_try(uint64_t *bar, uint32_t phase)
 {
     uint32_t ok;
@@ -66,19 +73,32 @@ __device__ __forceinline__ bool mbar_try(uint64_t *bar, uint32_t phase)
         : "memory");
     return ok != 0;
 }
+__device__ __forceinline__ bool mbar_try_suspend(uint64_t *bar, uint32_t phase)
+{
+    uint32_t ok;
+    asm volatile(
+        "{\n\t.reg .pred p;\n\t"
+        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2, %3;\n\t"
+        "selp.u32 %0, 1, 0, p;\n\t}"
+        : "=r"(ok)
+        : "r"(smem_u32(bar)), "r"(phase), "n"(kWaitSuspendNs)
+        : "memory");
+    return ok != 0;
+}
 __device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t phase)
 {
     if (mbar_try(bar, phase)) return;   // the usual case: the tile landed long ago
     // A warp that waits here has run ahead of the slowest warp of its CTA by the whole ring (the tile it wants
     // cannot be issued before its stage is released), so it should get out of the way: spinning on try_wait
     // with a clock read per trip was 3.9 % of all issued warp instructions of the kernel (ncu r02, 13 trips per
-    // wait), taken from the issue slots of the very warps it was waiting for.
-    for (uint32_t spins = 1;; spins++) {
-        __nanosleep(kWaitSleepNs);
-        if (mbar_try(bar, phase)) return;
-        // a tile that never lands means a broken launch contract: fail loudly, never hang the GPU
-        if (spins > (1u << 24)) __trap();
-    }
+    // wait), taken from the issue slots of the very warps it was waiting for.  A sleep-and-retry loop still
+    // cost about 32 trips per wait (r02); with the suspend-time hint the hardware parks the warp until the
+    // phase completes or the hint runs out.
+    // A tile that never lands means a broken launch contract: fail loudly, never hang the GPU.  The bound is
+    // on time, not tries: how long one try stays parked is up to the hardware.
+    const uint64_t t0 = globaltimer_ns();
+    while (!mbar_try_suspend(bar, phase))
+        if (globaltimer_ns() - t0 > kWaitTrapNs) __trap();
 }
 
 __device__ __forceinline__ uint32_t warp_sum(uint32_t v)
@@ -388,6 +408,9 @@ __global__ void __launch_bounds__(kCtaThreads, MODE == 3 ? 3 : kMinCtas) k_strea
 {
     constexpr bool EMIT = MODE == 1, BLOOMB = MODE == 2, COOP = MODE == 3;
     constexpr bool kTailTab = stream_tail_table(KT, MODE);
+    // screen with 64-bit hashes: the range gate is decided on the hash's high word.  (K1 parity emits every
+    // hash, the Bloom tier reads the low bits, the probe-everything kernel probes nearly every k-mer.)
+    constexpr bool kHiGate = MODE == 0 && KT > 16;
     // kStages tile buffers, filled kPrefetch tiles ahead through the TMA engine.
     // full[s]: the bytes of stage s have landed; empty[s]: all 8 warps copied their words of
     // stage s to registers.  No CTA-wide barrier in the loop: warps drift up to two tiles
@@ -464,7 +487,7 @@ __global__ void __launch_bounds__(kCtaThreads, MODE == 3 ? 3 : kMinCtas) k_strea
     uint64_t gate = a.do_mix ? mix_tau : 0;
     if (a.do_count) gate = a.do_filter ? (a.tab.max_key > gate ? a.tab.max_key : gate) : ~0ull;
     if (EMIT) gate = ~0ull;   // K1 parity runs want every hash
-    const uint32_t gate_hi = (uint32_t)(gate >> 32);
+    [[maybe_unused]] const uint32_t gate_hi = (uint32_t)(gate >> 32), gate_bound = hi_gate_bound(gate);
     // Bloom-tier instantiation: hashes <= lowgate are handled without the filter (direct probe, mixture insert)
     const uint64_t lowgate = a.do_mix ? (mix_tau > a.tab.dense_max ? mix_tau : a.tab.dense_max) : a.tab.dense_max;
     [[maybe_unused]] const uint32_t lowgate_hi = (uint32_t)(lowgate >> 32), max_hi = (uint32_t)(a.tab.max_key >> 32);
@@ -635,7 +658,41 @@ __global__ void __launch_bounds__(kCtaThreads, MODE == 3 ? 3 : kMinCtas) k_strea
                 }
             }
         };
-        if (!COOP && ok == ~0u) word(std::false_type{}); else word(std::true_type{});
+        // screen with 64-bit hashes: the gate on high words (kmer_core.cuh: murmur_finish_hi_floor); only the
+        // k-mers that pass, a few in a thousand, get their hash finished and the exact test
+        auto word_hi_gate = [&](auto check) {
+#pragma unroll 1
+            for (int half = 0; half < 2; half++) {
+                const uint32_t fa = half ? w.f0 : w.f1, fb = half ? w.f1 : w.f2, fc = half ? w.f2 : w.f3;
+                const uint32_t ra = half ? w.r1 : w.r0, rb = half ? w.r2 : w.r1, rc = half ? w.r3 : w.r2;
+#pragma unroll 1
+                for (int q = 0; q < 16; q += kIlp) {
+                    bool may[kIlp], any = false;
+#pragma unroll
+                    for (int u = 0; u < kIlp; u++) {
+                        const int j = half * 16 + q + u;
+                        const MurmurState st = murmur_state_premul_top(canonical_top_half(fa, fb, fc, ra, rb, rc, q + u), k, a.seed, L);
+                        may[u] = hi_gate_may_pass(murmur_finish_hi_floor(st), gate_bound) && (!decltype(check)::value || ((ok >> (31 - j)) & 1u));
+                        any |= may[u];
+                    }
+                    if (!any) continue;   // (ptxas: a min of the four high words and one compare)
+                    uint32_t pass = 0;
+#pragma unroll
+                    for (int u = 0; u < kIlp; u++) pass |= (uint32_t)may[u] << u;
+#pragma unroll 1
+                    for (; pass; pass &= pass - 1u) {
+                        const int u = __ffs(pass) - 1;
+                        const uint64_t h = murmur_finish(murmur_state_premul_top(canonical_top_half(fa, fb, fc, ra, rb, rc, q + u), k, a.seed, L));
+                        if (h <= gate) sink(half * 16 + q + u, h, ~0u);
+                    }
+                }
+            }
+        };
+        if constexpr (kHiGate) {
+            if (ok == ~0u) word_hi_gate(std::false_type{}); else word_hi_gate(std::true_type{});
+        } else {
+            if (!COOP && ok == ~0u) word(std::false_type{}); else word(std::true_type{});
+        }
     }
 
     n_valid = warp_sum(n_valid); n_probe = warp_sum(n_probe); n_reads = warp_sum(n_reads);
