@@ -13,8 +13,10 @@
 
 #if defined(__CUDACC__)
 #define HS_HD __host__ __device__ __forceinline__
+#define HS_HDC __host__ __device__ constexpr
 #else
 #define HS_HD inline
+#define HS_HDC constexpr
 #endif
 
 namespace hs {
@@ -395,15 +397,65 @@ HS_HD uint64_t canonical_top(const Win &w, int j)
                   : canonical_top_half(w.f0, w.f1, w.f2, w.r1, w.r2, w.r3, j - 16);
 }
 
-HS_HD uint32_t top_word_index64(uint64_t ct, int i, int k)
+// index byte of word i, times 2^lg (the table's entry stride)
+HS_HD uint32_t top_word_index(uint64_t ct, int i, int k, int lg)
 {
     const uint32_t w = i < 4 ? (uint32_t)(ct >> 32) : (uint32_t)ct;
-    const int sh = 18 - 8 * (i & 3);
+    const int sh = 24 - lg - 8 * (i & 3);
     const uint32_t x = sh >= 0 ? (w >> sh) : (w << (-sh));
     const int nb = k - 4 * i;   // bases of this word that belong to the k-mer
-    const uint32_t keep = nb >= 4 ? 0x3FC0u : ((0xFFu << (8 - 2 * nb)) & 0xFFu) << 6;
+    const uint32_t keep = (nb >= 4 ? 0xFFu : ((0xFFu << (8 - 2 * nb)) & 0xFFu)) << lg;
     return x & keep;
 }
+
+// ---- shared-memory layout of the stream kernel's tables (screen_kernels.cu: SmemPremul) -------------
+// The host tests model the 32 banks with these same functions.
+//   Premultiplied tables: 256 entries, COPIES lane copies each; entry b, copy c at b * 8 * COPIES + c * 8.
+//     Lane l reads copy l mod COPIES.  With 16 copies the entry stride is 128 B, so the 16 lanes of a
+//     half-warp read 16 different bank pairs whatever their entries: a 64-bit read takes 2 wavefronts, a
+//     32-bit read (the low word) 2.  The second table lies kBytes further on, reached through the
+//     load's immediate offset; the base is kBytes-aligned, so lane term and index combine with one OR.
+//   Tail-term table: 4^r entries, TCOPIES interleaved copies; entry e, copy c at (e * TCOPIES + c) * 8.
+//     Lane l reads copy l mod TCOPIES, so the lanes of different copies read disjoint sets of bank pairs.
+//     The table lies 2 * kBytes above the same base.
+template <int COPIES, int TCOPIES>
+struct SmemLayout {
+    static constexpr uint32_t kStride = 8u * COPIES, kBytes = 256u * kStride;
+    static constexpr int kStrideLog2 = COPIES == 16 ? 7 : COPIES == 8 ? 6 : -1;
+    static constexpr int kTailLog2 = TCOPIES == 2 ? 4 : TCOPIES == 1 ? 3 : -1;
+    static_assert(kStrideLog2 > 0 && kTailLog2 > 0, "layouts with 8 or 16 copies, 1 or 2 tail copies");
+    HS_HDC static uint32_t tail_bytes(int r) { return (8u * TCOPIES) << (2 * r); }
+    HS_HD static uint32_t lane_base(uint32_t lut, uint32_t lane) { return lut | ((lane & (COPIES - 1u)) << 3); }
+    HS_HD static uint32_t tail_base(uint32_t lut, uint32_t lane) { return lut | ((lane & (TCOPIES - 1u)) << 3); }
+    // Word i's entry (add kBytes for the second table).  A whole word's index byte sits on a byte boundary
+    // of the top-aligned k-mer: ONE byte permute (ALU pipe) and ONE multiply-add (FMA pipe) by `stride`
+    // (== kStride; the kernel passes it in a register the compiler cannot see through, or ptxas would
+    // strength-reduce the multiply back to a shift and a three-input logic op, two ALU-pipe instructions,
+    // and the kernel is bound by the half-rate ALU pipe).  A partial last word keeps the masked form.
+    HS_HD static uint32_t word_addr(uint64_t ct, int i, int k, uint32_t base, uint32_t stride)
+    {
+        if (k - 4 * i >= 4) {
+            const uint32_t w = i < 4 ? (uint32_t)(ct >> 32) : (uint32_t)ct;
+#if defined(__CUDA_ARCH__)
+            const uint32_t byte = __byte_perm(w, 0u, 0x4440u + (uint32_t)(3 - (i & 3)));
+            uint32_t addr;
+            asm("mad.lo.u32 %0, %1, %2, %3;" : "=r"(addr) : "r"(byte), "r"(stride), "r"(base));
+            return addr;
+#else
+            return ((w >> (8 * (3 - (i & 3)))) & 0xFFu) * stride + base;
+#endif
+        }
+        return top_word_index(ct, i, k, kStrideLog2) | base;
+    }
+    // the tail's entry (add 2 * kBytes): its letters start at the top of one 32-bit half of the k-mer
+    // (top_tail_index), so one shift and one AND-OR
+    HS_HD static uint32_t tail_addr(uint64_t ct, int k, uint32_t tbase)
+    {
+        const int r = k & 15;
+        const uint32_t w = (k >> 4) ? (uint32_t)ct : (uint32_t)(ct >> 32);
+        return ((w >> (32 - 2 * r - kTailLog2)) & (((1u << (2 * r)) - 1u) << kTailLog2)) | tbase;
+    }
+};
 
 template <class Pre>
 struct TopAdapter {   // `where` turns (k-mer, word number) into whatever the table accessor addresses by
@@ -438,7 +490,7 @@ HS_HD uint32_t top_tail_index(uint64_t ct, int k)
 struct PremulArithMsb {  // host-side stand-in for the shared-memory tables (tests)
     static constexpr bool kTail = true;
     HS_HD uint64_t tail(uint64_t ct, int k) const { return tail_entry(top_tail_index(ct, k), k & 15); }
-    HS_HD uint32_t where(uint64_t ct, int i, int k) const { return top_word_index64(ct, i, k); }
+    HS_HD uint32_t where(uint64_t ct, int i, int k) const { return top_word_index(ct, i, k, 6); }
     HS_HD uint64_t full(uint32_t index64, bool second) const { return premul_entry_msb(index64 >> 6, second); }
     HS_HD uint32_t low(uint32_t index64, bool second) const { return (uint32_t)full(index64, second); }
 };

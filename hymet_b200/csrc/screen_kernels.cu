@@ -323,80 +323,71 @@ __device__ __forceinline__ void mix_insert(const MixView &m, uint64_t *set, uint
 // ---------------------------------------------------------------------------
 // K1 + K2 (+ K3 insert): the streaming kernel
 // ---------------------------------------------------------------------------
+template <int WORDS>
 struct __align__(16) TileBuf {
-    uint64_t seq[kTileWords + 2];  // [1] = halo word, [2..] = the tile
-    uint32_t inv[kTileWords + 4];  // [3] = halo word, [4..] = the tile
+    uint64_t seq[WORDS + 2];  // [1] = halo word, [2..] = the stage's words
+    uint32_t inv[WORDS + 4];  // [3] = halo word, [4..] = the stage's words
 };
-static_assert(sizeof(TileBuf) % 16 == 0, "tile buffers must keep 16-byte alignment");
+static_assert(sizeof(TileBuf<kTileWords>) % 16 == 0 && sizeof(TileBuf<2 * kTileWords>) % 16 == 0,
+              "tile buffers must keep 16-byte alignment");
+
+// Shape of a stream-kernel CTA.  The screen kernels run as 2 CTAs of 512 threads per SM: one set of tables
+// serves 16 warps, and the space two more sets would take holds 16 lane copies of the premultiplied tables
+// (conflict-free reads, kmer_core.cuh: SmemLayout) and 2 copies of the tail-term table:
+//     1 KB system + 24.2 KB ring + slack to 32 KB + 2 x 32 KB tables + 16 KB tail = 112 KB, twice per SM.
+// (Before: 4 CTAs of 256 threads, 8 copies, one tail copy, 56 KB each; 22.9 wavefronts per warp-k-mer, ncu r02.)
+// The probe-everything kernel (MODE 3), which lives on L1/L2 traffic, keeps 3 CTAs of 256 threads with
+// 8 copies and no tail table: 32 KB of tables per CTA instead of 64 leave L1 its room.
+__host__ __device__ constexpr int stream_threads(int mode) { return mode == 3 ? 256 : 512; }
+__host__ __device__ constexpr int stream_copies(int mode) { return mode == 3 ? 8 : 16; }
+// compile-time k with a 1..5 letter tail (k = 21): the tail term comes from its own table
+__host__ __device__ constexpr bool stream_tail_table(int kt, int mode)
+{
+    return mode != 3 && kt > 0 && (kt & 15) >= 1 && (kt & 15) <= 5;
+}
+template <int KT, int MODE>
+using StreamLayout = SmemLayout<stream_copies(MODE), stream_tail_table(KT, MODE) ? 2 : 1>;
+// bytes of the table window: both premultiplied tables and, where used, the tail table
+template <int KT, int MODE>
+__host__ __device__ constexpr uint32_t stream_table_bytes()
+{
+    using Lay = StreamLayout<KT, MODE>;
+    return 2 * Lay::kBytes + (stream_tail_table(KT, MODE) ? Lay::tail_bytes(KT & 15) : 0u);
+}
 
 // Pre-multiplied murmur tables (kmer_core.cuh: hash_canonical_premul): (u64)letters*c1 and
-// (u64)letters*c2 for all 256 four-letter words, 8 lane copies each (entry b, copy c at
-// b*64 + c*8 bytes) = 16 KB per table, adjacent, at a 16 KB-ALIGNED shared address, so that the
-// address of a lookup is
-//     (index byte << 6, taken from the k-mer with one shift and the AND below) | (table base | (lane & 7) * 8)
-// i.e. one shift + one LOP3 instead of shift/and/or/lea -- the kernel is ALU-pipe bound (ncu).  A
-// half-warp's 64-bit loads touch each bank pair once per copy; two lanes share a copy (2-way conflict
-// when their entries differ in parity).  The second table is reached through the load's immediate
-// offset.  (First version: a 16-copy table of the ASCII letters and the multiply done in registers.)
-constexpr uint32_t kLutBytes = 16384;   // alignment and size of one table
-constexpr uint32_t kPreBytes = 256 * 8 * 8;
-static_assert(kPreBytes == 16384 && kPreBytes == kLutBytes, "SmemPremul's loads carry this offset as an immediate");
-constexpr uint32_t kTailBytes = 8192;   // 4^5 finished tail terms (kmer_core.cuh: tail_entry), right behind the two tables
-template <bool TAIL>
+// (u64)letters*c2 for all 256 four-letter words, in the lane-copied layout of SmemLayout at a
+// kBytes-ALIGNED shared address.  The second table and the tail table are reached through the loads'
+// immediate offsets.  (First version: a 16-copy table of the ASCII letters and the multiply done in registers.)
+template <bool TAIL, class Lay>
 struct SmemPremul {
     static constexpr bool kTail = TAIL;
-    uint32_t base;  // table address | (lane & 7) * 8
-    uint32_t k64;   // the constant 64 in a register the compiler cannot see through (below)
-    uint32_t lut;   // table address alone (16 KB aligned): the tail table has no lane copies
+    uint32_t base;    // Lay::lane_base
+    uint32_t stride;  // Lay::kStride in a register the compiler cannot see through (SmemLayout::word_addr)
+    uint32_t tbase;   // Lay::tail_base
     // finished tail term of a top-aligned k-mer: one shift, one AND-OR, one 64-bit load
     __device__ __forceinline__ uint64_t tail(uint64_t ct, int k) const
     {
-        const int r = k & 15;
-        const uint32_t w = (k >> 4) ? (uint32_t)ct : (uint32_t)(ct >> 32);
-        const uint32_t addr = ((w >> (29 - 2 * r)) & (((1u << (2 * r)) - 1u) << 3)) | lut;
         uint64_t v;
-        asm("ld.shared.u64 %0, [%1+32768];" : "=l"(v) : "r"(addr));
+        asm("ld.shared.u64 %0, [%1+%2];" : "=l"(v) : "r"(Lay::tail_addr(ct, k, tbase)), "n"(2 * Lay::kBytes));
         return v;
     }
-    // Address of word i's entry.  The index byte sits on a byte boundary of the top-aligned k-mer, so it
-    // is ONE byte permute (ALU pipe) and ONE multiply-add by 64 (FMA pipe) instead of a shift and a
-    // three-input logic op (two ALU-pipe instructions): the kernel is bound by the half-rate ALU pipe
-    // (ncu: 74 % busy) while the FMA pipe idles at 26 %.  A multiplier the compiler could see would be
-    // strength-reduced back to a shift/LEA on the ALU pipe.  Partial last words keep the masked form.
-    __device__ __forceinline__ uint32_t where(uint64_t ct, int i, int k) const
-    {
-        if (k - 4 * i >= 4) {
-            const uint32_t w = i < 4 ? (uint32_t)(ct >> 32) : (uint32_t)ct;
-            const uint32_t byte = __byte_perm(w, 0u, 0x4440u + (uint32_t)(3 - (i & 3)));
-            uint32_t addr;
-            asm("mad.lo.u32 %0, %1, %2, %3;" : "=r"(addr) : "r"(byte), "r"(k64), "r"(base));
-            return addr;
-        }
-        return top_word_index64(ct, i, k) | base;
-    }
+    __device__ __forceinline__ uint32_t where(uint64_t ct, int i, int k) const { return Lay::word_addr(ct, i, k, base, stride); }
     __device__ __forceinline__ uint64_t full(uint32_t addr, bool second) const
     {
         uint64_t v;
-        if (second) asm("ld.shared.u64 %0, [%1+16384];" : "=l"(v) : "r"(addr));
+        if (second) asm("ld.shared.u64 %0, [%1+%2];" : "=l"(v) : "r"(addr), "n"(Lay::kBytes));
         else asm("ld.shared.u64 %0, [%1];" : "=l"(v) : "r"(addr));
         return v;
     }
     __device__ __forceinline__ uint32_t low(uint32_t addr, bool second) const
     {
         uint32_t v;
-        if (second) asm("ld.shared.u32 %0, [%1+16384];" : "=r"(v) : "r"(addr));
+        if (second) asm("ld.shared.u32 %0, [%1+%2];" : "=r"(v) : "r"(addr), "n"(Lay::kBytes));
         else asm("ld.shared.u32 %0, [%1];" : "=r"(v) : "r"(addr));
         return v;
     }
 };
-
-constexpr int kMinCtas = 4;   // 48 KB of shared memory per CTA
-// compile-time k with a 1..5 letter tail (k = 21): the tail term comes from its own table.  It takes 8 KB
-// from the L1 of every CTA, so the probe-everything kernel (MODE 3), which lives on L1/L2 traffic, goes without
-__host__ __device__ constexpr bool stream_tail_table(int kt, int mode)
-{
-    return mode != 3 && kt > 0 && (kt & 15) >= 1 && (kt & 15) <= 5;
-}
 constexpr int kIlp = 4;   // k-mers hashed side by side per thread (measured, ms per Gbp: 1: 5.33, 2: 5.02, 4: 4.83, 8: 6.47)
 
 // MODE: 0 = screen, 1 = K1 parity (emit every hash), 2 = screen with the Bloom reads of a group of
@@ -404,15 +395,19 @@ constexpr int kIlp = 4;   // k-mers hashed side by side per thread (measured, ms
 // (nearly) every k-mer: the warp looks its hashes up cooperatively (coop_probe), control flow stays
 // warp-uniform and the CTA may use twice the registers (the kernel waits on HBM, not on issue slots)
 template <int KT, int MODE>
-__global__ void __launch_bounds__(kCtaThreads, MODE == 3 ? 3 : kMinCtas) k_stream(const StreamArgs a)
+__global__ void __launch_bounds__(stream_threads(MODE), MODE == 3 ? 3 : 2) k_stream(const StreamArgs a)
 {
     constexpr bool EMIT = MODE == 1, BLOOMB = MODE == 2, COOP = MODE == 3;
     constexpr bool kTailTab = stream_tail_table(KT, MODE);
+    using Lay = StreamLayout<KT, MODE>;
+    // one word per thread: a stage of the ring holds kSpan consecutive tiles of the chunk
+    constexpr uint32_t kThreads = stream_threads(MODE), kSpan = kThreads / kTileWords;
+    static_assert(kThreads % kTileWords == 0, "a stage holds whole tiles");
     // screen with 64-bit hashes: the range gate is decided on the hash's high word.  (K1 parity emits every
     // hash, the Bloom tier reads the low bits, the probe-everything kernel probes nearly every k-mer.)
     constexpr bool kHiGate = MODE == 0 && KT > 16;
     // kStages tile buffers, filled kPrefetch tiles ahead through the TMA engine.
-    // full[s]: the bytes of stage s have landed; empty[s]: all 8 warps copied their words of
+    // full[s]: the bytes of stage s have landed; empty[s]: all warps copied their words of
     // stage s to registers.  No CTA-wide barrier in the loop: warps drift up to two tiles
     // apart (ncu r01: 12 % of warp time sat in __syncthreads with the 2-stage version).
     // WHO issues a tile: whichever warp gets to an iteration first claims the outstanding tile
@@ -427,10 +422,10 @@ __global__ void __launch_bounds__(kCtaThreads, MODE == 3 ? 3 : kMinCtas) k_strea
     // other three CTAs of the SM fill the sleepers' issue slots; the limit is the ALU pipe, not the number of
     // warps awake.)
     constexpr uint32_t kStages = 4, kPrefetch = 2;
-    __shared__ TileBuf buf[kStages];
+    __shared__ TileBuf<kThreads> buf[kStages];
     __shared__ __align__(8) uint64_t full[kStages], empty[kStages];
     __shared__ uint32_t issue_next;   // ordinal (iteration index of this CTA) of the next tile nobody has issued
-    extern __shared__ __align__(16) uint8_t dyn_smem[];  // 2 * kLutBytes: room to align the table to 16 KB
+    extern __shared__ __align__(16) uint8_t dyn_smem[];  // the tables plus the room to align them to Lay::kBytes
 
     const int k = KT ? KT : a.k;
     const bool use64 = KT ? (KT > 16) : (a.use64 != 0);
@@ -439,35 +434,38 @@ __global__ void __launch_bounds__(kCtaThreads, MODE == 3 ? 3 : kMinCtas) k_strea
     if (tid == 0) {
         for (uint32_t i = 0; i < kStages; i++) {
             mbar_init(&full[i], 1);
-            mbar_init(&empty[i], kCtaThreads / 32);
+            mbar_init(&empty[i], kThreads / 32);
         }
         issue_next = kPrefetch;   // the prologue below issues ordinals 0 .. kPrefetch-1
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
         asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
     }
     const uint32_t dyn_addr = smem_u32(dyn_smem);
-    const uint32_t lut_addr = (dyn_addr + (kLutBytes - 1)) & ~(kLutBytes - 1);
+    const uint32_t lut_addr = (dyn_addr + (Lay::kBytes - 1)) & ~(Lay::kBytes - 1);
     {
         uint32_t dyn_size;
         asm("mov.u32 %0, %%dynamic_smem_size;" : "=r"(dyn_size));
-        if (lut_addr + 2 * kPreBytes + (kTailTab ? kTailBytes : 0u) > dyn_addr + dyn_size) __trap();  // launch did not leave room for the aligned tables
+        if (lut_addr + stream_table_bytes<KT, MODE>() > dyn_addr + dyn_size) __trap();  // launch did not leave room for the aligned tables
         uint64_t *t = reinterpret_cast<uint64_t *>(dyn_smem + (lut_addr - dyn_addr));
-        for (uint32_t i = tid; i < 2 * 256 * 8; i += kCtaThreads) t[i] = premul_entry_msb((i >> 3) & 255u, i >= 256 * 8);
+        constexpr uint32_t kCopies = stream_copies(MODE);
+        for (uint32_t i = tid; i < 2 * 256 * kCopies; i += kThreads) t[i] = premul_entry_msb((i / kCopies) & 255u, i >= 256 * kCopies);
         if (kTailTab)
-            for (uint32_t i = tid; i < (1u << (2 * (KT & 15))); i += kCtaThreads) t[2 * 256 * 8 + i] = tail_entry(i, KT & 15);
+            for (uint32_t i = tid; i < (2u << (2 * (KT & 15))); i += kThreads) t[2 * 256 * kCopies + i] = tail_entry(i >> 1, KT & 15);
     }
     __syncthreads();
-    uint32_t lut_lane = lut_addr | ((lane & 7u) << 3);
+    uint32_t lut_lane = Lay::lane_base(lut_addr, lane), tail_lane = Lay::tail_base(lut_addr, lane);
     asm volatile("mov.u32 %0, %0;" : "+r"(lut_lane));  // one opaque per-thread register: keeps ptxas from
                                                         // splitting it back into uniform base + lane term
-    uint32_t k64 = 64u;
-    asm volatile("mov.u32 %0, %0;" : "+r"(k64));
-    const SmemPremul<kTailTab> L{lut_lane, k64, lut_addr};
+    asm volatile("mov.u32 %0, %0;" : "+r"(tail_lane));
+    uint32_t stride = Lay::kStride;
+    asm volatile("mov.u32 %0, %0;" : "+r"(stride));
+    const SmemPremul<kTailTab, Lay> L{lut_lane, stride, tail_lane};
 
     auto issue = [&](uint32_t tile, uint32_t b) {
-        // tile 0 has no halo (positions before the chunk do not exist)
+        // tile 0 has no halo (positions before the chunk do not exist); a stage never reads past the launch's tiles
         const uint32_t sw = tile ? 2u : 0u, iw = tile ? 4u : 0u;
-        const uint32_t sbytes = (kTileWords + sw) * 8u, ibytes = (kTileWords + iw) * 4u;
+        const uint32_t nw = (a.n_tiles - tile >= kSpan ? kSpan : a.n_tiles - tile) * kTileWords;
+        const uint32_t sbytes = (nw + sw) * 8u, ibytes = (nw + iw) * 4u;
         mbar_expect_tx(&full[b], sbytes + ibytes);
         bulk_g2s(&buf[b].seq[2 - sw], a.seq + (size_t)tile * kTileWords - sw, sbytes, &full[b]);
         bulk_g2s(&buf[b].inv[4 - iw], a.inv + (size_t)tile * kTileWords - iw, ibytes, &full[b]);
@@ -492,12 +490,14 @@ __global__ void __launch_bounds__(kCtaThreads, MODE == 3 ? 3 : kMinCtas) k_strea
     const uint64_t lowgate = a.do_mix ? (mix_tau > a.tab.dense_max ? mix_tau : a.tab.dense_max) : a.tab.dense_max;
     [[maybe_unused]] const uint32_t lowgate_hi = (uint32_t)(lowgate >> 32), max_hi = (uint32_t)(a.tab.max_key >> 32);
     uint32_t n_valid = 0, n_probe = 0, n_reads = 0, n_hits = 0, n_mix = 0;
-    uint32_t tile = a.tile_begin + blockIdx.x, it = 0;
+    // first tile of this CTA's stages: ordinal it covers tiles tile_begin + (blockIdx.x + it * gridDim.x) * kSpan ...
+    const uint32_t tile_step = gridDim.x * kSpan;
+    uint32_t tile = a.tile_begin + blockIdx.x * kSpan, it = 0;
     if (tid == 0)
         for (uint32_t p = 0; p < kPrefetch; p++)
-            if ((uint64_t)tile + (uint64_t)p * gridDim.x < a.n_tiles) issue(tile + p * gridDim.x, p);
+            if ((uint64_t)tile + (uint64_t)p * tile_step < a.n_tiles) issue(tile + p * tile_step, p);
 
-    for (; tile < a.n_tiles; tile += gridDim.x, it++) {
+    for (; tile < a.n_tiles; tile += tile_step, it++) {
         if (lane == 0) {
             // Ordinals up to it + kPrefetch should be on their way; claim the ones that are not.  The tile this
             // warp is about to wait for (ordinal it) MUST be issued, so for it the stage's release is waited
@@ -506,7 +506,7 @@ __global__ void __launch_bounds__(kCtaThreads, MODE == 3 ? 3 : kMinCtas) k_strea
             // here for the slowest one, 4 % of all issued instructions).
             for (;;) {
                 const uint32_t nt = *reinterpret_cast<volatile uint32_t *>(&issue_next);
-                const uint64_t ntile = (uint64_t)a.tile_begin + blockIdx.x + (uint64_t)nt * gridDim.x;
+                const uint64_t ntile = (uint64_t)a.tile_begin + ((uint64_t)blockIdx.x + (uint64_t)nt * gridDim.x) * kSpan;
                 if (nt > it + kPrefetch || ntile >= a.n_tiles) break;
                 const uint32_t sb = nt % kStages;
                 const uint32_t par = ((nt / kStages) - 1u) & 1u;   // parity of the phase that frees the stage (ordinal nt - kStages consumed by all)
@@ -533,8 +533,10 @@ __global__ void __launch_bounds__(kCtaThreads, MODE == 3 ? 3 : kMinCtas) k_strea
 
         if (tile == 0 && tid == 0) { prev = 0; iprev = ~0u; }
         const uint64_t pos0 = ((uint64_t)tile * kTileWords + tid) * kBasesPerWord;
-        if (pos0 + kBasesPerWord > n_bases) {
-            const uint32_t nv = pos0 >= n_bases ? 0u : (uint32_t)(n_bases - pos0);
+        // (a word of a tile past the launch's last one belongs to the next launch: it was not loaded)
+        const bool beyond = kSpan > 1 && tile + tid / kTileWords >= a.n_tiles;
+        if (beyond || pos0 + kBasesPerWord > n_bases) {
+            const uint32_t nv = beyond || pos0 >= n_bases ? 0u : (uint32_t)(n_bases - pos0);
             icur |= nv ? ((1u << (32 - nv)) - 1u) : ~0u;
         }
         if (!COOP && icur == ~0u) continue;  // padding / all-N word: no k-mer ends here (COOP: every lane stays for the warp's lookups)
@@ -722,18 +724,19 @@ static cudaError_t launch_stream_t(const StreamArgs &a, int sm_count, cudaStream
     {
         std::lock_guard<std::mutex> lk(mu);
         if (!occ_dev[dev]) {
-            // the tables need a 16 KB-aligned 32 KB window.  Dynamic shared memory starts right after the
-            // 1 KB the system reserves per CTA and the kernel's static buffers, so ask for exactly the
-            // distance to the next 16 KB boundary plus the tables (the kernel traps if that ever stops
-            // being true): 4 CTAs of 48 KB per SM instead of 3 with a full 16 KB of slack.
+            // the tables need a window aligned to the size of one premultiplied table.  Dynamic shared memory
+            // starts right after the 1 KB the system reserves per CTA and the kernel's static buffers, so ask
+            // for exactly the distance to the next boundary plus the tables (the kernel traps if that ever
+            // stops being true): 2 CTAs of 112 KB per SM (MODE 3: 3 of 48 KB) instead of one with the
+            // whole alignment as slack.
+            constexpr uint32_t kAlign = StreamLayout<KT, MODE>::kBytes;
             cudaFuncAttributes fa;
             if ((e = cudaFuncGetAttributes(&fa, k_stream<KT, MODE>)) != cudaSuccess) return e;
             const uint32_t start = 1024u + (((uint32_t)fa.sharedSizeBytes + 15u) & ~15u);
-            const uint32_t d = (((start + kLutBytes - 1) & ~(kLutBytes - 1)) - start) + 2 * kPreBytes +
-                               (stream_tail_table(KT, MODE) ? kTailBytes : 0u);
+            const uint32_t d = (((start + kAlign - 1) & ~(kAlign - 1)) - start) + stream_table_bytes<KT, MODE>();
             if ((e = cudaFuncSetAttribute(k_stream<KT, MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)d)) != cudaSuccess) return e;
             int o = 0;
-            e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o, k_stream<KT, MODE>, kCtaThreads, d);
+            e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o, k_stream<KT, MODE>, stream_threads(MODE), d);
             if (e != cudaSuccess) return e;
             dyn_dev[dev] = d;
             occ_dev[dev] = o < 1 ? 1 : o;
@@ -741,10 +744,12 @@ static cudaError_t launch_stream_t(const StreamArgs &a, int sm_count, cudaStream
         occ = occ_dev[dev];
         dyn = dyn_dev[dev];
     }
+    constexpr uint32_t kSpan = stream_threads(MODE) / kTileWords;   // tiles per CTA iteration
     uint32_t grid = (uint32_t)sm_count * (uint32_t)occ;
-    if (grid > a.n_tiles - a.tile_begin) grid = a.n_tiles - a.tile_begin;
+    const uint32_t stages = (uint32_t)(((uint64_t)a.n_tiles - a.tile_begin + kSpan - 1) / kSpan);
+    if (grid > stages) grid = stages;
     if (!grid) return cudaSuccess;
-    k_stream<KT, MODE><<<grid, kCtaThreads, dyn, st>>>(a);
+    k_stream<KT, MODE><<<grid, stream_threads(MODE), dyn, st>>>(a);
     return cudaGetLastError();
 }
 

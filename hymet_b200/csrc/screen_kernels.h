@@ -8,8 +8,7 @@
 
 namespace hs {
 
-constexpr int kTileWords = 256;    // one CTA pass = 256 words = 8192 bases
-constexpr int kCtaThreads = 256;
+constexpr int kTileWords = 256;    // 256 words = 8192 bases; the stream kernel's CTAs take 1 or 2 tiles per pass
 constexpr uint32_t kNoEntry = 0xFFFFFFFFu;
 
 // counters accumulated by the streaming kernel (device, 64-bit each)
