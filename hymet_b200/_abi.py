@@ -52,6 +52,16 @@ class Stats(C.Structure):
         return {f: getattr(self, f) for f, _ in self._fields_}
 
 
+class SketchStats(C.Structure):
+    _fields_ = [("n_genomes", C.c_uint64), ("n_bases", C.c_uint64), ("n_positions", C.c_uint64),
+                ("n_batches", C.c_uint32), ("n_launches", C.c_uint32), ("n_passes", C.c_uint32),
+                ("ms_stream", C.c_float), ("ms_select", C.c_float),
+                ("t_read_s", C.c_double), ("t_pack_s", C.c_double), ("t_wait_s", C.c_double), ("t_total_s", C.c_double)]
+
+    def asdict(self):
+        return {f: getattr(self, f) for f, _ in self._fields_}
+
+
 # name -> (restype, argtypes).  Must list every symbol include/hymet_screen.h declares
 # (tests/test_abi.py checks the header against this table and against the .so).
 SIGNATURES = {
@@ -112,6 +122,13 @@ SIGNATURES = {
     "hs_gather_bench": (C.c_int, [C.c_void_p, C.c_uint64, C.c_uint64, C.POINTER(C.c_float)]),
     "hs_db_entry_ids": (C.c_int, [C.c_void_p, u32p]),
     "hs_stat_batch": (C.c_int, [C.c_uint32, C.c_uint64, C.c_uint64, u64p, u64p, f64p, f64p]),
+    "hs_sketcher_new": (C.c_int, [C.c_uint32, C.c_uint32, C.c_uint32, C.c_int, C.POINTER(C.c_void_p)]),
+    "hs_sketcher_add_file": (C.c_int, [C.c_void_p, C.c_char_p]),
+    "hs_sketcher_run": (C.c_int, [C.c_void_p]),
+    "hs_sketcher_result": (C.c_int, [C.c_void_p, C.c_uint64, C.POINTER(u64p), u32p, u64p, u64p,
+                                     C.POINTER(C.c_void_p), u64p]),
+    "hs_sketcher_stats": (C.c_int, [C.c_void_p, C.POINTER(SketchStats)]),
+    "hs_sketcher_free": (None, [C.c_void_p]),
     "hs_sketch_text": (C.c_int, [C.c_uint32, C.c_uint32, C.c_uint32, C.c_void_p, C.c_size_t, u64p, u32p, u64p]),
     "hs_sketch_packed_device": (C.c_int, [C.c_uint32, C.c_uint32, C.c_uint32, C.c_void_p, C.c_void_p, C.c_uint64,
                                           u64p, u32p]),

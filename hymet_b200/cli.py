@@ -180,12 +180,16 @@ Description:
 
   Create a sketch file (.msh): for every input file the s smallest distinct
   canonical k-mer hashes of all its records (one reference per file, named after
-  the file).  Computed on the GPU with the same hash kernel as `mash screen`.
+  the file).  Inputs are FASTA or FASTQ, gzipped or not.  Computed on the GPU
+  with the same hash kernel as `mash screen`, many genomes per kernel pass.
 
 Options:
 
   -h          Help
+  -l          List input. Each positional argument is a file that lists one
+              input path per line (empty lines are ignored).
   -o <path>   Output prefix (".msh" is appended unless present) [first input]
+  -p <int>    Host threads reading, inflating and packing input files [1]
   -k <int>    K-mer size, 1-32 [21]
   -s <int>    Sketch size [1000]
   -S <int>    Hash seed [42]
@@ -196,7 +200,7 @@ def sketch_main(args: List[str], stdout=None) -> int:
     """`mash sketch` (SURVEY.md 8f rank 1): HYMET never runs it (its three databases are
     downloaded pre-built, README.md:164-169) but a drop-in without it cannot refresh them."""
     stdout = stdout or sys.stdout
-    k, s, seed, out = 21, 1000, 42, None
+    k, s, seed, threads, out, lists = 21, 1000, 42, 1, None, False
     pos: List[str] = []
     i = 0
     try:
@@ -205,7 +209,9 @@ def sketch_main(args: List[str], stdout=None) -> int:
             if a == "-h":
                 stdout.write(SKETCH_USAGE)
                 return 0
-            if a in ("-o", "-k", "-s", "-S", "-p"):
+            if a == "-l":
+                lists = True
+            elif a in ("-o", "-k", "-s", "-S", "-p"):
                 if i + 1 >= len(args):
                     _err("-%s requires an argument" % a[1])
                     return 1
@@ -219,6 +225,8 @@ def sketch_main(args: List[str], stdout=None) -> int:
                     s = int(v)
                 elif a == "-S":
                     seed = int(v)
+                else:
+                    threads = int(v)
             elif a.startswith("-") and a != "-":
                 _err("Unrecognized option: %s" % a)
                 return 1
@@ -234,35 +242,49 @@ def sketch_main(args: List[str], stdout=None) -> int:
     if not (1 <= k <= 32) or s < 1:
         _err("k-mer size must be 1-32 and sketch size positive")
         return 1
-    import gzip
-
+    if threads < 1:
+        _err("option value out of range")
+        return 1
+    paths: List[str] = []
+    if lists:
+        for lf in pos:
+            try:
+                with open(lf, "rb") as fh:
+                    listed = fh.read()
+            except OSError:
+                _err("could not open %s for reading." % lf)
+                return 1
+            paths += [os.fsdecode(ln) for ln in listed.split(b"\n") if ln]
+        if not paths:
+            _err("no input files listed in %s" % " ".join(pos))
+            return 1
+    else:
+        paths = pos
+    for p in paths:
+        if not os.path.exists(p):
+            _err("could not open %s for reading." % p)
+            return 1
     import numpy as np
 
     from . import msh as mshfmt
     from . import screen as hs
     device = int(os.environ.get("HYMET_SCREEN_DEVICE", "0"))
-    names, comments, lengths, sketches = [], [], [], []
+    sys.stderr.write("Sketching %d file%s...\n" % (len(paths), "" if len(paths) == 1 else "s"))
     try:
-        for p in pos:
-            if not os.path.exists(p):
-                _err("could not open %s for reading." % p)
-                return 1
-            with (gzip.open(p, "rb") if p.endswith(".gz") else open(p, "rb")) as fh:
-                text = fh.read()
-            sys.stderr.write("Sketching %s...\n" % p)
-            h, total = hs.sketch_text(text, k, s, seed, device)
-            n_rec = text.count(b"\n>") + (1 if text.startswith(b">") else 0)
-            first = text[1:text.find(b"\n")].decode("utf-8", "replace").strip() if text.startswith(b">") else ""
-            if n_rec > 1:  # Mash's comment convention for multi-record genomes
-                first = "[%d seqs] %s [...]" % (n_rec, first)
-            names.append(p); comments.append(first); lengths.append(total); sketches.append(h)
+        sketches, _ = hs.sketch_files(paths, k, s, seed, threads, device)
     except hs.HsError as e:
         _err(e.msg)
         return 1
-    offsets = np.concatenate([[0], np.cumsum([len(h) for h in sketches])]).astype(np.uint64)
-    db = mshfmt.SketchDB(k=k, s=s, seed=seed, names=names, comments=comments,
-                         lengths=np.array(lengths, np.uint64), offsets=offsets,
-                         hashes=np.concatenate(sketches) if sketches else np.zeros(0, np.uint64))
+    comments = []
+    for g in sketches:
+        first = g.header.decode("utf-8", "replace").strip()
+        if g.n_records > 1:  # Mash's comment convention for multi-record genomes
+            first = "[%d seqs] %s [...]" % (g.n_records, first)
+        comments.append(first)
+    offsets = np.concatenate([[0], np.cumsum([len(g.hashes) for g in sketches])]).astype(np.uint64)
+    db = mshfmt.SketchDB(k=k, s=s, seed=seed, names=list(paths), comments=comments,
+                         lengths=np.array([g.length for g in sketches], np.uint64), offsets=offsets,
+                         hashes=np.concatenate([g.hashes for g in sketches]) if sketches else np.zeros(0, np.uint64))
     out = out or pos[0]
     if not out.endswith(".msh"):
         out += ".msh"

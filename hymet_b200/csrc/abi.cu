@@ -20,6 +20,7 @@
 #include <algorithm>
 #include <atomic>
 #include <chrono>
+#include <condition_variable>
 #include <mutex>
 #include <string>
 #include <thread>
@@ -2385,48 +2386,566 @@ HS_API int hs_stat_batch(uint32_t k, uint64_t set_size, uint64_t n, const uint64
     return HS_OK;
 }
 
+// =============================================================================
+// `mash sketch` of a genome collection (SURVEY.md 8f rank 1)
+// =============================================================================
+// Host threads read, inflate and pack whole files; the calling thread lays the packed genomes out
+// in batches -- every genome on a tile boundary, followed by at least one invalid position -- and
+// hashes a batch with one k_stream launch (MODE 4), each genome into its own set of the distinct
+// hashes <= its threshold tau.  One launch of k_sketch_select then sorts every set.
+//
+// Threshold.  With L = the genome's valid positions (>= its valid k-mers >= its distinct k-mers D),
+// tau = lambda / L of the hash range makes the set expect D * lambda / L <= lambda values, lambda =
+// s + 6 sqrt(s) + 8, and the set takes lambda + 6 sqrt(lambda) + 8 before it overflows (tau = the top
+// of the range, and room for L values, when L is smaller than that).
+// Exactness.  Without overflow the set holds every distinct hash <= tau, so its s smallest are the
+// sketch when it holds >= s of them or when tau is the top of the range.  Otherwise the genome is
+// streamed again with another tau: higher when it held too few (D << L: repeats), lower when it
+// overflowed.  The number of distinct hashes <= tau, N(tau), is monotone in tau.  A genome keeps the
+// largest tau known to give N < s (lo) and the smallest known to overflow (hi, N > limit > s); once
+// both exist the next tau is their midpoint, which lies strictly between them (N(hi) - N(lo) >= 3,
+// and distinct hashes are distinct integers), so the interval shrinks every pass.  Before that, tau
+// only grows (at least x2, to the top at most) or only shrinks (/8, and N(0) <= 1 cannot overflow):
+// the search ends, at the latest, after a few dozen passes.
 namespace {
-// bottom-s of one packed device-resident stream (shared by the two sketch entry points)
-int sketch_device(uint32_t k, uint32_t s_, uint32_t seed, const uint64_t *dseq, const uint32_t *dinv, uint64_t n_bases,
-                  uint64_t *out_hashes, uint32_t *n_out)
-{
-    unsigned long long *dst = nullptr;
-    CU(cudaMalloc((void **)&dst, ST_COUNT * sizeof(unsigned long long)));
-    CU(cudaMemset(dst, 0, ST_COUNT * sizeof(unsigned long long)));
-    MixEngine mix;
-    const bool use64 = pow(4.0, (double)k) > pow(2.0, 32.0);
-    int rc = mix.init(s_, use64);
-    if (rc == HS_OK) rc = mix.reset(0);
-    Chunk c{dseq, dinv, n_bases};
-    auto offer = [&]() -> int {
-        StreamArgs a = base_args(c, k, seed, use64);
-        a.do_mix = 1; a.mix = mix.view(mix.launch_cap(c.n_bases)); a.stats = dst;
-        CU(launch_stream(a, g_sm, 0));
-        CU(launch_mix_maintain(a.mix, 0));
+
+constexpr uint32_t kSketchBatchTiles = 4096;              // 32 M positions, 12 MB of packed words per batch
+constexpr uint64_t kSketchSetWords = (uint64_t)8 << 20;   // 64 MB of sets per batch: L2 holds them while they fill
+constexpr uint32_t kSketchMaxCap = 1u << 24;              // mixset_slot spreads a set over at most 2^24 slots
+constexpr uint64_t kTilePositions = (uint64_t)kTileWords * kBasesPerWord;
+
+// a buffer with a single owner that grows on demand (device memory, or pinned host memory)
+template <class T, bool HOST>
+struct Grow {
+    T *p = nullptr;
+    size_t cap = 0;
+    cudaError_t need(size_t n)
+    {
+        if (n <= cap) return cudaSuccess;
+        release();
+        n = std::max<size_t>(n + n / 2, 64);
+        const cudaError_t e = HOST ? cudaHostAlloc((void **)&p, n * sizeof(T), cudaHostAllocDefault)
+                                   : cudaMalloc((void **)&p, n * sizeof(T));
+        if (e == cudaSuccess) cap = n; else p = nullptr;
+        return e;
+    }
+    void release()
+    {
+        if (p) { if (HOST) cudaFreeHost(p); else cudaFree(p); }
+        p = nullptr; cap = 0;
+    }
+};
+
+// every CUDA resource of a sketcher, released in one place
+struct SketchDev {
+    bool ready = false;
+    cudaStream_t stream = nullptr;
+    cudaEvent_t ev[4] = {};
+    unsigned long long *stats = nullptr;
+    Grow<uint64_t, false> seq, sets, out, out_off;
+    Grow<uint32_t, false> inv, tile_genome, n_out;
+    Grow<SketchSlot, false> slots;
+    Grow<uint64_t, true> h_seq, h_out, h_out_off;
+    Grow<uint32_t, true> h_inv, h_tile_genome, h_n_out;
+    Grow<SketchSlot, true> h_slots;
+    int init()
+    {
+        if (ready) return HS_OK;
+        ready = true;   // from here on release() owns whatever was created
+        CU(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
+        for (auto &e : ev) CU(cudaEventCreate(&e));
+        CU(cudaMalloc((void **)&stats, ST_COUNT * sizeof(unsigned long long)));
+        CU(cudaMemsetAsync(stats, 0, ST_COUNT * sizeof(unsigned long long), stream));
         return HS_OK;
-    };
-    std::vector<uint64_t> out;
-    uint32_t launches = 0;
-    if (rc == HS_OK) rc = offer();
-    if (rc == HS_OK) rc = mix_finalize(mix, 0, out, launches, offer);
-    mix.destroy();
-    cudaFree(dst);
-    if (rc) return rc;
-    *n_out = (uint32_t)out.size();
-    memcpy(out_hashes, out.data(), out.size() * 8);
+    }
+    void release()
+    {
+        if (stream) cudaStreamSynchronize(stream);
+        seq.release(); sets.release(); out.release(); out_off.release(); inv.release(); tile_genome.release();
+        n_out.release(); slots.release(); h_seq.release(); h_out.release(); h_out_off.release(); h_inv.release();
+        h_tile_genome.release(); h_n_out.release(); h_slots.release();
+        cudaFree(stats); stats = nullptr;
+        for (auto &e : ev) { if (e) cudaEventDestroy(e); e = nullptr; }
+        if (stream) cudaStreamDestroy(stream);
+        stream = nullptr;
+        ready = false;
+    }
+};
+
+struct SkInput {
+    std::string path;                    // a file ...
+    const char *text = nullptr;          // ... or text in host memory (hs_sketch_text) ...
+    size_t n = 0;
+    bool packed = false;                 // ... or packed words already copied into the genome (hs_sketch_packed_device)
+};
+
+struct SkGenome {
+    std::vector<uint64_t> seq;           // packed words, kept until the sketch is final (a re-stream needs them)
+    std::vector<uint32_t> inv;
+    uint64_t n_pos = 0, valid = 0, length = 0, n_records = 0;
+    std::string header, err;
+    std::vector<uint64_t> hashes;
+    double t_read = 0, t_pack = 0;
+    uint64_t tau = 0, lo = 0, hi = 0;    // threshold, and the bounds of its search (see above)
+    bool has_lo = false, has_hi = false;
+    uint32_t cap = 0;                    // set slots
+    uint64_t tiles() const { return n_pos / kTilePositions + 1; }   // >= 1 invalid position at the end
+};
+
+}  // namespace
+
+struct hs_sketcher {
+    int device = 0;
+    uint32_t k = 21, s = 1000, seed = 42;
+    bool use64 = true;
+    int threads = 1;
+    bool ran = false;
+    std::vector<SkInput> inputs;
+    std::vector<SkGenome> gen;
+    std::vector<uint32_t> retry;         // genomes whose pass did not settle their sketch
+    hs_sketch_stats_t st{};
+    SketchDev dev;
+    uint64_t top() const { return use64 ? ~0ull : 0xFFFFFFFFull; }
+    double lambda() const { return (double)s + 6.0 * sqrt((double)s) + 8.0; }
+};
+
+namespace {
+
+// read + inflate + pack one input (host thread; no CUDA calls, no hs_last_error)
+void sketch_ingest(SkGenome &g, const SkInput &in)
+{
+    if (in.packed) return;
+    std::vector<char> buf;
+    const char *t = in.text;
+    size_t n = in.n;
+    double t0 = now_s();
+    if (!in.path.empty()) {
+        std::string err;
+        if (!slurp_file(in.path, buf, err)) { g.err = "could not open " + in.path + " for reading."; return; }
+        t = buf.data(); n = buf.size();
+        const double t1 = now_s();
+        g.t_read = t1 - t0;
+        t0 = t1;
+    }
+    // what the .msh comment is made of (cli.py): records = "\n>" count + a leading '>', first header line
+    g.n_records = (n && t[0] == '>') ? 1 : 0;
+    for (const char *p = t; n && (p = (const char *)memmem(p, (size_t)(t + n - p), "\n>", 2)); p += 2) g.n_records++;
+    if (n && t[0] == '>') {
+        const char *nl = (const char *)memchr(t, '\n', n);
+        const size_t end = nl ? (size_t)(nl - t) : n - 1;   // Python's text[1:text.find(b"\n")]
+        if (end > 1) g.header.assign(t + 1, end - 1);
+    }
+    g.seq.resize(pack_words_bound(n));
+    g.inv.resize(pack_words_bound(n));
+    PackStats ps;
+    pack_text_span(t, n, g.seq.data(), g.inv.data(), &ps);
+    const uint64_t words = (ps.n_positions + 31) / 32;
+    g.seq.resize(words); g.inv.resize(words);
+    g.n_pos = ps.n_positions;
+    g.length = ps.n_seq_bases;
+    for (uint32_t w : g.inv) g.valid += 32 - (uint64_t)__builtin_popcount(w);
+    g.t_pack = now_s() - t0;
+}
+
+// first threshold and set size of a genome
+int sketch_plan(hs_sketcher *sk, SkGenome &g)
+{
+    const double lam = sk->lambda(), room = lam + 6.0 * sqrt(lam) + 8.0;
+    uint64_t need;
+    if ((double)g.valid <= room) {
+        g.tau = sk->top();
+        need = g.valid;
+    } else {
+        const long double t = (long double)lam / (long double)g.valid * (sk->use64 ? 18446744073709551616.0L : 4294967296.0L);
+        g.tau = t >= (long double)sk->top() ? sk->top() : (uint64_t)t;
+        need = (uint64_t)ceil(room);
+    }
+    uint64_t cap = 64;
+    while (cap < 2 * need + 2) cap <<= 1;
+    if (cap > kSketchMaxCap) return fail(HS_EUNSUPPORTED, "sketch size too large for a genome of this size");
+    g.cap = (uint32_t)cap;
     return HS_OK;
 }
+
+// the genome's words [w0, w1) into the staging at tile t0, padded with invalid positions to `tiles` tiles
+uint32_t sketch_stage(SketchDev &d, const SkGenome &g, uint64_t w0, uint64_t w1, uint32_t tiles, uint32_t t0, uint32_t slot)
+{
+    uint64_t *sq = d.h_seq.p + (size_t)t0 * kTileWords;
+    uint32_t *iv = d.h_inv.p + (size_t)t0 * kTileWords;
+    memcpy(sq, g.seq.data() + w0, (w1 - w0) * 8);
+    memcpy(iv, g.inv.data() + w0, (w1 - w0) * 4);
+    const size_t pad = (size_t)tiles * kTileWords - (w1 - w0);
+    memset(sq + (w1 - w0), 0, pad * 8);
+    memset(iv + (w1 - w0), 0xFF, pad * 4);
+    for (uint32_t t = 0; t < tiles; t++) d.h_tile_genome.p[t0 + t] = slot;
+    return tiles;
+}
+
+// hash the staged tiles [0, tiles) into the batch's sets
+int sketch_launch(hs_sketcher *sk, uint32_t tiles)
+{
+    SketchDev &d = sk->dev;
+    const size_t words = (size_t)tiles * kTileWords;
+    CU(d.seq.need(words)); CU(d.inv.need(words)); CU(d.tile_genome.need(tiles));
+    CU(cudaMemcpyAsync(d.seq.p, d.h_seq.p, words * 8, cudaMemcpyHostToDevice, d.stream));
+    CU(cudaMemcpyAsync(d.inv.p, d.h_inv.p, words * 4, cudaMemcpyHostToDevice, d.stream));
+    CU(cudaMemcpyAsync(d.tile_genome.p, d.h_tile_genome.p, (size_t)tiles * 4, cudaMemcpyHostToDevice, d.stream));
+    StreamArgs a;
+    memset(&a, 0, sizeof a);
+    a.seq = d.seq.p; a.inv = d.inv.p; a.n_bases = tiles * kTilePositions; a.n_tiles = tiles;
+    a.k = (int)sk->k; a.seed = sk->seed; a.use64 = sk->use64; a.stats = d.stats;
+    a.sk = SketchView{d.tile_genome.p, d.slots.p, d.sets.p};
+    CU(cudaEventRecord(d.ev[0], d.stream));
+    CU(launch_stream(a, g_sm, d.stream));
+    CU(cudaEventRecord(d.ev[1], d.stream));
+    // the staging is refilled next: wait for the copies (and take the kernel time with them)
+    CU(cudaEventSynchronize(d.ev[1]));
+    float ms = 0;
+    CU(cudaEventElapsedTime(&ms, d.ev[0], d.ev[1]));
+    sk->st.ms_stream += ms;
+    sk->st.n_launches++;
+    return HS_OK;
+}
+
+// one batch: genomes ids (all of them fit kSketchBatchTiles, or a single genome streamed piece by piece)
+int sketch_batch(hs_sketcher *sk, const std::vector<uint32_t> &ids)
+{
+    SketchDev &d = sk->dev;
+    const uint32_t n = (uint32_t)ids.size();
+    CU(d.h_slots.need(n)); CU(d.slots.need(n)); CU(d.h_out_off.need(n)); CU(d.out_off.need(n));
+    CU(d.h_n_out.need(n)); CU(d.n_out.need(n));
+    uint64_t set_words = 0, out_words = 0, tiles = 0;
+    uint32_t max_cap = 0;
+    for (uint32_t j = 0; j < n; j++) {
+        const SkGenome &g = sk->gen[ids[j]];
+        SketchSlot &sl = d.h_slots.p[j];
+        memset(&sl, 0, sizeof sl);
+        sl.st.tau = g.tau;
+        sl.set_off = set_words;
+        sl.mask = g.cap - 1; sl.limit = g.cap / 2;
+        d.h_out_off.p[j] = out_words;
+        set_words += g.cap;
+        out_words += std::min<uint64_t>(sk->s, g.cap);
+        max_cap = std::max(max_cap, g.cap);
+        tiles += g.tiles();
+    }
+    CU(d.sets.need(set_words)); CU(d.out.need(out_words)); CU(d.h_out.need(out_words));
+    const uint64_t stage_tiles = std::min<uint64_t>(tiles, kSketchBatchTiles);
+    CU(d.h_seq.need(stage_tiles * kTileWords)); CU(d.h_inv.need(stage_tiles * kTileWords)); CU(d.h_tile_genome.need(stage_tiles));
+    CU(cudaMemcpyAsync(d.slots.p, d.h_slots.p, n * sizeof(SketchSlot), cudaMemcpyHostToDevice, d.stream));
+    CU(cudaMemcpyAsync(d.out_off.p, d.h_out_off.p, n * 8, cudaMemcpyHostToDevice, d.stream));
+    CU(cudaMemsetAsync(d.sets.p, 0xFF, set_words * 8, d.stream));
+    sk->st.n_batches++;
+    if (tiles <= kSketchBatchTiles) {
+        uint32_t t = 0;
+        for (uint32_t j = 0; j < n; j++) {
+            const SkGenome &g = sk->gen[ids[j]];
+            t += sketch_stage(d, g, 0, g.seq.size(), (uint32_t)g.tiles(), t, j);
+        }
+        int rc = sketch_launch(sk, t);
+        if (rc) return rc;
+    } else {
+        // a genome larger than a batch: pieces of one launch each, into the same set.  Each piece after the
+        // first starts one word early: k-mers that end in its second word read their first bases there
+        // (k <= 32), and the k-mers that end in the repeated word were offered before (sets keep one copy).
+        const SkGenome &g = sk->gen[ids[0]];
+        const uint64_t nw = g.seq.size(), piece = (uint64_t)kSketchBatchTiles * kTileWords - 1;
+        for (uint64_t w0 = 0;;) {
+            const uint64_t w1 = std::min(nw, w0 + piece);
+            int rc = sketch_launch(sk, sketch_stage(d, g, w0, w1, (uint32_t)((w1 - w0 + kTileWords - 1) / kTileWords), 0, 0));
+            if (rc) return rc;
+            if (w1 == nw) break;
+            w0 = w1 - 1;
+        }
+    }
+    CU(cudaEventRecord(d.ev[2], d.stream));
+    CU(launch_sketch_select(d.slots.p, n, max_cap, d.sets.p, sk->s, d.out_off.p, d.out.p, d.n_out.p, d.stream));
+    CU(cudaEventRecord(d.ev[3], d.stream));
+    sk->st.n_launches++;
+    CU(cudaMemcpyAsync(d.h_slots.p, d.slots.p, n * sizeof(SketchSlot), cudaMemcpyDeviceToHost, d.stream));
+    CU(cudaMemcpyAsync(d.h_n_out.p, d.n_out.p, n * 4, cudaMemcpyDeviceToHost, d.stream));
+    CU(cudaMemcpyAsync(d.h_out.p, d.out.p, out_words * 8, cudaMemcpyDeviceToHost, d.stream));
+    CU(cudaStreamSynchronize(d.stream));
+    float ms = 0;
+    CU(cudaEventElapsedTime(&ms, d.ev[2], d.ev[3]));
+    sk->st.ms_select += ms;
+    // settle or re-stream each genome (see the argument at the top of this section)
+    const uint64_t top = sk->top();
+    for (uint32_t j = 0; j < n; j++) {
+        SkGenome &g = sk->gen[ids[j]];
+        const MixState &r = d.h_slots.p[j].st;
+        const uint64_t have = (uint64_t)r.count + (r.has_max ? 1 : 0);
+        if (!r.overflow && (have >= sk->s || g.tau == top)) {
+            const uint64_t *h = d.h_out.p + d.h_out_off.p[j];
+            g.hashes.assign(h, h + d.h_n_out.p[j]);
+            if (r.has_max && g.hashes.size() < sk->s) g.hashes.push_back(~0ull);   // hash 2^64-1 (kEmptyKey) is never stored in a set
+            std::vector<uint64_t>().swap(g.seq);
+            std::vector<uint32_t>().swap(g.inv);
+            continue;
+        }
+        if (r.overflow) { g.hi = g.tau; g.has_hi = true; }
+        else { g.lo = g.tau; g.has_lo = true; }
+        if (g.has_lo && g.has_hi) {
+            g.tau = g.lo + (g.hi - g.lo) / 2;
+        } else if (g.has_hi) {
+            g.tau /= 8;
+        } else {
+            const long double f = std::max(2.0L, (long double)sk->lambda() / (long double)std::max<uint32_t>(r.count, 1));
+            const long double t = (long double)g.tau * f + 1.0L;
+            g.tau = t >= (long double)top ? top : (uint64_t)t;
+        }
+        sk->retry.push_back(ids[j]);
+        sk->st.n_passes++;
+    }
+    return HS_OK;
+}
+
+// batch the genomes in `order` (in that order) and sketch them
+template <class Next>
+int sketch_genomes(hs_sketcher *sk, Next &&next)
+{
+    std::vector<uint32_t> cur;
+    uint64_t cur_tiles = 0, cur_sets = 0;
+    auto flush = [&]() -> int {
+        if (cur.empty()) return HS_OK;
+        int rc = sketch_batch(sk, cur);
+        cur.clear(); cur_tiles = 0; cur_sets = 0;
+        return rc;
+    };
+    for (;;) {
+        int64_t i = -1;
+        int rc = next(i);
+        if (rc) return rc;
+        if (i < 0) break;
+        const SkGenome &g = sk->gen[(size_t)i];
+        if (!g.n_pos) continue;   // empty: an empty sketch
+        const uint64_t tg = g.tiles();
+        if (tg > kSketchBatchTiles) {
+            if ((rc = flush()) || (rc = sketch_batch(sk, {(uint32_t)i}))) return rc;
+            continue;
+        }
+        if (cur_tiles + tg > kSketchBatchTiles || (!cur.empty() && cur_sets + g.cap > kSketchSetWords))
+            if ((rc = flush())) return rc;
+        cur.push_back((uint32_t)i);
+        cur_tiles += tg; cur_sets += g.cap;
+    }
+    return flush();
+}
+
+int sketcher_run(hs_sketcher *sk)
+{
+    int rc = sk->dev.init();
+    if (rc) return rc;
+    const size_t n = sk->inputs.size();
+    sk->gen.resize(n);
+    // host threads take whole inputs in order and run at most ~two batches of positions ahead of the GPU
+    const uint64_t ahead_max = 2ull * kSketchBatchTiles * kTilePositions;
+    std::mutex mu;
+    std::condition_variable cv;
+    std::vector<char> ready(n, 0);
+    size_t next_in = 0, consumed = 0;
+    uint64_t ahead = 0;
+    bool stop = false;
+    auto worker = [&]() {
+        for (;;) {
+            size_t i;
+            {
+                std::unique_lock<std::mutex> lk(mu);
+                cv.wait(lk, [&] { return stop || next_in >= n || next_in <= consumed || ahead < ahead_max; });
+                if (stop || next_in >= n) return;
+                i = next_in++;
+            }
+            sketch_ingest(sk->gen[i], sk->inputs[i]);
+            {
+                std::lock_guard<std::mutex> lk(mu);
+                ready[i] = 1;
+                ahead += sk->gen[i].n_pos;
+            }
+            cv.notify_all();
+        }
+    };
+    std::vector<std::thread> pool;
+    for (int t = 0; t < std::min<int>(sk->threads, (int)std::max<size_t>(n, 1)); t++) pool.emplace_back(worker);
+    size_t at = 0;
+    rc = sketch_genomes(sk, [&](int64_t &i) -> int {
+        if (at == n) return HS_OK;
+        const double t0 = now_s();
+        {
+            std::unique_lock<std::mutex> lk(mu);
+            cv.wait(lk, [&] { return ready[at] != 0; });
+            consumed = at + 1;
+            ahead -= sk->gen[at].n_pos;
+        }
+        cv.notify_all();
+        sk->st.t_wait_s += now_s() - t0;
+        SkGenome &g = sk->gen[at];
+        if (!g.err.empty()) return fail(HS_EIO, g.err);
+        if (g.n_pos) {
+            int r = sketch_plan(sk, g);
+            if (r) return r;
+        }
+        i = (int64_t)at++;
+        return HS_OK;
+    });
+    {
+        std::lock_guard<std::mutex> lk(mu);
+        stop = true;
+    }
+    cv.notify_all();
+    for (auto &t : pool) t.join();
+    // re-streams: genomes whose first pass did not settle, batched again with their new thresholds
+    while (rc == HS_OK && !sk->retry.empty()) {
+        std::vector<uint32_t> again;
+        again.swap(sk->retry);
+        size_t r = 0;
+        rc = sketch_genomes(sk, [&](int64_t &i) -> int {
+            i = r < again.size() ? (int64_t)again[r++] : -1;
+            return HS_OK;
+        });
+    }
+    for (const SkGenome &g : sk->gen) {
+        sk->st.n_bases += g.length;
+        sk->st.n_positions += g.n_pos;
+        sk->st.t_read_s += g.t_read;
+        sk->st.t_pack_s += g.t_pack;
+    }
+    sk->st.n_genomes = n;
+    return rc;
+}
+
+int sketcher_new(uint32_t k, uint32_t s_, uint32_t seed, int threads, hs_sketcher **out)
+{
+    if (!out) return fail(HS_EINVAL, "null argument");
+    if (k == 0 || k > 32) return fail(HS_EUNSUPPORTED, "k-mer size must be 1..32");
+    if (s_ == 0) return fail(HS_EINVAL, "sketch size must be positive");
+    NEED_DEVICE();
+    auto *sk = new hs_sketcher();
+    sk->device = g_device;
+    sk->k = k; sk->s = s_; sk->seed = seed;
+    sk->use64 = k > 16;   // 4^k > 2^32: 64-bit hashes (S1)
+    sk->threads = threads < 1 ? 1 : threads;
+    *out = sk;
+    return HS_OK;
+}
+
+// a batch of one, for the single-genome entry points
+int sketch_one(hs_sketcher *sk, uint64_t *out_hashes, uint32_t *n_out, uint64_t *length)
+{
+    sk->ran = true;
+    int rc = sketcher_run(sk);
+    if (rc) return rc;
+    const SkGenome &g = sk->gen[0];
+    *n_out = (uint32_t)g.hashes.size();
+    memcpy(out_hashes, g.hashes.data(), g.hashes.size() * 8);
+    if (length) *length = g.length;
+    return HS_OK;
+}
+
 }  // namespace
+
+HS_API int hs_sketcher_new(uint32_t k, uint32_t s_, uint32_t seed, int host_threads, hs_sketcher **out)
+{
+    return sketcher_new(k, s_, seed, host_threads, out);
+}
+
+HS_API int hs_sketcher_add_file(hs_sketcher *sk, const char *path)
+{
+    if (!sk || !path) return fail(HS_EINVAL, "null argument");
+    if (sk->ran) return fail(HS_ESTATE, "the sketcher has already run");
+    SkInput in;
+    in.path = path;
+    if (in.path.empty()) return fail(HS_EINVAL, "empty path");
+    sk->inputs.push_back(in);
+    return HS_OK;
+}
+
+HS_API int hs_sketcher_run(hs_sketcher *sk)
+{
+    if (!sk) return fail(HS_EINVAL, "null argument");
+    if (sk->ran) return fail(HS_ESTATE, "the sketcher has already run");
+    ON_DEVICE(sk->device);
+    sk->ran = true;
+    const double t0 = now_s();
+    const int rc = sketcher_run(sk);
+    sk->st.t_total_s = now_s() - t0;
+    return rc;
+}
+
+HS_API int hs_sketcher_result(const hs_sketcher *sk, uint64_t i, const uint64_t **hashes, uint32_t *n, uint64_t *length,
+                              uint64_t *n_records, const char **header, uint64_t *header_len)
+{
+    if (!sk) return fail(HS_EINVAL, "null argument");
+    if (!sk->ran || sk->gen.size() != sk->inputs.size()) return fail(HS_ESTATE, "hs_sketcher_run has not completed");
+    if (i >= sk->gen.size()) return fail(HS_EINVAL, "input index out of range");
+    const SkGenome &g = sk->gen[i];
+    if (hashes) *hashes = g.hashes.data();
+    if (n) *n = (uint32_t)g.hashes.size();
+    if (length) *length = g.length;
+    if (n_records) *n_records = g.n_records;
+    if (header) *header = g.header.data();
+    if (header_len) *header_len = g.header.size();
+    return HS_OK;
+}
+
+HS_API int hs_sketcher_stats(const hs_sketcher *sk, hs_sketch_stats_t *stats)
+{
+    if (!sk || !stats) return fail(HS_EINVAL, "null argument");
+    *stats = sk->st;
+    return HS_OK;
+}
+
+HS_API void hs_sketcher_free(hs_sketcher *sk)
+{
+    if (!sk) return;
+    if (sk->dev.ready) {
+        cudaSetDevice(sk->device);
+        sk->dev.release();
+    }
+    delete sk;
+}
 
 HS_API int hs_sketch_packed_device(uint32_t k, uint32_t s_, uint32_t seed, const void *d_seq2, const void *d_inv,
                                    uint64_t n_bases, uint64_t *out_hashes, uint32_t *n_out)
 {
     if (!out_hashes || !n_out || ((!d_seq2 || !d_inv) && n_bases)) return fail(HS_EINVAL, "null argument");
-    if (k == 0 || k > 32) return fail(HS_EUNSUPPORTED, "k-mer size must be 1..32");
-    NEED_DEVICE();
+    hs_sketcher *sk = nullptr;
+    int rc = sketcher_new(k, s_ ? s_ : 1, seed, 1, &sk);
+    if (rc) return rc;
     *n_out = 0;
-    if (!n_bases) return HS_OK;
-    return sketch_device(k, s_, seed, (const uint64_t *)d_seq2, (const uint32_t *)d_inv, n_bases, out_hashes, n_out);
+    SkInput in;
+    in.packed = true;
+    sk->inputs.push_back(in);
+    sk->gen.resize(1);
+    SkGenome &g = sk->gen[0];
+    const uint64_t words = (n_bases + 31) / 32;
+    g.seq.resize(words); g.inv.resize(words);
+    cudaError_t e = cudaMemcpy(g.seq.data(), d_seq2, words * 8, cudaMemcpyDeviceToHost);
+    if (e == cudaSuccess) e = cudaMemcpy(g.inv.data(), d_inv, words * 4, cudaMemcpyDeviceToHost);
+    if (e != cudaSuccess) rc = fail(HS_ECUDA, std::string("copying the packed genome: ") + cudaGetErrorString(e));
+    if (rc == HS_OK) {
+        if (n_bases % 32) g.inv[words - 1] |= (1u << (32 - n_bases % 32)) - 1u;   // positions >= n_bases are not the genome's
+        g.n_pos = n_bases;
+        for (uint32_t w : g.inv) g.valid += 32 - (uint64_t)__builtin_popcount(w);
+        rc = sketch_one(sk, out_hashes, n_out, nullptr);
+    }
+    hs_sketcher_free(sk);
+    return rc;
+}
+
+HS_API int hs_sketch_text(uint32_t k, uint32_t s_, uint32_t seed, const char *text, size_t n, uint64_t *out_hashes,
+                          uint32_t *n_out, uint64_t *length)
+{
+    if ((!text && n) || !out_hashes || !n_out) return fail(HS_EINVAL, "null argument");
+    hs_sketcher *sk = nullptr;
+    int rc = sketcher_new(k, s_ ? s_ : 1, seed, 1, &sk);
+    if (rc) return rc;
+    *n_out = 0;
+    SkInput in;
+    in.text = text; in.n = n;
+    sk->inputs.push_back(in);
+    rc = sketch_one(sk, out_hashes, n_out, length);
+    hs_sketcher_free(sk);
+    return rc;
 }
 
 HS_API int hs_pack_codes_device(const void *d_codes, uint64_t n, void *d_seq2, void *d_inv, void *cuda_stream)
@@ -2436,36 +2955,6 @@ HS_API int hs_pack_codes_device(const void *d_codes, uint64_t n, void *d_seq2, v
     CU(launch_pack_codes((const uint8_t *)d_codes, n, (uint64_t *)d_seq2, (uint32_t *)d_inv, hs_packed_words(n),
                          (cudaStream_t)cuda_stream));
     return HS_OK;
-}
-
-HS_API int hs_sketch_text(uint32_t k, uint32_t s_, uint32_t seed, const char *text, size_t n, uint64_t *out_hashes,
-                          uint32_t *n_out, uint64_t *length)
-{
-    if ((!text && n) || !out_hashes || !n_out) return fail(HS_EINVAL, "null argument");
-    if (k == 0 || k > 32) return fail(HS_EUNSUPPORTED, "k-mer size must be 1..32");
-    NEED_DEVICE();
-    std::vector<uint64_t> seq(pack_words_bound(n));
-    std::vector<uint32_t> inv(pack_words_bound(n));
-    PackStats ps;
-    pack_text_span(text, n, seq.data(), inv.data(), &ps);
-    if (length) *length = ps.n_seq_bases;
-    *n_out = 0;
-    if (!ps.n_positions) return HS_OK;
-    const uint64_t words = (ps.n_positions + 31) / 32, alloc = hs_packed_words(ps.n_positions);
-    uint64_t *dseq = nullptr;
-    uint32_t *dinv = nullptr;
-    unsigned long long *dst = nullptr;
-    CU(cudaMalloc((void **)&dseq, alloc * 8));
-    CU(cudaMalloc((void **)&dinv, alloc * 4));
-    CU(cudaMalloc((void **)&dst, ST_COUNT * sizeof(unsigned long long)));
-    CU(cudaMemset(dseq, 0, alloc * 8));
-    CU(cudaMemset(dinv, 0xFF, alloc * 4));
-    CU(cudaMemset(dst, 0, ST_COUNT * sizeof(unsigned long long)));
-    CU(cudaMemcpy(dseq, seq.data(), words * 8, cudaMemcpyHostToDevice));
-    CU(cudaMemcpy(dinv, inv.data(), words * 4, cudaMemcpyHostToDevice));
-    int rc = sketch_device(k, s_, seed, dseq, dinv, ps.n_positions, out_hashes, n_out);
-    cudaFree(dseq); cudaFree(dinv); cudaFree(dst);
-    return rc;
 }
 
 // =============================================================================

@@ -393,11 +393,12 @@ constexpr int kIlp = 4;   // k-mers hashed side by side per thread (measured, ms
 // MODE: 0 = screen, 1 = K1 parity (emit every hash), 2 = screen with the Bloom reads of a group of
 // kIlp k-mers issued together (databases with keys above the dense range), 3 = screen that probes for
 // (nearly) every k-mer: the warp looks its hashes up cooperatively (coop_probe), control flow stays
-// warp-uniform and the CTA may use twice the registers (the kernel waits on HBM, not on issue slots)
+// warp-uniform and the CTA may use twice the registers (the kernel waits on HBM, not on issue slots),
+// 4 = `mash sketch` of a batch of genomes: each word's gate and set are its genome's (SketchView)
 template <int KT, int MODE>
 __global__ void __launch_bounds__(stream_threads(MODE), MODE == 3 ? 3 : 2) k_stream(const StreamArgs a)
 {
-    constexpr bool EMIT = MODE == 1, BLOOMB = MODE == 2, COOP = MODE == 3;
+    constexpr bool EMIT = MODE == 1, BLOOMB = MODE == 2, COOP = MODE == 3, SKETCH = MODE == 4;
     constexpr bool kTailTab = stream_tail_table(KT, MODE);
     using Lay = StreamLayout<KT, MODE>;
     // one word per thread: a stage of the ring holds kSpan consecutive tiles of the chunk
@@ -540,6 +541,45 @@ __global__ void __launch_bounds__(stream_threads(MODE), MODE == 3 ? 3 : 2) k_str
             icur |= nv ? ((1u << (32 - nv)) - 1u) : ~0u;
         }
         if (!COOP && icur == ~0u) continue;  // padding / all-N word: no k-mer ends here (COOP: every lane stays for the warp's lookups)
+        if constexpr (SKETCH) {
+            // the word's genome: its own threshold and set (the batch layout keeps every k-mer inside one genome)
+            SketchSlot *gs = a.sk.slots + __ldg(a.sk.tile_genome + tile + tid / kTileWords);
+            MixView v{};
+            v.mask = gs->mask; v.limit = gs->limit; v.st = &gs->st;
+            uint64_t *set = a.sk.sets + gs->set_off;
+            const uint64_t tau = __ldcg(&gs->st.tau);
+            // 64-bit hashes: the high-word gate of kmer_core.cuh, whose bound holds for any gate
+            const uint32_t bound = hi_gate_bound(tau);
+            const uint32_t ok = ~invalid_kmer_ends(iprev, icur, k);
+            n_valid += (uint32_t)__popc(ok);
+            const Win w = win_init_top(prev, cur, k);
+#pragma unroll 1
+            for (int half = 0; half < 2; half++) {
+                const uint32_t fa = half ? w.f0 : w.f1, fb = half ? w.f1 : w.f2, fc = half ? w.f2 : w.f3;
+                const uint32_t ra = half ? w.r1 : w.r0, rb = half ? w.r2 : w.r1, rc = half ? w.r3 : w.r2;
+#pragma unroll 1
+                for (int q = 0; q < 16; q += kIlp) {
+                    uint32_t pass = 0;
+#pragma unroll
+                    for (int u = 0; u < kIlp; u++) {
+                        const MurmurState ms = murmur_state_premul_top(canonical_top_half(fa, fb, fc, ra, rb, rc, q + u), k, a.seed, L);
+                        const bool may = use64 ? hi_gate_may_pass(murmur_finish_hi_floor(ms), bound)
+                                               : (murmur_finish(ms) & 0xFFFFFFFFull) <= tau;
+                        pass |= (uint32_t)(may && ((ok >> (31 - (half * 16 + q + u))) & 1u)) << u;
+                    }
+#pragma unroll 1
+                    for (; pass; pass &= pass - 1u) {
+                        const int u = __ffs(pass) - 1;
+                        const uint64_t h = hash_canonical_premul_top(canonical_top_half(fa, fb, fc, ra, rb, rc, q + u), k, a.seed, use64, L);
+                        if (h <= tau) {
+                            n_mix++;
+                            mix_insert(v, set, h);
+                        }
+                    }
+                }
+            }
+            continue;
+        }
 
         auto sink = [&](int j, uint64_t h, uint32_t bloom_word) {
             if (EMIT) {
@@ -756,6 +796,13 @@ static cudaError_t launch_stream_t(const StreamArgs &a, int sm_count, cudaStream
 cudaError_t launch_stream(const StreamArgs &a, int sm_count, cudaStream_t st)
 {
     if (a.emit_hash) return launch_stream_t<0, 1>(a, sm_count, st);   // parity runs: generic-k instantiation
+    if (a.sk.slots) {
+        switch (a.k) {
+        case 21: return launch_stream_t<21, 4>(a, sm_count, st);
+        case 31: return launch_stream_t<31, 4>(a, sm_count, st);
+        default: return launch_stream_t<0, 4>(a, sm_count, st);
+        }
+    }
     if (a.probe_all && a.do_count) {
         switch (a.k) {
         case 21: return launch_stream_t<21, 3>(a, sm_count, st);
@@ -1128,6 +1175,39 @@ cudaError_t launch_sort_unique(uint64_t *data, uint32_t n, uint64_t *scratch, ui
     const bool in_smem = n_pad <= kSortSmemMax;
     k_sort_unique<<<1, 1024, in_smem ? n_pad * sizeof(uint64_t) : 0, st>>>(data, n, nullptr, n_pad, in_smem ? nullptr : scratch,
                                                                           n_unique);
+    return cudaGetLastError();
+}
+
+// ---- `mash sketch`: the s smallest of every genome of a batch ------------------------
+// The set of a genome holds exactly its distinct hashes <= tau (when it did not overflow) and kEmptyKey in
+// its free slots, which sorts last: sorting the whole set (a power of two) puts the answer at the front.
+__global__ void __launch_bounds__(1024) k_sketch_select(const SketchSlot *slots, uint64_t *sets, uint32_t s,
+                                                        const uint64_t *out_off, uint64_t *out, uint32_t *n_out)
+{
+    extern __shared__ uint64_t sm[];
+    const SketchSlot &g = slots[blockIdx.x];
+    const uint32_t cap = g.mask + 1u;
+    uint64_t *set = sets + g.set_off;
+    uint64_t *w = cap <= kSortSmemMax ? sm : set;
+    if (w == sm)
+        for (uint32_t i = threadIdx.x; i < cap; i += blockDim.x) sm[i] = set[i];
+    __syncthreads();
+    bitonic_sort_block(w, cap);
+    const uint32_t keep = min(s, min(g.st.count, cap));
+    for (uint32_t i = threadIdx.x; i < keep; i += blockDim.x) out[out_off[blockIdx.x] + i] = w[i];
+    if (threadIdx.x == 0) n_out[blockIdx.x] = keep;
+}
+
+cudaError_t launch_sketch_select(const SketchSlot *slots, uint32_t n_slots, uint32_t max_cap, uint64_t *sets, uint32_t s,
+                                 const uint64_t *out_off, uint64_t *out, uint32_t *n_out, cudaStream_t st)
+{
+    if (!n_slots) return cudaSuccess;
+    // (per call: the attribute belongs to the current device's context, and it costs no device work)
+    cudaError_t e = cudaFuncSetAttribute(k_sketch_select, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                         (int)(kSortSmemMax * sizeof(uint64_t)));
+    if (e != cudaSuccess) return e;
+    const uint32_t smem = (max_cap < kSortSmemMax ? max_cap : kSortSmemMax) * (uint32_t)sizeof(uint64_t);
+    k_sketch_select<<<n_slots, 1024, smem, st>>>(slots, sets, s, out_off, out, n_out);
     return cudaGetLastError();
 }
 

@@ -74,6 +74,21 @@ struct MixView {
     MixState *st;
 };
 
+// `mash sketch` of many genomes in one launch (k_stream MODE 4).  Every genome starts on a tile
+// boundary of the batch and ends with at least one invalid position, so no k-mer spans two genomes,
+// and tile_genome[] names each tile's genome.  A genome's set holds the distinct hashes <= its own
+// threshold st.tau; mix_insert sees st (count, overflow, has_max) as it sees the mixture's.
+struct SketchSlot {
+    MixState st;
+    uint64_t set_off;       // its set: SketchView::sets + set_off, mask + 1 slots (a power of two)
+    uint32_t mask, limit;   // limit: distinct values before `overflow` is raised
+};
+struct SketchView {
+    const uint32_t *tile_genome;   // slot index of every tile of the launch
+    SketchSlot *slots;             // NULL: not a sketch launch
+    uint64_t *sets;
+};
+
 struct StreamArgs {
     const uint64_t *seq;    // packed words (16-byte aligned), n_tiles * kTileWords allocated
     const uint32_t *inv;
@@ -95,6 +110,7 @@ struct StreamArgs {
     uint64_t *emit_hash;    // optional: per position hash (K1 parity), n_bases entries
     uint8_t *emit_valid;
     int probe_all;          // (nearly) every k-mer probes: use the warp-cooperative instantiation
+    SketchView sk;          // sk.slots set: per-genome bottom-s sets, nothing else (do_count = do_mix = 0)
 };
 
 // ---- streaming (K1+K2+K3 insert) -------------------------------------------
@@ -134,6 +150,10 @@ cudaError_t launch_mix_select(const MixView &v, uint32_t s, bool use64, uint32_t
                               uint32_t n_pad, uint64_t *scratch, cudaStream_t st);
 // sort ascending + unique in place (n <= cap_pow2 handled by padding); *n_unique out
 cudaError_t launch_sort_unique(uint64_t *data, uint32_t n, uint64_t *scratch, uint32_t *n_unique, cudaStream_t st);
+// one CTA per genome of a sketch batch: sort its set and write its min(s, count) smallest values to
+// out + out_off[g], the number to n_out[g].  Sets larger than the shared-memory sort are sorted in place.
+cudaError_t launch_sketch_select(const SketchSlot *slots, uint32_t n_slots, uint32_t max_cap, uint64_t *sets, uint32_t s,
+                                 const uint64_t *out_off, uint64_t *out, uint32_t *n_out, cudaStream_t st);
 
 // ---- per-sketch reduction (K4), winner-take-all (K5), statistics (K6) ---------
 // DENSE forms (O(stored hashes)): the fallback when the touched list overflowed or counts wrapped

@@ -9,6 +9,7 @@ method names follow the stages Mash prints on stderr (S20): load, stream, sum sh
 from __future__ import annotations
 
 import ctypes as C
+import os
 from dataclasses import dataclass
 from typing import List, Optional, Sequence
 
@@ -411,6 +412,39 @@ def sketch_text(text: bytes, k: int, s: int, seed: int = 42, device: int = 0):
     n = C.c_uint32(); ln = C.c_uint64()
     check(_abi.load().hs_sketch_text(k, s, seed, text, len(text), _ptr(out, C.c_uint64), C.byref(n), C.byref(ln)))
     return out[:n.value].copy(), int(ln.value)
+
+
+@dataclass
+class GenomeSketch:
+    """One input of `sketch_files`: what its .msh entry is made of."""
+    hashes: np.ndarray     # uint64, ascending, <= s
+    length: int            # sequence bases
+    n_records: int         # occurrences of "\n>" plus one if the text starts with '>'
+    header: bytes          # first header line after its '>' (empty unless the text starts with '>')
+
+
+def sketch_files(paths: Sequence[str], k: int, s: int, seed: int = 42, threads: int = 1, device: int = 0):
+    """`mash sketch` of a collection: one sketch per file (plain or gzip FASTA/FASTQ), many genomes per
+    kernel pass, `threads` host threads reading and packing.  Returns ([GenomeSketch] in input order, stats)."""
+    _abi.init(device)
+    L = _abi.load()
+    h = C.c_void_p()
+    check(L.hs_sketcher_new(k, s, seed, threads, C.byref(h)))
+    try:
+        for p in paths:
+            check(L.hs_sketcher_add_file(h, os.fsencode(p)))
+        check(L.hs_sketcher_run(h))
+        out = []
+        hp, n, ln, nrec, hdr, hl = _abi.u64p(), C.c_uint32(), C.c_uint64(), C.c_uint64(), C.c_void_p(), C.c_uint64()
+        for i in range(len(paths)):
+            check(L.hs_sketcher_result(h, i, C.byref(hp), C.byref(n), C.byref(ln), C.byref(nrec), C.byref(hdr), C.byref(hl)))
+            hashes = np.ctypeslib.as_array(hp, shape=(n.value,)).copy() if n.value else np.zeros(0, np.uint64)
+            out.append(GenomeSketch(hashes, int(ln.value), int(nrec.value), C.string_at(hdr, hl.value) if hl.value else b""))
+        st = _abi.SketchStats()
+        check(L.hs_sketcher_stats(h, C.byref(st)))
+        return out, st.asdict()
+    finally:
+        L.hs_sketcher_free(h)
 
 
 def gather_bench(d_buf_ptr: int, nbytes: int, n_reads: int) -> float:

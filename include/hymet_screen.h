@@ -271,8 +271,42 @@ int hs_db_entry_ids(hs_db *db, uint32_t *out);
 /* K6 alone (rows a14/a15). */
 int hs_stat_batch(uint32_t k, uint64_t set_size, uint64_t n, const uint64_t *shared, const uint64_t *size,
                   double *identity, double *pvalue);
-/* `mash sketch` of one genome held as FASTA text: s smallest distinct hashes
- * (SURVEY.md 8f rank 1; reuses K1 + the mixture bottom-s machinery). */
+/* ---- `mash sketch` of a genome collection (SURVEY.md 8f rank 1) ------------------------------------
+ * One sketch per input file: the s smallest distinct canonical k-mer hashes of all its records.
+ * host_threads threads each take whole files (plain or gzip FASTA/FASTQ), inflate and pack them while
+ * the GPU hashes the previous batch; a batch holds many genomes and one kernel pass gives each its own
+ * bottom-s set.  Results come back in the order the files were added. */
+typedef struct hs_sketcher hs_sketcher;
+typedef struct {
+    uint64_t n_genomes;      /* inputs sketched */
+    uint64_t n_bases;        /* sequence bases of all inputs */
+    uint64_t n_positions;    /* packed positions hashed by first passes (bases + record separators) */
+    uint32_t n_batches;      /* batches sent to the GPU, re-stream batches included */
+    uint32_t n_launches;     /* kernels launched */
+    uint32_t n_passes;       /* genome re-streams the exactness check asked for (threshold raised or lowered) */
+    float ms_stream;         /* device time of the hashing launches (CUDA events) */
+    float ms_select;         /* device time of the per-genome selections */
+    double t_read_s;         /* host thread-seconds reading and inflating files */
+    double t_pack_s;         /* host thread-seconds packing text */
+    double t_wait_s;         /* time the GPU-feeding thread waited for packed genomes */
+    double t_total_s;        /* wall clock of hs_sketcher_run */
+} hs_sketch_stats_t;
+
+/* k 1..32, s >= 1; host_threads < 1 means 1. */
+int hs_sketcher_new(uint32_t k, uint32_t s, uint32_t seed, int host_threads, hs_sketcher **out);
+/* Queue one file; it is read by hs_sketcher_run (HS_EIO there if it cannot be read). */
+int hs_sketcher_add_file(hs_sketcher *sk, const char *path);
+/* Sketch everything queued.  Once per handle. */
+int hs_sketcher_run(hs_sketcher *sk);
+/* Input i after run: n ascending hashes (owned by the handle), total sequence length, record count
+ * (occurrences of "\n>" plus one if the text starts with '>') and the bytes of the first header line
+ * after its '>' (empty unless the text starts with '>'; not NUL-terminated: header_len bytes). */
+int hs_sketcher_result(const hs_sketcher *sk, uint64_t i, const uint64_t **hashes, uint32_t *n, uint64_t *length,
+                       uint64_t *n_records, const char **header, uint64_t *header_len);
+int hs_sketcher_stats(const hs_sketcher *sk, hs_sketch_stats_t *stats);
+void hs_sketcher_free(hs_sketcher *sk);
+
+/* `mash sketch` of one genome held as FASTA text: s smallest distinct hashes (a sketcher batch of one). */
 int hs_sketch_text(uint32_t k, uint32_t s, uint32_t seed, const char *text, size_t n, uint64_t *out_hashes,
                    uint32_t *n_out, uint64_t *length);
 
