@@ -100,15 +100,12 @@ SIGNATURES = {
     "hs_screen_flush": (C.c_int, [C.c_void_p]),
     "hs_screen_flush_async": (C.c_int, [C.c_void_p]),
     "hs_screen_counts_devptr": (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p), u64p]),
-    "hs_screen_counts_compact": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, u32p]),
     "hs_screen_counts_compact_async": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p]),
-    "hs_screen_counts_scatter_add": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64]),
     "hs_screen_counts_absorb": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32]),
-    "hs_screen_absorb_screen": (C.c_int, [C.c_void_p, C.c_void_p]),
+    "hs_screen_absorb_screens": (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p), C.c_uint32]),
     "hs_screen_mixture_get": (C.c_int, [C.c_void_p, u64p, u32p]),
     "hs_screen_mixture_record": (C.c_int, [C.c_void_p, C.c_void_p]),
     "hs_screen_mixture_merge_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32]),
-    "hs_screen_mixture_merge": (C.c_int, [C.c_void_p, u64p, C.c_uint32]),
     "hs_screen_segment_set_size": (C.c_int, [C.c_void_p, C.c_uint32, u64p]),
     "hs_screen_finish": (C.c_int, [C.c_void_p, C.c_int, u64p, u32p, f64p, f64p, C.POINTER(Stats)]),
     "hs_screen_finish_hits": (C.c_int, [C.c_void_p, C.c_int, u32p, C.POINTER(Stats)]),

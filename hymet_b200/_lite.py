@@ -127,9 +127,10 @@ class LiteScreen:
     def feed_fasta_range(self, path: str, begin: int, end: int, threads: int):
         check(_abi.load().hs_screen_feed_fasta_range(self._h, path.encode(), begin, end, threads))
 
-    def absorb(self, other: "LiteScreen"):
-        """Add another GPU's counts and mixture (both flushed) into this screen."""
-        check(_abi.load().hs_screen_absorb_screen(self._h, other._h))
+    def absorb(self, others: List["LiteScreen"]):
+        """Add other GPUs' counts and mixtures (all flushed) into this screen, in one call."""
+        arr = (C.c_void_p * len(others))(*[o._h.value for o in others])
+        check(_abi.load().hs_screen_absorb_screens(self._h, arr, len(others)))
 
     def set_option(self, key: str, value: int):
         check(_abi.load().hs_screen_set_option(self._h, key.encode(), int(value)))
@@ -270,9 +271,10 @@ class MultiGpu:
         for e in errs:
             if e is not None:
                 raise e
-        for i in range(1, n):
-            scrs[0].absorb(scrs[i])
-            scrs[i].close()
+        if n > 1:
+            scrs[0].absorb(scrs[1:])
+        for scr in scrs[1:]:
+            scr.close()
         return scrs[0]
 
 

@@ -1728,19 +1728,6 @@ HS_API int hs_screen_counts_devptr(hs_screen *s, void **d_counts, uint64_t *n)
     return HS_OK;
 }
 
-HS_API int hs_screen_counts_compact(hs_screen *s, void *d_pairs, uint32_t cap, uint32_t *n)
-{
-    if (!s || !d_pairs || !n) return fail(HS_EINVAL, "null argument");
-    ON_DEVICE(s->db->device);
-    if (!s->flushed) return fail(HS_ESTATE, "call hs_screen_flush first");
-    uint32_t *d_n = s->mix.field(offsetof(MixState, n_out));   // free scratch word once the mixture is settled
-    int rc = hs_screen_counts_compact_async(s, d_pairs, cap, d_n);
-    if (rc) return rc;
-    CU(cudaMemcpyAsync(n, d_n, sizeof(uint32_t), cudaMemcpyDeviceToHost, s->stream));
-    CU(cudaStreamSynchronize(s->stream));
-    return HS_OK;
-}
-
 HS_API int hs_screen_counts_compact_async(hs_screen *s, void *d_pairs, uint32_t cap, void *d_n_out)
 {
     if (!s || !d_pairs || !d_n_out) return fail(HS_EINVAL, "null argument");
@@ -1752,17 +1739,6 @@ HS_API int hs_screen_counts_compact_async(hs_screen *s, void *d_pairs, uint32_t 
     if (!s->touched_valid) sp.touched = nullptr;
     CU(launch_counts_compact(sp, s->d_counts, s->db->n_entries, (unsigned long long *)d_pairs, cap, (uint32_t *)d_n_out, s->stream));
     s->st.n_launches += sp.touched ? 2 : 1;
-    return HS_OK;
-}
-
-HS_API int hs_screen_counts_scatter_add(hs_screen *s, const void *d_pairs, uint64_t n_pairs)
-{
-    if (!s || (!d_pairs && n_pairs)) return fail(HS_EINVAL, "null argument");
-    ON_DEVICE(s->db->device);
-    SparseView sp = sparse_view(s);
-    if (!s->touched_valid) sp.touched = nullptr;
-    CU(launch_counts_scatter_add(sp, s->d_counts, s->db->n_entries, (const unsigned long long *)d_pairs, n_pairs, s->stream));
-    s->st.n_launches++;
     return HS_OK;
 }
 
@@ -1778,57 +1754,106 @@ HS_API int hs_screen_counts_absorb(hs_screen *s, const void *d_rows, uint32_t n_
     return HS_OK;
 }
 
-HS_API int hs_screen_absorb_screen(hs_screen *dst, hs_screen *src)
+namespace {
+
+// [length | s hashes, zero padded]: a settled mixture (<= s values) as one row of the mixture merge
+void mixture_row(const hs_screen *s, uint64_t *row)
 {
-    if (!dst || !src || dst == src) return fail(HS_EINVAL, "two different screens are needed");
-    if (!dst->flushed || !src->flushed) return fail(HS_ESTATE, "flush both screens first");
-    if (dst->db->n_entries != src->db->n_entries || dst->db->k != src->db->k || dst->db->s != src->db->s)
-        return fail(HS_EINVAL, "the two screens are not over the same sketch database");
-    // src's non-zero counts as (entry id, count) pairs on ITS device, copied device to device (NVLink peer
-    // copy when the GPUs are peers), added on dst's device: the in-process form of the multi-GPU exchange
-    const uint64_t E = src->db->n_entries;
-    ON_DEVICE(src->db->device);
-    uint32_t n = 0;
-    unsigned long long *sp = nullptr, *dp = nullptr;
-    {
-        uint32_t *d_n = src->mix.field(offsetof(MixState, n_out));
-        CU(cudaMemcpyAsync(src->h_sparse, src->d_sparse, sizeof(SparseState), cudaMemcpyDeviceToHost, src->stream));
-        CU(cudaStreamSynchronize(src->stream));
-        const bool listed = src->sparse_enabled && src->touched_valid && src->h_sparse->n_touched <= src->touched_cap;
-        const uint64_t cap = listed ? src->h_sparse->n_touched : E;
-        if (cap) {
-            CU(cudaMalloc((void **)&sp, cap * 8));
-            int rc = hs_screen_counts_compact_async(src, sp, (uint32_t)cap, d_n);
-            if (rc) { cudaFree(sp); return rc; }
-            CU(cudaMemcpyAsync(&n, d_n, sizeof n, cudaMemcpyDeviceToHost, src->stream));
-            CU(cudaStreamSynchronize(src->stream));
-        }
+    const size_t n = s->mixture.size();
+    memset(row, 0, ((size_t)s->db->s + 1) * 8);
+    row[0] = n;
+    if (n) memcpy(row + 1, s->mixture.data(), n * 8);
+}
+
+// what hs_screen_mixture_merge_device left in h_sparse / h_mixture becomes the screen's mixture
+void adopt_merged_mixture(hs_screen *s)
+{
+    const uint32_t nm = std::min<uint32_t>(s->h_sparse->n_mix, s->db->s);
+    s->mixture.assign(s->h_mixture, s->h_mixture + nm);
+    s->st.n_mixture = nm;
+    s->st.set_size = s->h_sparse->set_size[0];
+}
+
+}  // namespace
+
+HS_API int hs_screen_absorb_screens(hs_screen *dst, hs_screen *const *src, uint32_t n_src)
+{
+    // every check before any device work: a refused call leaves every handle as it was
+    if (!dst || !src || !n_src) return fail(HS_EINVAL, "a screen and at least one source are needed");
+    for (uint32_t i = 0; i < n_src; i++) {
+        if (!src[i] || src[i] == dst) return fail(HS_EINVAL, "every source must be a screen other than dst");
+        for (uint32_t j = 0; j < i; j++)
+            if (src[j] == src[i]) return fail(HS_EINVAL, "a source is listed twice: it would be counted twice");
     }
-    int rc = HS_OK;
-    if (n) {
-        if (cudaSetDevice(dst->db->device) != cudaSuccess || cudaMalloc((void **)&dp, (size_t)n * 8) != cudaSuccess) {
-            cudaSetDevice(src->db->device); cudaFree(sp);
-            return fail(HS_ECUDA, "allocation for the pair exchange failed");
-        }
-        cudaError_t e = cudaMemcpyPeerAsync(dp, dst->db->device, sp, src->db->device, (size_t)n * 8, dst->stream);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(dst->stream);
-        if (e != cudaSuccess) rc = fail(HS_ECUDA, std::string("peer copy of the count pairs: ") + cudaGetErrorString(e));
-        if (rc == HS_OK) rc = hs_screen_counts_scatter_add(dst, dp, n);
-        if (rc == HS_OK && cudaStreamSynchronize(dst->stream) != cudaSuccess) rc = fail(HS_ECUDA, "scatter-add of the count pairs failed");
-        cudaFree(dp);
+    if (dst->mixture_on_device) return fail(HS_ESTATE, "this screen has already absorbed others; call hs_screen_reset first");
+    if (!dst->flushed) return fail(HS_ESTATE, "flush every screen first");
+    const hs_db *db = dst->db;
+    for (uint32_t i = 0; i < n_src; i++) {
+        const hs_screen *s = src[i];
+        if (!s->flushed) return fail(HS_ESTATE, "flush every screen first");
+        if (s->mixture_on_device) return fail(HS_ESTATE, "a source has merged mixtures on the device: its own is stale");
+        if (s->db->n_entries != db->n_entries || s->db->k != db->k || s->db->s != db->s || s->db->seg_s.size() != db->seg_s.size())
+            return fail(HS_EINVAL, "the screens are not over the same sketch database");
     }
-    cudaSetDevice(src->db->device);
-    cudaFree(sp);
-    if (rc) return rc;
-    rc = hs_screen_mixture_merge(dst, src->mixture.data(), (uint32_t)src->mixture.size());
-    if (rc) return rc;
-    dst->st.n_bases += src->st.n_bases; dst->st.n_records += src->st.n_records; dst->st.n_positions += src->st.n_positions;
-    dst->st.n_valid_kmers += src->st.n_valid_kmers; dst->st.n_probes += src->st.n_probes;
-    dst->st.n_bucket_reads += src->st.n_bucket_reads; dst->st.n_hits += src->st.n_hits;
-    dst->st.n_mix_inserts += src->st.n_mix_inserts; dst->st.h2d_bytes += src->st.h2d_bytes;
-    dst->st.n_launches += src->st.n_launches;
-    dst->st.ms_stream = std::max(dst->st.ms_stream, src->st.ms_stream);
-    return HS_OK;
+    // The distributed exchange with peer copies instead of the all-gather: each source's pair record
+    // [n | (entry id << 32 | count) ...] is built on its own device, copied into row 1 + i of a buffer on
+    // dst's device (row 0, dst's own, is empty and skipped), and hs_screen_counts_absorb and
+    // hs_screen_mixture_merge_device take it from there.
+    std::vector<unsigned long long *> rec(n_src, nullptr);
+    unsigned long long *rows = nullptr;
+    const int rc = [&]() -> int {
+        std::vector<uint32_t> n(n_src);
+        uint32_t cap = 1;
+        for (uint32_t i = 0; i < n_src; i++) {
+            hs_screen *s = src[i];
+            ON_DEVICE(s->db->device);
+            CU(cudaMemcpyAsync(s->h_sparse, s->d_sparse, sizeof(SparseState), cudaMemcpyDeviceToHost, s->stream));
+            CU(cudaStreamSynchronize(s->stream));
+            const bool listed = s->sparse_enabled && s->touched_valid && s->h_sparse->n_touched <= s->touched_cap;
+            const uint64_t rcap = listed ? s->h_sparse->n_touched : db->n_entries;
+            CU(cudaMalloc((void **)&rec[i], (rcap + 1) * 8));
+            CU(cudaMemsetAsync(rec[i], 0, 8, s->stream));
+            int r = hs_screen_counts_compact_async(s, rec[i] + 1, (uint32_t)rcap, rec[i]);
+            if (r) return r;
+            CU(cudaMemcpyAsync(&n[i], rec[i], sizeof(uint32_t), cudaMemcpyDeviceToHost, s->stream));
+            CU(cudaStreamSynchronize(s->stream));
+            cap = std::max(cap, n[i]);
+        }
+        ON_DEVICE(db->device);
+        const size_t R = (size_t)n_src + 1, stride = (size_t)cap + 1, mstride = (size_t)db->s + 1;
+        CU(cudaMalloc((void **)&rows, R * (stride + mstride) * 8));
+        unsigned long long *mix = rows + R * stride;
+        CU(cudaMemsetAsync(rows, 0, 8, dst->stream));
+        for (uint32_t i = 0; i < n_src; i++)
+            CU(cudaMemcpyPeerAsync(rows + (i + 1) * stride, db->device, rec[i], src[i]->db->device, ((size_t)n[i] + 1) * 8,
+                                   dst->stream));
+        std::vector<uint64_t> h_mix(R * mstride);
+        mixture_row(dst, h_mix.data());
+        for (uint32_t i = 0; i < n_src; i++) mixture_row(src[i], h_mix.data() + (i + 1) * mstride);
+        CU(cudaMemcpyAsync(mix, h_mix.data(), h_mix.size() * 8, cudaMemcpyHostToDevice, dst->stream));
+        int r = hs_screen_counts_absorb(dst, rows, (uint32_t)R, cap, 0);
+        if (!r) r = hs_screen_mixture_merge_device(dst, mix, (uint32_t)R);
+        if (r) return r;
+        // the merged mixture and its set size now, as for a single screen after flush (stats read before finish)
+        CU(cudaMemcpyAsync(dst->h_sparse, dst->d_sparse, sizeof(SparseState), cudaMemcpyDeviceToHost, dst->stream));
+        if (db->s) CU(cudaMemcpyAsync(dst->h_mixture, dst->d_mixture, (size_t)db->s * 8, cudaMemcpyDeviceToHost, dst->stream));
+        CU(cudaStreamSynchronize(dst->stream));
+        adopt_merged_mixture(dst);
+        for (uint32_t i = 0; i < n_src; i++) {
+            const hs_stats_t &t = src[i]->st;
+            dst->st.n_bases += t.n_bases; dst->st.n_records += t.n_records; dst->st.n_positions += t.n_positions;
+            dst->st.n_valid_kmers += t.n_valid_kmers; dst->st.n_probes += t.n_probes;
+            dst->st.n_bucket_reads += t.n_bucket_reads; dst->st.n_hits += t.n_hits;
+            dst->st.n_mix_inserts += t.n_mix_inserts; dst->st.h2d_bytes += t.h2d_bytes;
+            dst->st.n_launches += t.n_launches;
+            dst->st.ms_stream = std::max(dst->st.ms_stream, t.ms_stream);
+        }
+        return HS_OK;
+    }();
+    if (rows && cudaSetDevice(db->device) == cudaSuccess) cudaFree(rows);
+    for (uint32_t i = 0; i < n_src; i++)
+        if (rec[i] && cudaSetDevice(src[i]->db->device) == cudaSuccess) cudaFree(rec[i]);
+    return rc;
 }
 
 HS_API int hs_screen_mixture_get(hs_screen *s, uint64_t *hashes, uint32_t *n)
@@ -1853,14 +1878,10 @@ HS_API int hs_screen_mixture_record(hs_screen *s, void *d_record)
         return HS_OK;
     }
     if (!s->flushed) return fail(HS_ESTATE, "call hs_screen_flush first");
-    // [length | s hashes, zero padded]: what every rank contributes to the mixture all-gather.  The
-    // settled local mixture is <= s values; it goes up from pinned memory on the screen's stream and
-    // the record stays on the device for the collective.
-    const size_t n = s->mixture.size(), words = (size_t)s->db->s + 1;
-    memset(s->h_mixture, 0, words * 8);
-    s->h_mixture[0] = n;
-    if (n) memcpy(s->h_mixture + 1, s->mixture.data(), n * 8);
-    CU(cudaMemcpyAsync(d_record, s->h_mixture, words * 8, cudaMemcpyHostToDevice, s->stream));
+    // what every rank contributes to the mixture all-gather: it goes up from pinned memory on the
+    // screen's stream and the record stays on the device for the collective
+    mixture_row(s, s->h_mixture);
+    CU(cudaMemcpyAsync(d_record, s->h_mixture, ((size_t)s->db->s + 1) * 8, cudaMemcpyHostToDevice, s->stream));
     return HS_OK;
 }
 
@@ -1893,28 +1914,6 @@ HS_API int hs_screen_segment_set_size(hs_screen *s, uint32_t segment, uint64_t *
     if (!s->flushed) return fail(HS_ESTATE, "call hs_screen_flush first");
     if (segment >= s->db->seg_s.size()) return fail(HS_EINVAL, "segment index out of range");
     *set_size = set_size_of(s->mixture, s->db->use64, s->db->seg_s[segment]);
-    return HS_OK;
-}
-
-HS_API int hs_screen_mixture_merge(hs_screen *s, const uint64_t *hashes, uint32_t n)
-{
-    if (!s || (!hashes && n)) return fail(HS_EINVAL, "null argument");
-    if (!s->flushed) return fail(HS_ESTATE, "call hs_screen_flush first");
-    // union of per-rank bottom-s sets, keep the s smallest (<= G*s values: control-plane work).
-    // Both sides are normally ascending (hs_screen_mixture_get order): a linear merge, not a sort --
-    // seven sorts of 2000 values were 0.4 ms of an 8-GPU step.
-    if (std::is_sorted(hashes, hashes + n)) {
-        std::vector<uint64_t> merged(s->mixture.size() + n);
-        std::merge(s->mixture.begin(), s->mixture.end(), hashes, hashes + n, merged.begin());
-        s->mixture.swap(merged);
-    } else {
-        s->mixture.insert(s->mixture.end(), hashes, hashes + n);
-        std::sort(s->mixture.begin(), s->mixture.end());
-    }
-    s->mixture.erase(std::unique(s->mixture.begin(), s->mixture.end()), s->mixture.end());
-    if (s->mixture.size() > s->db->s) s->mixture.resize(s->db->s);
-    s->st.n_mixture = s->mixture.size();
-    s->st.set_size = set_size_of(s->mixture, s->db->use64, s->db->seg_s[0]);
     return HS_OK;
 }
 
@@ -2030,7 +2029,6 @@ int enqueue_hits(hs_screen *s, bool dense)
 // results on the host (all N references as columns, or only the references with hits as rows)
 int finish_core(hs_screen *s, bool wta, bool hits)
 {
-    hs_db *db = s->db;
     // Single-GPU order: the per-sketch reduction needs only counts[], so it is enqueued BEFORE the
     // mixture is settled and runs underneath the host round trips of that (flush); a caller that
     // flushed first (multi-GPU: flush -> exchange -> finish) gets it here, after the exchange.
@@ -2088,12 +2086,7 @@ int finish_core(hs_screen *s, bool wta, bool hits)
         if (rc) return rc;
         s->flushed = true;
     }
-    if (s->mixture_on_device) {   // the merged mixture and its set size arrive with the results
-        const uint32_t nm = std::min<uint32_t>(s->h_sparse->n_mix, db->s);
-        s->mixture.assign(s->h_mixture, s->h_mixture + nm);
-        s->st.n_mixture = nm;
-        s->st.set_size = s->h_sparse->set_size[0];
-    }
+    if (s->mixture_on_device) adopt_merged_mixture(s);   // the merged mixture and its set size arrive with the results
     s->st.exchange_overflow = s->h_sparse->xchg_overflow;
     s->st.exchange_max_pairs = s->h_sparse->xchg_max;
     if (!dense && (s->h_sparse->n_touched > s->touched_cap || s->h_sparse->wrapped || s->h_sparse->overflow)) {

@@ -2301,13 +2301,6 @@ __device__ __forceinline__ void add_pair(const SparseView &sp, uint32_t *counts,
     if (id < n_counts && c) count_add(sp, counts, (uint32_t)id, c);   // padding carries id 0xFFFFFFFF
 }
 
-__global__ void __launch_bounds__(256) k_counts_scatter_add(const SparseView sp, uint32_t *counts, uint64_t n_counts,
-                                                            const unsigned long long *pairs, uint64_t n_pairs)
-{
-    for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n_pairs; i += (uint64_t)gridDim.x * blockDim.x)
-        add_pair(sp, counts, n_counts, pairs[i]);
-}
-
 __global__ void __launch_bounds__(256) k_counts_absorb(const SparseView sp, uint32_t *counts, uint64_t n_counts,
                                                        const unsigned long long *rows, uint32_t n_rows, uint32_t cap,
                                                        uint32_t skip)
@@ -2334,14 +2327,6 @@ cudaError_t launch_counts_compact(const SparseView &sp, const uint32_t *counts, 
     if (!n) return cudaSuccess;
     if (sp.touched) k_touched_pairs<<<148 * 4, 256, 0, st>>>(sp, counts, pairs, cap, n_out);
     k_counts_compact<<<grid_for(n, 256, 148 * 8), 256, 0, st>>>(sp, counts, n, pairs, cap, n_out);
-    return cudaGetLastError();
-}
-
-cudaError_t launch_counts_scatter_add(const SparseView &sp, uint32_t *counts, uint64_t n_counts,
-                                      const unsigned long long *pairs, uint64_t n_pairs, cudaStream_t st)
-{
-    if (!n_pairs) return cudaSuccess;
-    k_counts_scatter_add<<<grid_for(n_pairs, 256, 148 * 8), 256, 0, st>>>(sp, counts, n_counts, pairs, n_pairs);
     return cudaGetLastError();
 }
 

@@ -216,8 +216,6 @@ cudaError_t launch_counts_clear_if_overflow(const SparseView &sp, uint32_t *coun
 // touched list itself overflowed.
 cudaError_t launch_counts_compact(const SparseView &sp, const uint32_t *counts, uint64_t n, unsigned long long *pairs,
                                   uint32_t cap, uint32_t *n_out, cudaStream_t st);
-cudaError_t launch_counts_scatter_add(const SparseView &sp, uint32_t *counts, uint64_t n_counts,
-                                      const unsigned long long *pairs, uint64_t n_pairs, cudaStream_t st);
 // All ranks' records at once: rows of (1 + cap) words, word 0 = pair count; row `skip` is this
 // rank's own.  Nothing is added (and xchg_overflow is raised) if any row holds more than cap pairs.
 cudaError_t launch_counts_absorb(const SparseView &sp, uint32_t *counts, uint64_t n_counts,

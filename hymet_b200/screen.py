@@ -267,16 +267,8 @@ class Screen:
         check(_abi.load().hs_screen_counts_devptr(self._h, C.byref(p), C.byref(n)))
         return p.value, n.value
 
-    def counts_compact(self, d_pairs_ptr: int, cap: int) -> int:
-        n = C.c_uint32()
-        check(_abi.load().hs_screen_counts_compact(self._h, C.c_void_p(d_pairs_ptr), cap, C.byref(n)))
-        return n.value
-
     def counts_compact_async(self, d_pairs_ptr: int, cap: int, d_n_out_ptr: int):
         check(_abi.load().hs_screen_counts_compact_async(self._h, C.c_void_p(d_pairs_ptr), cap, C.c_void_p(d_n_out_ptr)))
-
-    def counts_scatter_add(self, d_pairs_ptr: int, n_pairs: int):
-        check(_abi.load().hs_screen_counts_scatter_add(self._h, C.c_void_p(d_pairs_ptr), n_pairs))
 
     def counts_absorb(self, d_rows_ptr: int, n_rows: int, cap: int, skip_row: int):
         """All ranks' pair records (device memory, after the all-gather) added in one launch."""
@@ -299,10 +291,6 @@ class Screen:
         v = C.c_uint64()
         check(_abi.load().hs_screen_segment_set_size(self._h, segment, C.byref(v)))
         return v.value
-
-    def merge_mixture(self, hashes):
-        hashes = np.ascontiguousarray(hashes, np.uint64)
-        check(_abi.load().hs_screen_mixture_merge(self._h, _ptr(hashes, C.c_uint64), len(hashes)))
 
     # ---- reduction ---------------------------------------------------------
     def finish(self, wta: bool = False) -> ScreenResult:

@@ -197,30 +197,29 @@ int hs_screen_flush_async(hs_screen *s);
  * entry id; device pointer) may be summed across ranks in place, and every rank's local
  * mixture hashes merged into every other rank, before finish. */
 int hs_screen_counts_devptr(hs_screen *s, void **d_counts, uint64_t *n);
-/* Sparse form of the same exchange, for when few hashes were hit: compact the non-zero
- * counts into (entry id << 32 | count) pairs in a DEVICE buffer of `cap` pairs (*n = pairs
- * found, may exceed cap: then nothing useful was written), and add another rank's pairs into
- * counts[] (pairs whose id is >= n_entries are padding and ignored). */
-int hs_screen_counts_compact(hs_screen *s, void *d_pairs, uint32_t cap, uint32_t *n);
-/* (The pairs come from the screen's record of which counts left zero -- O(present hashes) -- or, when
- * that record overflowed, from a scan of all counts.)
- * Same compaction, enqueued on the screen's stream without waiting: the pair count goes to the
- * uint32 at d_n_out (device memory), so a whole exchange needs a single host synchronisation.
- * May be called before hs_screen_flush (after the last feed): counts[] no longer changes, and the
- * collective that carries the pairs can then run underneath the flush. */
+/* Sparse form of the same exchange, for when few hashes were hit: compact the non-zero counts into
+ * (entry id << 32 | count) pairs in a DEVICE buffer of `cap` pairs.  The pairs come from the screen's
+ * record of which counts left zero -- O(present hashes) -- or, when that record overflowed, from a
+ * scan of all counts.  Enqueued on the screen's stream without waiting: the pair count goes to the
+ * uint32 at d_n_out (device memory; it may exceed cap: then the pairs are incomplete), so a whole
+ * exchange needs a single host synchronisation.  May be called before hs_screen_flush (after the last
+ * feed): counts[] no longer changes, and the collective that carries the pairs can then run
+ * underneath the flush. */
 int hs_screen_counts_compact_async(hs_screen *s, void *d_pairs, uint32_t cap, void *d_n_out);
-int hs_screen_counts_scatter_add(hs_screen *s, const void *d_pairs, uint64_t n_pairs);
 /* The whole exchange in one launch: d_rows = what an all-gather of every rank's record leaves in
  * DEVICE memory, n_rows records of (1 + cap) 64-bit words each, word 0 = that rank's pair count, then
  * its pairs; row `skip_row` (this rank's own) is not added.  If any record holds more than cap pairs
  * nothing is added and hs_stats_t.exchange_overflow is set by the next hs_screen_finish -- every rank
  * sees the same records, so every rank takes the same decision.  No host synchronisation. */
 int hs_screen_counts_absorb(hs_screen *s, const void *d_rows, uint32_t n_rows, uint32_t cap, uint32_t skip_row);
-/* Several GPUs in ONE process (HYMET_SCREEN_GPUS): after both are flushed, add src's counts and mixture
- * into dst -- src's (entry id, count) pairs travel device to device (peer copy over NVLink when the GPUs
- * are peers).  The two screens must be over the same sketch database (one copy per GPU).  dst then
- * finishes for everybody. */
-int hs_screen_absorb_screen(hs_screen *dst, hs_screen *src);
+/* Several GPUs in ONE process (HYMET_SCREEN_GPUS): add the counts and mixtures of n_src flushed screens
+ * into dst (flushed too; all over copies of the same sketch database, one per GPU).  The in-process form
+ * of the distributed exchange: each source's pair record is built on its own device and peer-copied
+ * (over NVLink when the GPUs are peers) to dst's, then hs_screen_counts_absorb and
+ * hs_screen_mixture_merge_device do the rest.  dst then finishes for everybody.  Refused, with every
+ * handle left as it was: dst among the sources, a source listed twice, an unflushed screen, or a dst
+ * that has already absorbed since its last reset (HS_EINVAL / HS_ESTATE). */
+int hs_screen_absorb_screens(hs_screen *dst, hs_screen *const *src, uint32_t n_src);
 int hs_screen_mixture_get(hs_screen *s, uint64_t *hashes /*[s]*/, uint32_t *n);
 /* Mixture exchange without the host: write this rank's record [length | s hashes, zero padded]
  * ((s + 1) 64-bit words, DEVICE memory) after flush; after the all-gather, merge n_rows such records
@@ -228,7 +227,6 @@ int hs_screen_mixture_get(hs_screen *s, uint64_t *hashes /*[s]*/, uint32_t *n);
  * then takes the set size from device memory and returns the merged mixture with the results. */
 int hs_screen_mixture_record(hs_screen *s, void *d_record);
 int hs_screen_mixture_merge_device(hs_screen *s, const void *d_rows, uint32_t n_rows);
-int hs_screen_mixture_merge(hs_screen *s, const uint64_t *hashes, uint32_t n);
 /* Set size (S10) used for the p-values of one file of a multi-file db (after flush). */
 int hs_screen_segment_set_size(hs_screen *s, uint32_t segment, uint64_t *set_size);
 
