@@ -21,12 +21,15 @@
 #include <atomic>
 #include <chrono>
 #include <condition_variable>
+#include <memory>
 #include <mutex>
 #include <string>
 #include <thread>
+#include <type_traits>
 #include <vector>
 
 #include "../../include/hymet_screen.h"
+#include "cuda_owned.h"
 #include "fasta_pack.h"
 #include "kmer_core.cuh"
 #include "lca_kernels.h"
@@ -64,19 +67,6 @@ int fail(int code, const std::string &msg)
     } while (0)
 #define ON_DEVICE(dev) CU(cudaSetDevice(dev))
 
-// device allocations of a build step: freed on every return path unless released to their owner
-struct DevBufs {
-    std::vector<void *> p;
-    template <class T> cudaError_t alloc(T **out, size_t bytes)
-    {
-        void *q = nullptr;
-        cudaError_t e = cudaMalloc(&q, bytes ? bytes : 1);
-        if (e == cudaSuccess) { p.push_back(q); *out = (T *)q; }
-        return e;
-    }
-    ~DevBufs() { for (void *q : p) cudaFree(q); }
-};
-
 double now_s()
 {
     return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count();
@@ -86,22 +76,21 @@ uint64_t tiles_for(uint64_t n_bases) { return ((n_bases + 31) / 32 + kTileWords 
 
 // ---- device arena for query chunks ------------------------------------------
 struct Arena {
-    struct Slab { char *p; size_t cap, used; };
+    struct Slab { DevBuf<char> mem; size_t used = 0; };
     std::vector<Slab> slabs;
     size_t slab_bytes = (size_t)256 << 20;
-    size_t total = 0, cur = 0;
+    size_t cur = 0;
     cudaError_t alloc(size_t n, void **out)
     {
         n = (n + 255) & ~(size_t)255;
-        while (cur < slabs.size() && slabs[cur].used + n > slabs[cur].cap) cur++;
+        while (cur < slabs.size() && slabs[cur].used + n > slabs[cur].mem.cap()) cur++;
         if (cur == slabs.size()) {
-            Slab s{nullptr, std::max(n, slab_bytes), 0};
-            cudaError_t e = cudaMalloc((void **)&s.p, s.cap);
+            Slab s;
+            cudaError_t e = s.mem.grow(std::max(n, slab_bytes));
             if (e != cudaSuccess) return e;
-            slabs.push_back(s);
-            total += s.cap;
+            slabs.push_back(std::move(s));
         }
-        *out = slabs[cur].p + slabs[cur].used;
+        *out = slabs[cur].mem.get() + slabs[cur].used;
         slabs[cur].used += n;
         return cudaSuccess;
     }
@@ -109,12 +98,6 @@ struct Arena {
     {   // slabs stay allocated: a steady-state screen never calls cudaMalloc/cudaFree
         for (auto &s : slabs) s.used = 0;
         cur = 0;
-    }
-    void release()
-    {
-        for (auto &s : slabs) cudaFree(s.p);
-        slabs.clear();
-        total = 0; cur = 0;
     }
 };
 
@@ -128,57 +111,66 @@ struct Chunk {
 // ---- device-side FASTA ingest: raw text slots + scan scratch ------------------------
 struct Ingest {
     static constexpr int kSlots = 4;
-    struct Slot { uint8_t *raw = nullptr, *codes = nullptr; size_t cap = 0; cudaEvent_t done = nullptr, copied = nullptr; };
+    struct Slot { DevBuf<uint8_t> raw, codes; Event done, copied; };
     Slot slots[kSlots];
     int next = 0;
+    DevBuf<char> scan;                                  // the eight FaScratch arrays (carve)
     FaScratch sc{};
     size_t tile_cap = 0;
-    std::vector<unsigned long long *> counter_blocks;   // per-chunk position counters (512 per block)
+    std::vector<DevBuf<unsigned long long>> counter_blocks;   // per-chunk position counters (512 per block)
     size_t counters_used = 0;
-    unsigned long long *d_totals = nullptr;             // [0] positions [1] bases [2] records
+    DevBuf<unsigned long long> d_totals;                // [0] positions [1] bases [2] records
     bool ready = false;
 
+    // points sc's arrays into base (tile capacity cap), each on a 256-byte boundary as if allocated
+    // alone; returns the bytes they take
+    size_t carve(char *base, size_t cap)
+    {
+        size_t off = 0;
+        auto part = [&](auto *&p, size_t n) {
+            p = reinterpret_cast<std::remove_reference_t<decltype(p)>>(reinterpret_cast<uintptr_t>(base) + off);
+            off += (n * sizeof(*p) + 255) & ~(size_t)255;
+        };
+        part(sc.masks, cap * 256); part(sc.emit, cap * 256);
+        part(sc.tile_event, cap); part(sc.tile_carry, cap); part(sc.tile_event_b, cap); part(sc.tile_carry_b, cap);
+        part(sc.tile_count, cap); part(sc.tile_offset, cap);
+        return off;
+    }
     int ensure(size_t bytes, cudaStream_t st)
     {
         if (!ready) {
-            CU(cudaMalloc((void **)&d_totals, 4 * sizeof(unsigned long long)));
+            CU(d_totals.grow(4));
             // on the stream that will accumulate into it: the legacy default stream is not ordered
             // against a non-blocking stream
-            CU(cudaMemsetAsync(d_totals, 0, 4 * sizeof(unsigned long long), st));
+            CU(cudaMemsetAsync(d_totals.get(), 0, 4 * sizeof(unsigned long long), st));
             for (auto &sl : slots) {
-                CU(cudaEventCreateWithFlags(&sl.done, cudaEventDisableTiming | cudaEventBlockingSync));
-                CU(cudaEventCreateWithFlags(&sl.copied, cudaEventDisableTiming));
+                CU(sl.done.create(cudaEventDisableTiming | cudaEventBlockingSync));
+                CU(sl.copied.create(cudaEventDisableTiming));
             }
             ready = true;
         }
         const size_t tiles = (bytes + kFaTileBytes - 1) / kFaTileBytes + 1;
         if (tiles > tile_cap) {
             cudaDeviceSynchronize();
-            cudaFree(sc.tile_event); cudaFree(sc.tile_carry); cudaFree(sc.tile_event_b); cudaFree(sc.tile_carry_b);
-            cudaFree(sc.tile_count); cudaFree(sc.tile_offset); cudaFree(sc.masks); cudaFree(sc.emit);
-            tile_cap = tiles + tiles / 4;
-            CU(cudaMalloc((void **)&sc.masks, tile_cap * 256 * sizeof(uint4)));
-            CU(cudaMalloc((void **)&sc.emit, tile_cap * 256 * sizeof(uint2)));
-            CU(cudaMalloc((void **)&sc.tile_event, tile_cap * 4));
-            CU(cudaMalloc((void **)&sc.tile_carry, tile_cap * 4));
-            CU(cudaMalloc((void **)&sc.tile_event_b, tile_cap * 4));
-            CU(cudaMalloc((void **)&sc.tile_carry_b, tile_cap * 4));
-            CU(cudaMalloc((void **)&sc.tile_count, tile_cap * 4));
-            CU(cudaMalloc((void **)&sc.tile_offset, tile_cap * 8));
+            tile_cap = 0;   // sc points nowhere until the new scratch is carved
+            const size_t cap = tiles + tiles / 4;
+            CU(scan.grow(carve(nullptr, cap)));
+            carve(scan.get(), cap);
+            tile_cap = cap;
         }
-        sc.totals = d_totals;
+        sc.totals = d_totals.get();
         return HS_OK;
     }
     int slot_for(size_t bytes, Slot **out)
     {
         Slot &sl = slots[next];
         next = (next + 1) % kSlots;
-        CU(cudaEventSynchronize(sl.done));  // throttle: at most kSlots chunks of raw text in flight
-        if (sl.cap < bytes) {
-            cudaFree(sl.raw); cudaFree(sl.codes);
-            sl.cap = bytes + bytes / 8 + 64;
-            CU(cudaMalloc((void **)&sl.raw, sl.cap));
-            CU(cudaMalloc((void **)&sl.codes, sl.cap));
+        CU(cudaEventSynchronize(sl.done.get()));  // throttle: at most kSlots chunks of raw text in flight
+        if (sl.raw.cap() < bytes || sl.codes.cap() < bytes) {
+            const size_t cap = bytes + bytes / 8 + 64;
+            sl.raw.reset(); sl.codes.reset();   // both go before either grows
+            CU(sl.raw.grow(cap));
+            CU(sl.codes.grow(cap));
         }
         *out = &sl;
         return HS_OK;
@@ -186,24 +178,13 @@ struct Ingest {
     int counter(unsigned long long **out)
     {
         if (counters_used == counter_blocks.size() * 512) {
-            unsigned long long *b = nullptr;
-            CU(cudaMalloc((void **)&b, 512 * sizeof(unsigned long long)));
-            counter_blocks.push_back(b);
+            DevBuf<unsigned long long> b;
+            CU(b.grow(512));
+            counter_blocks.push_back(std::move(b));
         }
-        *out = counter_blocks[counters_used / 512] + counters_used % 512;
+        *out = counter_blocks[counters_used / 512].get() + counters_used % 512;
         counters_used++;
         return HS_OK;
-    }
-    void release()
-    {
-        for (auto &sl : slots) {
-            cudaFree(sl.raw); cudaFree(sl.codes);
-            if (sl.done) cudaEventDestroy(sl.done);
-            if (sl.copied) cudaEventDestroy(sl.copied);
-        }
-        cudaFree(sc.tile_event); cudaFree(sc.tile_carry); cudaFree(sc.tile_event_b); cudaFree(sc.tile_carry_b);
-        cudaFree(sc.tile_count); cudaFree(sc.tile_offset); cudaFree(sc.masks); cudaFree(sc.emit); cudaFree(d_totals);
-        for (auto *b : counter_blocks) cudaFree(b);
     }
 };
 
@@ -214,14 +195,14 @@ struct Ingest {
 struct MixEngine {
     uint32_t s = 0, cap = 0, cand_cap = 0;
     bool use64 = true;     // 32-bit hashes (k <= 16) live in [0, 2^32): caps and tau start there
-    uint64_t *d_set[2] = {nullptr, nullptr};
-    MixState *d_state = nullptr;
-    MixState *h_state = nullptr;  // pinned mirror, valid after sync_state()
-    uint64_t *d_cand = nullptr, *d_scratch = nullptr;
-    uint32_t *d_hist = nullptr;   // device-side selection: 2048 bins
+    DevBuf<uint64_t> d_set[2];
+    DevBuf<MixState> d_state;
+    PinnedBuf<MixState> h_state;  // pinned mirror, valid after sync_state()
+    DevBuf<uint64_t> d_cand, d_scratch;
+    DevBuf<uint32_t> d_hist;      // device-side selection: 2048 bins
     uint32_t sel_pad = 0;         // its sort capacity (power of two >= s + slack, <= cand_cap)
     bool fast_select = true;
-    uint64_t *h_cand = nullptr;   // pinned: the settled mixture travels with the state, one sync for both
+    PinnedBuf<uint64_t> h_cand;   // pinned: the settled mixture travels with the state, one sync for both
     bool auto_tau = true;  // first pass: cap tau per launch so expected offers stay <= cap/8
     uint32_t passes = 1;
 
@@ -233,31 +214,24 @@ struct MixEngine {
         while ((uint64_t)cap < 64ull * s) cap <<= 1;
         cand_cap = 8192;
         while (cand_cap < 4 * s) cand_cap <<= 1;
-        for (int i = 0; i < 2; i++) CU(cudaMalloc((void **)&d_set[i], (size_t)cap * 8));
-        CU(cudaMalloc((void **)&d_state, sizeof(MixState)));
-        CU(cudaHostAlloc((void **)&h_state, sizeof(MixState), cudaHostAllocDefault));
-        CU(cudaMalloc((void **)&d_cand, (size_t)cand_cap * 8));
-        CU(cudaMalloc((void **)&d_scratch, (size_t)cand_cap * 8));
-        CU(cudaMalloc((void **)&d_hist, (2 * 2048 + 8) * sizeof(uint32_t)));   // bin counts | bin starts | last bin
+        for (int i = 0; i < 2; i++) CU(d_set[i].grow(cap));
+        CU(d_state.grow(1));
+        CU(h_state.grow(1));
+        CU(d_cand.grow(cand_cap));
+        CU(d_scratch.grow(cand_cap));
+        CU(d_hist.grow(2 * 2048 + 8));   // bin counts | bin starts | last bin
         sel_pad = 2048;
         while (sel_pad < s + 1024) sel_pad <<= 1;
         if (sel_pad > cand_cap) sel_pad = cand_cap;
         if (const char *e = getenv("HYMET_SCREEN_FAST_SELECT")) fast_select = atoi(e) != 0;
-        CU(cudaHostAlloc((void **)&h_cand, (size_t)s * 8, cudaHostAllocDefault));
+        CU(h_cand.grow(s));
         return HS_OK;
     }
-    void destroy()
-    {
-        for (int i = 0; i < 2; i++) cudaFree(d_set[i]);
-        cudaFree(d_state); cudaFree(d_cand); cudaFree(d_scratch); cudaFree(d_hist);
-        if (h_state) cudaFreeHost(h_state);
-        if (h_cand) cudaFreeHost(h_cand);
-    }
-    uint32_t *field(size_t off) const { return reinterpret_cast<uint32_t *>(reinterpret_cast<char *>(d_state) + off); }
+    uint32_t *field(size_t off) const { return reinterpret_cast<uint32_t *>(reinterpret_cast<char *>(d_state.get()) + off); }
     int reset(cudaStream_t st, uint64_t new_tau = ~0ull, bool automatic = true)
     {
-        CU(cudaMemsetAsync(d_set[0], 0xFF, (size_t)cap * 8, st));
-        CU(launch_mix_state_init(d_state, new_tau, st));
+        CU(cudaMemsetAsync(d_set[0].get(), 0xFF, (size_t)cap * 8, st));
+        CU(launch_mix_state_init(d_state.get(), new_tau, st));
         auto_tau = automatic;  // a re-offer pass runs at exactly the tau the finaliser chose
         return HS_OK;
     }
@@ -272,13 +246,13 @@ struct MixEngine {
     MixView view(uint64_t tau_cap) const
     {
         MixView v;
-        v.sets[0] = d_set[0]; v.sets[1] = d_set[1];
-        v.mask = cap - 1; v.limit = cap / 2; v.tau_cap = tau_cap; v.st = d_state;
+        v.sets[0] = d_set[0].get(); v.sets[1] = d_set[1].get();
+        v.mask = cap - 1; v.limit = cap / 2; v.tau_cap = tau_cap; v.st = d_state.get();
         return v;
     }
     int sync_state(cudaStream_t st)
     {
-        CU(cudaMemcpyAsync(h_state, d_state, sizeof(MixState), cudaMemcpyDeviceToHost, st));
+        CU(cudaMemcpyAsync(h_state.get(), d_state.get(), sizeof(MixState), cudaMemcpyDeviceToHost, st));
         CU(cudaStreamSynchronize(st));
         return HS_OK;
     }
@@ -298,51 +272,47 @@ struct hs_db {
     uint64_t n_refs = 0, n_entries = 0, n_distinct = 0, max_key = 0, dense_max = 0;
     std::vector<std::string> names, comments;
     std::vector<uint64_t> lengths, offsets;
-    uint64_t *d_buckets = nullptr;           // n_buckets x 128 bytes: keys | canonical entry ids | overflow flag
+    DevBuf<uint64_t> d_buckets;              // n_buckets x 128 bytes: keys | canonical entry ids | overflow flag
     uint32_t n_buckets = 0, special = kNoEntry;
-    uint32_t *d_canon = nullptr;             // per stored hash: canonical entry id of its key (reference -> hashes, dense path)
-    uint32_t *d_next = nullptr;              // per stored hash: next entry holding the same key (hash -> references, sparse path)
-    uint64_t *d_offsets = nullptr, *d_lengths = nullptr, *d_seg_begin = nullptr;
-    uint32_t *d_seg_s = nullptr;
+    DevBuf<uint32_t> d_canon;                // per stored hash: canonical entry id of its key (reference -> hashes, dense path)
+    DevBuf<uint32_t> d_next;                 // per stored hash: next entry holding the same key (hash -> references, sparse path)
+    DevBuf<uint64_t> d_offsets, d_lengths, d_seg_begin;
+    DevBuf<uint32_t> d_seg_s;
     uint64_t device_bytes = 0;
     double t_parse = 0, t_build = 0;
-    uint32_t *d_bloom = nullptr;
+    DevBuf<uint32_t> d_bloom;
     uint32_t bloom_mask = 0;
     uint64_t bloom_keys = 0;                 // keys above dense_max (what the Bloom filter holds)
     // Several .msh files screened in one pass (run_hymet_cami.sh:85-97 streams the query three times):
     // references [seg_begin[j], seg_begin[j+1]) came from file j, whose sketch size was seg_s[j].
     std::vector<uint64_t> seg_begin;
     std::vector<uint32_t> seg_s;
-    TableView view() const { return TableView{d_buckets, n_buckets, max_key, special, d_bloom, bloom_mask, d_bloom ? dense_max : max_key}; }
+    TableView view() const
+    {
+        return TableView{d_buckets.get(), n_buckets, max_key, special, d_bloom.get(), bloom_mask, d_bloom.get() ? dense_max : max_key};
+    }
 };
 
 // pinned ring the file readers pread() into: two slots per reader thread
 struct FileRing {
-    char *base = nullptr;
+    PinnedBuf<char> base;
     size_t slot_cap = 0;
-    std::vector<cudaEvent_t> free_ev;   // recorded on the copy stream once a slot's text is in HBM
-    void release()
-    {
-        if (base) cudaFreeHost(base);
-        base = nullptr; slot_cap = 0;
-        for (auto e : free_ev) cudaEventDestroy(e);
-        free_ev.clear();
-    }
+    std::vector<Event> free_ev;   // recorded on the copy stream once a slot's text is in HBM
 };
 
 struct Staging {
-    uint64_t *seq = nullptr;
-    uint32_t *inv = nullptr;
+    PinnedBuf<uint64_t> seq;
+    PinnedBuf<uint32_t> inv;
     uint64_t cap_words = 0;
-    cudaEvent_t free_ev = nullptr;
+    Event free_ev;
 };
 
 struct hs_screen {
     hs_db *db = nullptr;
-    cudaStream_t stream = nullptr;
-    bool own_stream = false;
-    cudaStream_t copy_stream = nullptr;      // H2D of query chunks overlaps the kernels of earlier chunks
-    std::vector<cudaEvent_t> copy_evs;
+    // declared first, so released last (members go in reverse order, after the destructor's wait)
+    Stream stream;                           // the handle's own, or the caller's (hs_screen_set_stream)
+    Stream copy_stream;                      // H2D of query chunks overlaps the kernels of earlier chunks
+    std::vector<Event> copy_evs;
     size_t copy_ev_used = 0;
     Ingest ingest;
     int ingest_mode = 2;   // 0 = host packer only, 1 = device parser only, 2 = both compete for chunks (pinned text)
@@ -357,25 +327,27 @@ struct hs_screen {
     int file_mode = -1;   // plain FASTA files: 0 pread ring + device parser, 1 mmap + host packers, -1 by host capability
     std::mutex ingest_mu;                       // one thread at a time hands a span to the device parser
     std::mutex giant_mu;                        // records larger than a ring slot take the host path, one at a time
-    uint32_t *d_counts = nullptr;
-    unsigned long long *d_stats = nullptr;
+    DevBuf<uint32_t> d_counts;
+    DevBuf<unsigned long long> d_stats;
     // O(present hashes) bookkeeping (SparseState): ids of the non-zero counts, references with hits,
     // their depth segments.  touched_valid: the list covers every non-zero count as far as the HOST
     // knows (a dense all-reduce into counts[] invalidates it; the device flags overflow and wraps).
-    SparseState *d_sparse = nullptr, *h_sparse = nullptr;
-    uint32_t *d_touched = nullptr, *d_hit = nullptr, *d_seg_start = nullptr, *d_seg_fill = nullptr, *d_plain = nullptr;
-    uint32_t *d_depths = nullptr;
+    DevBuf<SparseState> d_sparse;
+    PinnedBuf<SparseState> h_sparse;
+    DevBuf<uint32_t> d_touched, d_depths;
+    DevBuf<uint32_t> d_ref_rows;   // one block: hit | seg_start | seg_fill | plain
+    uint32_t *d_hit = nullptr, *d_seg_start = nullptr, *d_seg_fill = nullptr, *d_plain = nullptr;
     uint32_t touched_cap = 0, pair_cap = 0;
     bool touched_valid = true, sparse_enabled = true;
     uint32_t last_reduce_dense = 0;
     // multi-GPU: mixture merged on the device (hs_screen_mixture_merge_device)
-    uint64_t *d_mixture = nullptr, *d_merge_work = nullptr, *d_merge_scratch = nullptr, *h_mixture = nullptr;
-    uint32_t merge_cap = 0;
+    DevBuf<uint64_t> d_mixture, d_merge_work, d_merge_scratch;
+    PinnedBuf<uint64_t> h_mixture;
     bool mixture_on_device = false;
-    cudaEvent_t rst0 = nullptr, rst1 = nullptr;
+    Event rst0, rst1;
     bool rst_pending = false;
     // result rows of the references with hits (hs_screen_finish_hits): pinned, host-mapped, written by the GPU
-    char *h_rows = nullptr;
+    PinnedBuf<char> h_rows;
     HitRows rows_host{}, rows_dev{};
     std::vector<uint32_t> hit_order;   // indices into the rows, ascending by reference, shared > 0 only
     MixEngine mix;
@@ -384,10 +356,10 @@ struct hs_screen {
     bool flush_pending = false;   // hs_screen_flush_async: selection enqueued, verdict read after the next synchronisation
     bool flush_parsed = false;    // ... and it fetched the device parser's totals
     int force_unsettled = 0;      // tests: the next mixture record says "not settled" (HYMET_SCREEN_FORCE_UNSETTLED)
+    DevBuf<double> d_result;   // one block: identity | p-value | shared | median
     uint32_t *d_shared = nullptr, *d_median = nullptr;
     double *d_identity = nullptr, *d_pvalue = nullptr;
-    unsigned long long *d_best_score = nullptr, *d_best_len = nullptr;
-    uint32_t *d_winner = nullptr;
+    DevBuf<char> d_win;        // -w on the dense path: best score | best length | winner
     Arena arena;
     std::vector<Chunk> chunks;
     std::vector<Staging> staging;
@@ -395,12 +367,17 @@ struct hs_screen {
     bool filter = true;
     uint64_t chunk_text = (uint64_t)16 << 20;
     hs_stats_t st;
-    std::vector<std::pair<cudaEvent_t, cudaEvent_t>> ev_pool;
+    std::vector<std::pair<Event, Event>> ev_pool;
     size_t ev_used = 0;
-    cudaEvent_t red0 = nullptr, red1 = nullptr, red2 = nullptr, red3 = nullptr;
-    unsigned long long *h_stats = nullptr;   // pinned: [0, ST_COUNT) kernel counters, then 4 device-parser totals
-    char *h_result = nullptr;   // pinned landing zone for the four result columns (24 B per sketch):
+    Event red0, red1, red2, red3;
+    PinnedBuf<unsigned long long> h_stats;   // pinned: [0, ST_COUNT) kernel counters, then 4 device-parser totals
+    PinnedBuf<char> h_result;   // pinned landing zone for the four result columns (24 B per sketch):
                                 // a D2H copy into the caller's pageable arrays costs ~0.3 ms at N = 50 000
+    ~hs_screen()
+    {   // the copy stream reads the staging and the ring; both streams write buffers released below
+        if (stream.get()) cudaStreamSynchronize(stream.get());
+        if (copy_stream.get()) cudaStreamSynchronize(copy_stream.get());
+    }
 };
 
 namespace {
@@ -465,34 +442,33 @@ int db_build(hs_db *db, const uint64_t *hashes)
     if (db->seg_begin.empty()) { db->seg_begin = {0, N}; db->seg_s = {db->s}; }
     if (db->seg_s.size() > 8) return fail(HS_EUNSUPPORTED, "more than 8 sketch files in one table");
 
-    DevBufs tmp;   // build scratch: released on every path out of here
-    uint64_t *d_hashes = nullptr;
-    uint32_t *d_flags = nullptr;
-    unsigned long long *d_nd = nullptr;
-    // the handle owns what it was given so far: hs_db_free() releases it if a later step fails
-    CU(cudaMalloc((void **)&db->d_buckets, nb * kBucketWords * 8));
-    CU(cudaMalloc((void **)&db->d_canon, std::max<uint64_t>(E, 1) * 4));
-    CU(cudaMalloc((void **)&db->d_next, std::max<uint64_t>(E, 1) * 4));
-    CU(cudaMalloc((void **)&db->d_offsets, (N + 1) * 8));
-    CU(cudaMalloc((void **)&db->d_lengths, std::max<uint64_t>(N, 1) * 8));
-    CU(cudaMalloc((void **)&db->d_seg_begin, db->seg_begin.size() * 8));
-    CU(cudaMalloc((void **)&db->d_seg_s, db->seg_s.size() * 4));
-    CU(tmp.alloc(&d_hashes, E * 8));
-    CU(tmp.alloc(&d_flags, 2 * sizeof(uint32_t)));
-    CU(tmp.alloc(&d_nd, sizeof(unsigned long long)));
+    // build scratch; the handle's buffers are its own from here on (deleting it releases them)
+    DevBuf<uint64_t> d_hashes;
+    DevBuf<uint32_t> d_flags;
+    DevBuf<unsigned long long> d_nd;
+    CU(db->d_buckets.grow(nb * kBucketWords));
+    CU(db->d_canon.grow(std::max<uint64_t>(E, 1)));
+    CU(db->d_next.grow(std::max<uint64_t>(E, 1)));
+    CU(db->d_offsets.grow(N + 1));
+    CU(db->d_lengths.grow(std::max<uint64_t>(N, 1)));
+    CU(db->d_seg_begin.grow(db->seg_begin.size()));
+    CU(db->d_seg_s.grow(db->seg_s.size()));
+    CU(d_hashes.grow(std::max<uint64_t>(E, 1)));
+    CU(d_flags.grow(2));
+    CU(d_nd.grow(1));
     db->device_bytes = nb * kBucketWords * 8 + E * 8 + (N + 1) * 8 + N * 8;
-    CU(cudaMemset(db->d_next, 0xFF, std::max<uint64_t>(E, 1) * 4));   // kNoEntry = end of chain
-    CU(cudaMemset(d_flags, 0xFF, sizeof(uint32_t)));      // [0] special = kNoEntry
-    CU(cudaMemset(d_flags + 1, 0, sizeof(uint32_t)));     // [1] fail
-    CU(cudaMemset(d_nd, 0, sizeof(unsigned long long)));
-    if (E) CU(cudaMemcpy(d_hashes, hashes, E * 8, cudaMemcpyHostToDevice));
-    CU(cudaMemcpy(db->d_offsets, db->offsets.data(), (N + 1) * 8, cudaMemcpyHostToDevice));
-    if (N) CU(cudaMemcpy(db->d_lengths, db->lengths.data(), N * 8, cudaMemcpyHostToDevice));
-    CU(cudaMemcpy(db->d_seg_begin, db->seg_begin.data(), db->seg_begin.size() * 8, cudaMemcpyHostToDevice));
-    CU(cudaMemcpy(db->d_seg_s, db->seg_s.data(), db->seg_s.size() * 4, cudaMemcpyHostToDevice));
-    CU(launch_table_insert(db->d_buckets, db->n_buckets, d_hashes, E, d_flags, d_flags + 1, 0));
+    CU(cudaMemset(db->d_next.get(), 0xFF, std::max<uint64_t>(E, 1) * 4));   // kNoEntry = end of chain
+    CU(cudaMemset(d_flags.get(), 0xFF, sizeof(uint32_t)));      // [0] special = kNoEntry
+    CU(cudaMemset(d_flags.get() + 1, 0, sizeof(uint32_t)));     // [1] fail
+    CU(cudaMemset(d_nd.get(), 0, sizeof(unsigned long long)));
+    if (E) CU(cudaMemcpy(d_hashes.get(), hashes, E * 8, cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(db->d_offsets.get(), db->offsets.data(), (N + 1) * 8, cudaMemcpyHostToDevice));
+    if (N) CU(cudaMemcpy(db->d_lengths.get(), db->lengths.data(), N * 8, cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(db->d_seg_begin.get(), db->seg_begin.data(), db->seg_begin.size() * 8, cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(db->d_seg_s.get(), db->seg_s.data(), db->seg_s.size() * 4, cudaMemcpyHostToDevice));
+    CU(launch_table_insert(db->d_buckets.get(), db->n_buckets, d_hashes.get(), E, d_flags.get(), d_flags.get() + 1, 0));
     uint32_t flags[2];
-    CU(cudaMemcpy(flags, d_flags, sizeof flags, cudaMemcpyDeviceToHost));
+    CU(cudaMemcpy(flags, d_flags.get(), sizeof flags, cudaMemcpyDeviceToHost));
     if (flags[1]) return fail(HS_ECUDA, "hash table build failed (table full)");
     db->special = flags[0];
     if (db->special != kNoEntry) db->max_key = ~0ull;
@@ -505,18 +481,18 @@ int db_build(hs_db *db, const uint64_t *hashes)
         if (pass > 0.01 && plan.bloom && E) {
             uint64_t words = 4096;
             while (words < plan.words) words <<= 1;
-            CU(cudaMalloc((void **)&db->d_bloom, words * 4));
-            CU(cudaMemset(db->d_bloom, 0, words * 4));
+            CU(db->d_bloom.grow(words));
+            CU(cudaMemset(db->d_bloom.get(), 0, words * 4));
             db->bloom_mask = (uint32_t)(words - 1);
             db->dense_max = plan.dense_max;
             db->bloom_keys = (uint64_t)plan.keys_above;
-            CU(launch_bloom_build(db->d_bloom, db->bloom_mask, db->dense_max, db->use64, d_hashes, E, 0));
+            CU(launch_bloom_build(db->d_bloom.get(), db->bloom_mask, db->dense_max, db->use64, d_hashes.get(), E, 0));
             db->device_bytes += words * 4;
         }
     }
-    CU(launch_table_canon(db->view(), d_hashes, E, db->d_canon, db->d_next, d_nd, 0));
+    CU(launch_table_canon(db->view(), d_hashes.get(), E, db->d_canon.get(), db->d_next.get(), d_nd.get(), 0));
     unsigned long long nd = 0;
-    CU(cudaMemcpy(&nd, d_nd, sizeof nd, cudaMemcpyDeviceToHost));
+    CU(cudaMemcpy(&nd, d_nd.get(), sizeof nd, cudaMemcpyDeviceToHost));
     db->n_distinct = nd;
     db->t_build = now_s() - t0;
     return HS_OK;
@@ -528,8 +504,8 @@ void fill_info(const hs_db *db, hs_db_info_t *o)
     o->k = db->k; o->s = db->s; o->seed = db->seed; o->use64 = db->use64;
     o->n_refs = db->n_refs; o->n_entries = db->n_entries; o->n_distinct = db->n_distinct;
     o->n_buckets = db->n_buckets; o->max_key = db->max_key; o->device_bytes = db->device_bytes;
-    o->bloom_bytes = db->d_bloom ? ((uint64_t)db->bloom_mask + 1) * 4 : 0;
-    o->dense_max = db->d_bloom ? db->dense_max : db->max_key;
+    o->bloom_bytes = db->d_bloom.get() ? ((uint64_t)db->bloom_mask + 1) * 4 : 0;
+    o->dense_max = db->d_bloom.get() ? db->dense_max : db->max_key;
     o->bloom_keys = db->bloom_keys;
     o->t_parse_s = db->t_parse; o->t_build_s = db->t_build;
 }
@@ -555,27 +531,27 @@ int launch_chunk(hs_screen *s, const Chunk &c, bool count, bool mix, uint64_t ti
     a.n_bases_dev = c.n_dev;
     a.tile_begin = (uint32_t)tile_begin; a.n_tiles = (uint32_t)tile_end;
     a.do_count = count; a.do_filter = s->filter; a.do_mix = mix;
-    a.tab = s->db->view(); a.counts = s->d_counts;
+    a.tab = s->db->view(); a.counts = s->d_counts.get();
     // the range test removes probes only when the keys are confined to a sliver of the hash range; a db
     // whose keys cover a quarter of it or more and has no Bloom tier probes for most k-mers: that is
     // the warp-cooperative kernel's job, as is "filter" = 0
-    a.probe_all = !s->filter || (!s->db->d_bloom && s->db->max_key >= ((uint64_t)1 << 62));
-    if (count && s->sparse_enabled) a.sparse = SparseView{s->d_touched, s->touched_cap, s->d_sparse};
+    a.probe_all = !s->filter || (!s->db->d_bloom.get() && s->db->max_key >= ((uint64_t)1 << 62));
+    if (count && s->sparse_enabled) a.sparse = SparseView{s->d_touched.get(), s->touched_cap, s->d_sparse.get()};
     const uint64_t launch_positions = (tile_end - tile_begin) * kTileWords * 32;
     a.mix = s->mix.view(mix ? s->mix.launch_cap(launch_positions) : ~0ull);
-    a.stats = count ? s->d_stats : s->d_stats + ST_COUNT;  // re-offer passes must not double count
+    a.stats = count ? s->d_stats.get() : s->d_stats.get() + ST_COUNT;  // re-offer passes must not double count
     if (s->ev_used == s->ev_pool.size()) {
-        cudaEvent_t e0, e1;
-        CU(cudaEventCreate(&e0)); CU(cudaEventCreate(&e1));
-        s->ev_pool.emplace_back(e0, e1);
+        Event e0, e1;
+        CU(e0.create()); CU(e1.create());
+        s->ev_pool.emplace_back(std::move(e0), std::move(e1));
     }
     auto &ev = s->ev_pool[s->ev_used++];
-    CU(cudaEventRecord(ev.first, s->stream));
-    CU(launch_stream(a, s->db->sm, s->stream));
-    CU(cudaEventRecord(ev.second, s->stream));
+    CU(cudaEventRecord(ev.first.get(), s->stream.get()));
+    CU(launch_stream(a, s->db->sm, s->stream.get()));
+    CU(cudaEventRecord(ev.second.get(), s->stream.get()));
     s->st.n_launches++;
     if (mix) {
-        CU(launch_mix_maintain(a.mix, s->stream));
+        CU(launch_mix_maintain(a.mix, s->stream.get()));
         s->st.n_launches += 3;
     }
     if (!c.n_dev)  // device-parsed chunks are accounted from the parser's own totals at flush
@@ -583,38 +559,38 @@ int launch_chunk(hs_screen *s, const Chunk &c, bool count, bool mix, uint64_t ti
     return HS_OK;
 }
 
-SparseView sparse_view(const hs_screen *s) { return SparseView{s->sparse_enabled ? s->d_touched : nullptr, s->touched_cap, s->d_sparse}; }
+SparseView sparse_view(const hs_screen *s) { return SparseView{s->sparse_enabled ? s->d_touched.get() : nullptr, s->touched_cap, s->d_sparse.get()}; }
 
 int screen_zero(hs_screen *s)
 {
-    CU(cudaEventRecord(s->rst0, s->stream));
+    CU(cudaEventRecord(s->rst0.get(), s->stream.get()));
     if (s->sparse_enabled && s->touched_valid) {
         // counts[] back to zero in O(touched); if the list overflowed on the device, the conditional
         // dense clear does the work instead (both are enqueued, one of them returns at once)
-        CU(launch_sparse_reset(sparse_view(s), s->d_counts, s->db->sm, s->stream));
-        CU(launch_counts_clear_if_overflow(sparse_view(s), s->d_counts, s->db->n_entries, s->stream));
+        CU(launch_sparse_reset(sparse_view(s), s->d_counts.get(), s->db->sm, s->stream.get()));
+        CU(launch_counts_clear_if_overflow(sparse_view(s), s->d_counts.get(), s->db->n_entries, s->stream.get()));
     } else {
-        CU(cudaMemsetAsync(s->d_counts, 0, std::max<uint64_t>(s->db->n_entries, 1) * 4, s->stream));
+        CU(cudaMemsetAsync(s->d_counts.get(), 0, std::max<uint64_t>(s->db->n_entries, 1) * 4, s->stream.get()));
     }
-    CU(cudaMemsetAsync(s->d_sparse, 0, sizeof(SparseState), s->stream));
+    CU(cudaMemsetAsync(s->d_sparse.get(), 0, sizeof(SparseState), s->stream.get()));
     s->touched_valid = true;
     s->mixture_on_device = false;
-    CU(cudaMemsetAsync(s->d_stats, 0, 2 * ST_COUNT * sizeof(unsigned long long), s->stream));
-    int rc = s->mix.reset(s->stream);
+    CU(cudaMemsetAsync(s->d_stats.get(), 0, 2 * ST_COUNT * sizeof(unsigned long long), s->stream.get()));
+    int rc = s->mix.reset(s->stream.get());
     if (rc) return rc;
-    CU(cudaEventRecord(s->rst1, s->stream));
+    CU(cudaEventRecord(s->rst1.get(), s->stream.get()));
     s->rst_pending = true;
     s->mix.passes = 1;
     s->mixture.clear();
     s->flushed = false;
     s->flush_pending = false;
     s->chunks.clear();
-    if (s->copy_stream) CU(cudaStreamSynchronize(s->copy_stream));
+    if (s->copy_stream.get()) CU(cudaStreamSynchronize(s->copy_stream.get()));
     s->arena.reset();
     s->ev_used = 0;
     s->copy_ev_used = 0;
     s->ingest.counters_used = 0;
-    if (s->ingest.ready) CU(cudaMemsetAsync(s->ingest.d_totals, 0, 4 * sizeof(unsigned long long), s->stream));
+    if (s->ingest.ready) CU(cudaMemsetAsync(s->ingest.d_totals.get(), 0, 4 * sizeof(unsigned long long), s->stream.get()));
     memset(&s->st, 0, sizeof s->st);
     return HS_OK;
 }
@@ -630,15 +606,15 @@ int mix_finalize(MixEngine &m, cudaStream_t st, std::vector<uint64_t> &out, uint
         // collects, sorts and dedups; state and the s smallest come back together.  Anything unusual --
         // the set overflowed, fewer than s values below tau, a crowded histogram bin -- is left to the
         // iterative path below, which starts from the same device state.
-        CU(launch_mix_select(m.view(~0ull), m.s, m.use64, m.d_hist, m.d_cand, m.sel_pad, m.d_scratch, st));
+        CU(launch_mix_select(m.view(~0ull), m.s, m.use64, m.d_hist.get(), m.d_cand.get(), m.sel_pad, m.d_scratch.get(), st));
         n_launches += 4;
-        CU(cudaMemcpyAsync(m.h_cand, m.d_cand, (size_t)m.s * 8, cudaMemcpyDeviceToHost, st));
+        CU(cudaMemcpyAsync(m.h_cand.get(), m.d_cand.get(), (size_t)m.s * 8, cudaMemcpyDeviceToHost, st));
         int rc = m.sync_state(st);
         if (rc) return rc;
-        const MixState &hs_ = *m.h_state;
+        const MixState &hs_ = *m.h_state.get();
         if (!hs_.overflow && !hs_.sel_too_many && hs_.n_out <= m.sel_pad && (hs_.n_unique >= m.s || hs_.tau == ~0ull)) {
             const uint32_t nu = std::min(hs_.n_unique, m.s);
-            out.assign(m.h_cand, m.h_cand + nu);
+            out.assign(m.h_cand.get(), m.h_cand.get() + nu);
             if (hs_.has_max && out.size() < m.s) out.push_back(~0ull);  // hash == 2^64-1 present
             return HS_OK;
         }
@@ -646,8 +622,8 @@ int mix_finalize(MixEngine &m, cudaStream_t st, std::vector<uint64_t> &out, uint
     for (int round = 0; round < 40; round++) {
         int rc = m.sync_state(st);
         if (rc) return rc;
-        if (m.h_state->overflow) {  // too many distinct values below tau: lower it and re-offer
-            const uint64_t nt = m.h_state->tau >> 4;
+        if (m.h_state.get()->overflow) {  // too many distinct values below tau: lower it and re-offer
+            const uint64_t nt = m.h_state.get()->tau >> 4;
             rc = m.reset(st, nt ? nt : 1, false);
             if (rc) return rc;
             m.passes++;
@@ -655,18 +631,18 @@ int mix_finalize(MixEngine &m, cudaStream_t st, std::vector<uint64_t> &out, uint
             if (rc) return rc;
             continue;
         }
-        const uint64_t tau = m.h_state->tau;
-        const uint64_t *live = m.d_set[m.h_state->cur & 1u];
+        const uint64_t tau = m.h_state.get()->tau;
+        const uint64_t *live = m.d_set[m.h_state.get()->cur & 1u].get();
         // distinct values <= tau (older, larger ones may linger from before tau dropped)
         uint64_t thr = tau;
         uint32_t M = 0;
         for (int iter = 0; iter < 64; iter++) {
             CU(cudaMemsetAsync(m.field(offsetof(MixState, n_out)), 0, sizeof(uint32_t), st));
-            CU(launch_mix_collect(live, m.cap, thr, m.d_cand, m.cand_cap, m.field(offsetof(MixState, n_out)), st));
+            CU(launch_mix_collect(live, m.cap, thr, m.d_cand.get(), m.cand_cap, m.field(offsetof(MixState, n_out)), st));
             n_launches++;
             rc = m.sync_state(st);
             if (rc) return rc;
-            M = m.h_state->n_out;
+            M = m.h_state.get()->n_out;
             if (M <= m.cand_cap && (M >= m.s || thr == tau)) break;
             if (M > m.cand_cap) {
                 // aim for ~1.5 s candidates assuming hashes are uniform below thr
@@ -690,16 +666,16 @@ int mix_finalize(MixEngine &m, cudaStream_t st, std::vector<uint64_t> &out, uint
         }
         out.clear();
         if (M) {
-            CU(launch_sort_unique(m.d_cand, M, m.d_scratch, m.field(offsetof(MixState, n_unique)), st));
+            CU(launch_sort_unique(m.d_cand.get(), M, m.d_scratch.get(), m.field(offsetof(MixState, n_unique)), st));
             n_launches++;
             const uint32_t take = std::min(M, m.s);   // >= what is kept (n_unique <= M)
-            CU(cudaMemcpyAsync(m.h_cand, m.d_cand, (size_t)take * 8, cudaMemcpyDeviceToHost, st));
+            CU(cudaMemcpyAsync(m.h_cand.get(), m.d_cand.get(), (size_t)take * 8, cudaMemcpyDeviceToHost, st));
             rc = m.sync_state(st);
             if (rc) return rc;
-            const uint32_t nu = std::min(m.h_state->n_unique, take);
-            out.assign(m.h_cand, m.h_cand + nu);
+            const uint32_t nu = std::min(m.h_state.get()->n_unique, take);
+            out.assign(m.h_cand.get(), m.h_cand.get() + nu);
         }
-        if (m.h_state->has_max && out.size() < m.s) out.push_back(~0ull);  // hash == 2^64-1 present
+        if (m.h_state.get()->has_max && out.size() < m.s) out.push_back(~0ull);  // hash == 2^64-1 present
         return HS_OK;
     }
     return fail(HS_ECUDA, "mixture threshold search did not settle");
@@ -719,7 +695,7 @@ int collect_stream_ms(hs_screen *s)
     float total = 0;
     for (size_t i = 0; i < s->ev_used; i++) {
         float ms = 0;
-        CU(cudaEventElapsedTime(&ms, s->ev_pool[i].first, s->ev_pool[i].second));
+        CU(cudaEventElapsedTime(&ms, s->ev_pool[i].first.get(), s->ev_pool[i].second.get()));
         total += ms;
     }
     s->st.ms_stream = total;
@@ -951,14 +927,7 @@ HS_API int hs_db_ref(const hs_db *db, uint64_t i, const char **name, const char 
     if (n_hashes) *n_hashes = db->offsets[i + 1] - db->offsets[i];
     return HS_OK;
 }
-HS_API void hs_db_free(hs_db *db)
-{
-    if (!db) return;
-    cudaSetDevice(db->device);
-    cudaFree(db->d_buckets); cudaFree(db->d_canon); cudaFree(db->d_next); cudaFree(db->d_offsets); cudaFree(db->d_lengths);
-    cudaFree(db->d_seg_begin); cudaFree(db->d_seg_s); cudaFree(db->d_bloom);
-    delete db;
-}
+HS_API void hs_db_free(hs_db *db) { if (db) delete db; }
 
 // =============================================================================
 // screen
@@ -967,21 +936,19 @@ HS_API int hs_screen_new(hs_db *db, hs_screen **out)
 {
     if (!db || !out) return fail(HS_EINVAL, "null argument");
     ON_DEVICE(db->device);
-    auto *s = new hs_screen();
+    std::unique_ptr<hs_screen> s(new hs_screen());   // a failed step below deletes the half-built handle
     s->db = db;
     const uint64_t N = std::max<uint64_t>(db->n_refs, 1), E = std::max<uint64_t>(db->n_entries, 1);
     const uint64_t E4 = (E + 3) / 4 * 4;
-    auto bail = [&](int rc) { hs_screen_free(s); return rc; };
-#define CUB(x) do { cudaError_t e_ = (x); if (e_ != cudaSuccess) { fail(HS_ECUDA, std::string(#x) + ": " + cudaGetErrorString(e_)); return bail(HS_ECUDA); } } while (0)
-    CUB(cudaStreamCreateWithFlags(&s->stream, cudaStreamNonBlocking));
-    s->own_stream = true;
-    CUB(cudaStreamCreateWithFlags(&s->copy_stream, cudaStreamNonBlocking));
-    CUB(cudaMalloc((void **)&s->d_counts, E4 * 4));
-    CUB(cudaMemsetAsync(s->d_counts, 0, E4 * 4, s->stream));
-    CUB(cudaMalloc((void **)&s->d_stats, 2 * ST_COUNT * sizeof(unsigned long long)));
+    CU(s->stream.create());
+    CU(s->copy_stream.create());
+    CU(s->d_counts.grow(E4));
+    CU(cudaMemsetAsync(s->d_counts.get(), 0, E4 * 4, s->stream.get()));
+    CU(s->d_stats.grow(2 * ST_COUNT));
     // the four result columns share one allocation (identity | p-value | shared | median) so that
     // they travel to the host in a single copy
-    CUB(cudaMalloc((void **)&s->d_identity, N * 24));
+    CU(s->d_result.grow(N * 3));
+    s->d_identity = s->d_result.get();
     s->d_pvalue = s->d_identity + N;
     s->d_shared = reinterpret_cast<uint32_t *>(s->d_pvalue + N);
     s->d_median = s->d_shared + N;
@@ -992,29 +959,24 @@ HS_API int hs_screen_new(hs_db *db, hs_screen **out)
     if (const char *e = getenv("HYMET_SCREEN_TOUCHED_CAP")) s->touched_cap = (uint32_t)std::max(1ll, atoll(e));   // tests: force the fallbacks
     if (const char *e = getenv("HYMET_SCREEN_PAIR_CAP")) s->pair_cap = (uint32_t)std::max(1ll, atoll(e));
     if (const char *e = getenv("HYMET_SCREEN_FORCE_UNSETTLED")) s->force_unsettled = atoi(e);
-    CUB(cudaMalloc((void **)&s->d_sparse, sizeof(SparseState)));
-    CUB(cudaMemsetAsync(s->d_sparse, 0, sizeof(SparseState), s->stream));
-    CUB(cudaHostAlloc((void **)&s->h_sparse, sizeof(SparseState), cudaHostAllocDefault));
-    CUB(cudaMalloc((void **)&s->d_touched, (size_t)s->touched_cap * 4));
-    CUB(cudaMalloc((void **)&s->d_depths, (size_t)s->pair_cap * 4));
-    CUB(cudaMalloc((void **)&s->d_hit, N * 16));   // hit | seg_start | seg_fill | plain
+    CU(s->d_sparse.grow(1));
+    CU(cudaMemsetAsync(s->d_sparse.get(), 0, sizeof(SparseState), s->stream.get()));
+    CU(s->h_sparse.grow(1));
+    CU(s->d_touched.grow(s->touched_cap));
+    CU(s->d_depths.grow(s->pair_cap));
+    CU(s->d_ref_rows.grow(N * 4));
+    s->d_hit = s->d_ref_rows.get();
     s->d_seg_start = s->d_hit + N; s->d_seg_fill = s->d_seg_start + N; s->d_plain = s->d_seg_fill + N;
-    CUB(cudaEventCreate(&s->red0));
-    CUB(cudaEventCreate(&s->red1));
-    CUB(cudaEventCreate(&s->red2));
-    CUB(cudaEventCreate(&s->red3));
-    CUB(cudaEventCreate(&s->rst0));
-    CUB(cudaEventCreate(&s->rst1));
-    CUB(cudaHostAlloc((void **)&s->h_result, N * 24, cudaHostAllocDefault));
-    CUB(cudaHostAlloc((void **)&s->h_stats, (ST_COUNT + 4) * sizeof(unsigned long long), cudaHostAllocDefault));
-    CUB(cudaHostAlloc((void **)&s->h_mixture, ((size_t)db->s + 1) * 8, cudaHostAllocDefault));
-#undef CUB
+    for (Event *e : {&s->red0, &s->red1, &s->red2, &s->red3, &s->rst0, &s->rst1}) CU(e->create());
+    CU(s->h_result.grow(N * 24));
+    CU(s->h_stats.grow(ST_COUNT + 4));
+    CU(s->h_mixture.grow((size_t)db->s + 1));
     int rc = s->mix.init(db->s, db->use64);
-    if (rc) return bail(rc);
+    if (rc) return rc;
     s->touched_valid = false;   // nothing recorded yet and counts[] was just cleared: screen_zero need not walk a list
-    rc = screen_zero(s);
-    if (rc) return bail(rc);
-    *out = s;
+    rc = screen_zero(s.get());
+    if (rc) return rc;
+    *out = s.release();
     return HS_OK;
 }
 
@@ -1022,14 +984,9 @@ HS_API int hs_screen_set_stream(hs_screen *s, void *cuda_stream)
 {
     if (!s) return fail(HS_EINVAL, "null handle");
     ON_DEVICE(s->db->device);
-    CU(cudaStreamSynchronize(s->stream));
-    if (s->own_stream) { cudaStreamDestroy(s->stream); s->own_stream = false; }
-    if (cuda_stream) {
-        s->stream = (cudaStream_t)cuda_stream;
-    } else {
-        CU(cudaStreamCreateWithFlags(&s->stream, cudaStreamNonBlocking));
-        s->own_stream = true;
-    }
+    CU(cudaStreamSynchronize(s->stream.get()));
+    if (cuda_stream) s->stream.borrow((cudaStream_t)cuda_stream);
+    else CU(s->stream.create());
     return HS_OK;
 }
 
@@ -1083,26 +1040,26 @@ int feed_host_chunk(hs_screen *s, const uint64_t *seq, const uint32_t *inv, uint
         const uint64_t w1 = std::min(alloc, w0 + kPieceWords);      // tile aligned
         const uint64_t cw1 = std::min(words, w1);                   // words that exist in the host buffer
         if (cw1 > w0) {
-            CU(cudaMemcpyAsync((char *)dseq + w0 * 8, seq + w0, (cw1 - w0) * 8, cudaMemcpyHostToDevice, s->copy_stream));
-            CU(cudaMemcpyAsync((char *)dinv + w0 * 4, inv + w0, (cw1 - w0) * 4, cudaMemcpyHostToDevice, s->copy_stream));
+            CU(cudaMemcpyAsync((char *)dseq + w0 * 8, seq + w0, (cw1 - w0) * 8, cudaMemcpyHostToDevice, s->copy_stream.get()));
+            CU(cudaMemcpyAsync((char *)dinv + w0 * 4, inv + w0, (cw1 - w0) * 4, cudaMemcpyHostToDevice, s->copy_stream.get()));
         }
         if (w1 > cw1) {
             const uint64_t p0 = std::max(cw1, w0);
-            CU(cudaMemsetAsync((char *)dseq + p0 * 8, 0, (w1 - p0) * 8, s->copy_stream));
-            CU(cudaMemsetAsync((char *)dinv + p0 * 4, 0xFF, (w1 - p0) * 4, s->copy_stream));
+            CU(cudaMemsetAsync((char *)dseq + p0 * 8, 0, (w1 - p0) * 8, s->copy_stream.get()));
+            CU(cudaMemsetAsync((char *)dinv + p0 * 4, 0xFF, (w1 - p0) * 4, s->copy_stream.get()));
         }
         if (s->copy_ev_used == s->copy_evs.size()) {
-            cudaEvent_t e;
-            CU(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-            s->copy_evs.push_back(e);
+            Event e;
+            CU(e.create(cudaEventDisableTiming));
+            s->copy_evs.push_back(std::move(e));
         }
-        cudaEvent_t ev = s->copy_evs[s->copy_ev_used++];
-        CU(cudaEventRecord(ev, s->copy_stream));
-        CU(cudaStreamWaitEvent(s->stream, ev, 0));
+        cudaEvent_t ev = s->copy_evs[s->copy_ev_used++].get();
+        CU(cudaEventRecord(ev, s->copy_stream.get()));
+        CU(cudaStreamWaitEvent(s->stream.get(), ev, 0));
         int rc = launch_chunk(s, c, true, true, w0 / kTileWords, w1 / kTileWords);
         if (rc) return rc;
     }
-    if (done_ev) CU(cudaEventRecord(done_ev, s->copy_stream));  // the host buffer may be reused
+    if (done_ev) CU(cudaEventRecord(done_ev, s->copy_stream.get()));  // the host buffer may be reused
     return HS_OK;
 }
 
@@ -1116,7 +1073,7 @@ int feed_span_device(hs_screen *s, const char *text, size_t len, cudaEvent_t hos
     Ingest::Slot *sl = nullptr;
     {
         std::lock_guard<std::mutex> lk(s->mu);
-        int rc = in.ensure(len, s->stream);
+        int rc = in.ensure(len, s->stream.get());
         if (rc) return rc;
     }
     int rc = in.slot_for(len, &sl);   // may wait for the GPU (outside the lock)
@@ -1129,15 +1086,15 @@ int feed_span_device(hs_screen *s, const char *text, size_t len, cudaEvent_t hos
     void *dseq = nullptr, *dinv = nullptr;
     CU(s->arena.alloc(alloc * 8, &dseq));
     CU(s->arena.alloc(alloc * 4, &dinv));
-    CU(cudaMemcpyAsync(sl->raw, text, len, cudaMemcpyHostToDevice, s->copy_stream));
-    CU(cudaEventRecord(sl->copied, s->copy_stream));
-    if (host_free_ev) CU(cudaEventRecord(host_free_ev, s->copy_stream));
-    CU(cudaStreamWaitEvent(s->stream, sl->copied, 0));
+    CU(cudaMemcpyAsync(sl->raw.get(), text, len, cudaMemcpyHostToDevice, s->copy_stream.get()));
+    CU(cudaEventRecord(sl->copied.get(), s->copy_stream.get()));
+    if (host_free_ev) CU(cudaEventRecord(host_free_ev, s->copy_stream.get()));
+    CU(cudaStreamWaitEvent(s->stream.get(), sl->copied.get(), 0));
     FaScratch sc = in.sc;
     sc.chunk_positions = d_npos;
-    CU(launch_fasta_to_codes(sl->raw, (uint32_t)len, sl->codes, sc, s->stream));
-    CU(launch_pack_codes_dyn(sl->codes, d_npos, (uint64_t *)dseq, (uint32_t *)dinv, alloc, s->stream));
-    CU(cudaEventRecord(sl->done, s->stream));
+    CU(launch_fasta_to_codes(sl->raw.get(), (uint32_t)len, sl->codes.get(), sc, s->stream.get()));
+    CU(launch_pack_codes_dyn(sl->codes.get(), d_npos, (uint64_t *)dseq, (uint32_t *)dinv, alloc, s->stream.get()));
+    CU(cudaEventRecord(sl->done.get(), s->stream.get()));
     s->st.n_launches += 7;
     s->st.h2d_bytes += len;
     Chunk c{(const uint64_t *)dseq, (const uint32_t *)dinv, (uint64_t)len, d_npos};
@@ -1181,8 +1138,8 @@ int feed_text_impl(hs_screen *s, const char *text, size_t n, int threads)
     const size_t need = (size_t)threads * 2;
     while (s->staging.size() < need) {
         Staging g;
-        CU(cudaEventCreateWithFlags(&g.free_ev, cudaEventDisableTiming));
-        s->staging.push_back(g);
+        CU(g.free_ev.create(cudaEventDisableTiming));
+        s->staging.push_back(std::move(g));
     }
     std::atomic<size_t> next{0};
     std::atomic<int> rc_all{HS_OK};
@@ -1218,20 +1175,21 @@ int feed_text_impl(hs_screen *s, const char *text, size_t n, int threads)
             const uint64_t bound = pack_words_bound(len);
             int rc = HS_OK;
             if (g.cap_words < bound) {
-                if (g.seq) { cudaEventSynchronize(g.free_ev); cudaFreeHost(g.seq); cudaFreeHost(g.inv); g.seq = nullptr; g.inv = nullptr; }
-                g.cap_words = bound + bound / 8;
-                if (cudaHostAlloc((void **)&g.seq, g.cap_words * 8, cudaHostAllocDefault) != cudaSuccess ||
-                    cudaHostAlloc((void **)&g.inv, g.cap_words * 4, cudaHostAllocDefault) != cudaSuccess) {
-                    g.cap_words = 0;
+                if (g.seq.get()) cudaEventSynchronize(g.free_ev.get());
+                g.seq.reset(); g.inv.reset();   // both go before either grows
+                g.cap_words = 0;
+                const uint64_t cap = bound + bound / 8;
+                if (g.seq.grow(cap) != cudaSuccess || g.inv.grow(cap) != cudaSuccess)
                     rc = fail(HS_ENOMEM, "pinned staging allocation failed");
-                }
+                else
+                    g.cap_words = cap;
             } else {
-                cudaEventSynchronize(g.free_ev);  // previous H2D from this buffer has finished
+                cudaEventSynchronize(g.free_ev.get());  // previous H2D from this buffer has finished
             }
             PackStats ps;
             if (rc == HS_OK) {
                 const double t0 = now_s();
-                pack_text_span(text + spans[i].first, len, g.seq, g.inv, &ps);
+                pack_text_span(text + spans[i].first, len, g.seq.get(), g.inv.get(), &ps);
                 const double t1 = now_s();
                 my_ms = 1e3 * (t1 - t0);
                 pack_us_per_span.store((pack_us_per_span.load() * 3 + (int)(1e3 * my_ms)) / 4);
@@ -1239,7 +1197,7 @@ int feed_text_impl(hs_screen *s, const char *text, size_t n, int threads)
                 const double t2 = now_s();
                 s->st.n_bases += ps.n_seq_bases;
                 s->st.n_records += ps.n_records;
-                rc = feed_host_chunk(s, g.seq, g.inv, ps.n_positions, g.free_ev);
+                rc = feed_host_chunk(s, g.seq.get(), g.inv.get(), ps.n_positions, g.free_ev.get());
                 if (g_debug_timing)
                     fprintf(stderr, "[hs] span %zu thr %d: %zu B pack %.2f ms (%.2f GB/s) lock-wait %.2f ms feed %.2f ms\n", i, t,
                             len, 1e3 * (t1 - t0), len / (t1 - t0) / 1e9, 1e3 * (t2 - t1), 1e3 * (now_s() - t2));
@@ -1270,7 +1228,7 @@ int feed_text_impl(hs_screen *s, const char *text, size_t n, int threads)
                 if (nx >= spans.size()) break;
                 int busy = 0;
                 for (int q = 0; q < Ingest::kSlots; q++)
-                    if (s->ingest.slots[q].done && cudaEventQuery(s->ingest.slots[q].done) == cudaErrorNotReady) busy++;
+                    if (s->ingest.slots[q].done.get() && cudaEventQuery(s->ingest.slots[q].done.get()) == cudaErrorNotReady) busy++;
                 cudaGetLastError();
                 const int alive = packers_alive.load();
                 const double rest_ms = (double)(spans.size() - nx) * pack_us_per_span.load() * 1e-3 / (alive > 0 ? alive : 1);
@@ -1315,8 +1273,8 @@ int feed_text_impl(hs_screen *s, const char *text, size_t n, int threads)
     if (rc_all == HS_OK && next.load() < spans.size()) {
         while (s->staging.size() < 2) {
             Staging g;
-            CU(cudaEventCreateWithFlags(&g.free_ev, cudaEventDisableTiming));
-            s->staging.push_back(g);
+            CU(g.free_ev.create(cudaEventDisableTiming));
+            s->staging.push_back(std::move(g));
         }
         worker(0, false);
     }
@@ -1368,14 +1326,14 @@ int feed_file_stream(hs_screen *s, int fd, uint64_t size, int threads, uint64_t 
     if ((uint64_t)T > n_blocks) T = (int)n_blocks;
     const size_t cap = (size_t)(B + B / 2 + 4096);
     if (s->ring.slot_cap < cap || s->ring.free_ev.size() < (size_t)2 * T) {
-        CU(cudaStreamSynchronize(s->copy_stream));
-        s->ring.release();
-        CU(cudaHostAlloc((void **)&s->ring.base, cap * 2 * T, cudaHostAllocDefault));
+        CU(cudaStreamSynchronize(s->copy_stream.get()));
+        s->ring = FileRing();
+        CU(s->ring.base.grow(cap * 2 * T));
         s->ring.slot_cap = cap;
         for (int i = 0; i < 2 * T; i++) {
-            cudaEvent_t e;
-            CU(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-            s->ring.free_ev.push_back(e);
+            Event e;
+            CU(e.create(cudaEventDisableTiming));
+            s->ring.free_ev.push_back(std::move(e));
         }
     }
     std::atomic<uint64_t> next{0};
@@ -1393,8 +1351,8 @@ int feed_file_stream(hs_screen *s, int fd, uint64_t size, int threads, uint64_t 
             const uint64_t j = next.fetch_add(1);
             if (j >= n_blocks || rc_all.load() != HS_OK) break;
             const size_t slot = (size_t)t * 2 + (size_t)(flip ^= 1);
-            char *buf = s->ring.base + slot * s->ring.slot_cap;
-            if (cudaEventSynchronize(s->ring.free_ev[slot]) != cudaSuccess) { bail(fail(HS_ECUDA, "ring event")); break; }
+            char *buf = s->ring.base.get() + slot * s->ring.slot_cap;
+            if (cudaEventSynchronize(s->ring.free_ev[slot].get()) != cudaSuccess) { bail(fail(HS_ECUDA, "ring event")); break; }
             const double t0 = now_s();
             const uint64_t nominal_begin = range_begin + j * B;
             const uint64_t off0 = nominal_begin ? nominal_begin - 1 : 0;   // one byte early: is there a newline before the block?
@@ -1444,7 +1402,7 @@ int feed_file_stream(hs_screen *s, int fd, uint64_t size, int threads, uint64_t 
                 rc = feed_text_impl(s, rec.data(), rec.size(), 1);
             } else {
                 std::lock_guard<std::mutex> lk(s->ingest_mu);
-                rc = feed_span_device(s, buf + b, e - b, s->ring.free_ev[slot]);
+                rc = feed_span_device(s, buf + b, e - b, s->ring.free_ev[slot].get());
             }
             if (g_debug_timing)
                 fprintf(stderr, "[hs] block %llu reader %d: %zu B read %.2f ms (%.2f GB/s) submit %.2f ms%s\n", (unsigned long long)j,
@@ -1619,7 +1577,7 @@ namespace {
 // what hs_screen_flush does once the stream has been synchronised: counters, timings, state
 int flush_epilogue(hs_screen *s, bool parsed)
 {
-    unsigned long long *h = s->h_stats, *t = s->h_stats + ST_COUNT;
+    unsigned long long *h = s->h_stats.get(), *t = s->h_stats.get() + ST_COUNT;
     if (parsed) { s->st.n_positions += t[0]; s->st.n_bases += t[1]; s->st.n_records += t[2]; }
     s->st.n_valid_kmers = h[ST_VALID]; s->st.n_probes = h[ST_PROBES]; s->st.n_bucket_reads = h[ST_BUCKETS];
     s->st.n_hits = h[ST_HITS]; s->st.n_mix_inserts = h[ST_MIXINS];
@@ -1630,7 +1588,7 @@ int flush_epilogue(hs_screen *s, bool parsed)
     if (rc) return rc;
     if (s->rst_pending) {
         float ms = 0;
-        CU(cudaEventElapsedTime(&ms, s->rst0, s->rst1));
+        CU(cudaEventElapsedTime(&ms, s->rst0.get(), s->rst1.get()));
         s->st.ms_reset = ms;
         s->rst_pending = false;
     }
@@ -1654,18 +1612,18 @@ HS_API int hs_screen_flush_async(hs_screen *s)
     if (s->flushed || s->flush_pending) return HS_OK;
     if (!s->mix.fast_select) return hs_screen_flush(s);
     std::lock_guard<std::mutex> lk(s->mu);
-    CU(cudaEventRecord(s->red0, s->stream));
+    CU(cudaEventRecord(s->red0.get(), s->stream.get()));
     const bool parsed = s->ingest.ready && s->ingest.counters_used;
-    CU(cudaMemcpyAsync(s->h_stats, s->d_stats, ST_COUNT * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s->stream));
+    CU(cudaMemcpyAsync(s->h_stats.get(), s->d_stats.get(), ST_COUNT * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s->stream.get()));
     if (parsed) {
-        CU(cudaMemcpyAsync(s->h_stats + ST_COUNT, s->ingest.d_totals, 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s->stream));
-        CU(cudaMemsetAsync(s->ingest.d_totals, 0, 4 * sizeof(unsigned long long), s->stream));
+        CU(cudaMemcpyAsync(s->h_stats.get() + ST_COUNT, s->ingest.d_totals.get(), 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s->stream.get()));
+        CU(cudaMemsetAsync(s->ingest.d_totals.get(), 0, 4 * sizeof(unsigned long long), s->stream.get()));
     }
     MixEngine &m = s->mix;
-    CU(launch_mix_select(m.view(~0ull), m.s, m.use64, m.d_hist, m.d_cand, m.sel_pad, m.d_scratch, s->stream));
+    CU(launch_mix_select(m.view(~0ull), m.s, m.use64, m.d_hist.get(), m.d_cand.get(), m.sel_pad, m.d_scratch.get(), s->stream.get()));
     s->st.n_launches += 4;
-    CU(cudaMemcpyAsync(m.h_cand, m.d_cand, (size_t)m.s * 8, cudaMemcpyDeviceToHost, s->stream));
-    CU(cudaMemcpyAsync(m.h_state, m.d_state, sizeof(MixState), cudaMemcpyDeviceToHost, s->stream));
+    CU(cudaMemcpyAsync(m.h_cand.get(), m.d_cand.get(), (size_t)m.s * 8, cudaMemcpyDeviceToHost, s->stream.get()));
+    CU(cudaMemcpyAsync(m.h_state.get(), m.d_state.get(), sizeof(MixState), cudaMemcpyDeviceToHost, s->stream.get()));
     s->flush_pending = true;
     s->flush_parsed = parsed;
     return HS_OK;
@@ -1680,24 +1638,24 @@ HS_API int hs_screen_flush(hs_screen *s)
     if (s->flush_pending) {
         // an enqueued selection is abandoned (its verdict was "not settled", or the caller changed its mind):
         // the iterative finaliser below starts from the same device state
-        CU(cudaStreamSynchronize(s->stream));
+        CU(cudaStreamSynchronize(s->stream.get()));
         if (s->flush_parsed) {   // the parser totals were folded into h_stats and cleared on the device: keep them
-            unsigned long long *t = s->h_stats + ST_COUNT;
+            unsigned long long *t = s->h_stats.get() + ST_COUNT;
             s->st.n_positions += t[0]; s->st.n_bases += t[1]; s->st.n_records += t[2];
         }
         s->flush_pending = false;
     }
-    CU(cudaEventRecord(s->red0, s->stream));
+    CU(cudaEventRecord(s->red0.get(), s->stream.get()));
     // the counters are final once the streaming launches are (re-offer passes count elsewhere): fetch
     // them with the first synchronisation of the mixture finaliser instead of one of their own
-    unsigned long long *h = s->h_stats, *t = s->h_stats + ST_COUNT;
+    unsigned long long *h = s->h_stats.get(), *t = s->h_stats.get() + ST_COUNT;
     const bool parsed = s->ingest.ready && s->ingest.counters_used;
-    CU(cudaMemcpyAsync(h, s->d_stats, ST_COUNT * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s->stream));
+    CU(cudaMemcpyAsync(h, s->d_stats.get(), ST_COUNT * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s->stream.get()));
     if (parsed) {
-        CU(cudaMemcpyAsync(t, s->ingest.d_totals, 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s->stream));
-        CU(cudaMemsetAsync(s->ingest.d_totals, 0, 4 * sizeof(unsigned long long), s->stream));  // folded: do not fold twice
+        CU(cudaMemcpyAsync(t, s->ingest.d_totals.get(), 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s->stream.get()));
+        CU(cudaMemsetAsync(s->ingest.d_totals.get(), 0, 4 * sizeof(unsigned long long), s->stream.get()));  // folded: do not fold twice
     }
-    int rc = mix_finalize(s->mix, s->stream, s->mixture, s->st.n_launches, [&]() -> int {
+    int rc = mix_finalize(s->mix, s->stream.get(), s->mixture, s->st.n_launches, [&]() -> int {
         for (const Chunk &c : s->chunks) {
             int r = launch_chunk(s, c, false, true);
             if (r) return r;
@@ -1706,12 +1664,12 @@ HS_API int hs_screen_flush(hs_screen *s)
         return HS_OK;
     });
     if (rc) return rc;
-    CU(cudaEventRecord(s->red1, s->stream));
-    CU(cudaEventSynchronize(s->red1));   // mix_finalize ended on a synchronisation: nothing is left to wait for
+    CU(cudaEventRecord(s->red1.get(), s->stream.get()));
+    CU(cudaEventSynchronize(s->red1.get()));   // mix_finalize ended on a synchronisation: nothing is left to wait for
     rc = flush_epilogue(s, parsed);
     if (rc) return rc;
     float ms = 0;
-    CU(cudaEventElapsedTime(&ms, s->red0, s->red1));
+    CU(cudaEventElapsedTime(&ms, s->red0.get(), s->red1.get()));
     s->st.ms_reduce = ms;
     s->flushed = true;
     return HS_OK;
@@ -1720,7 +1678,7 @@ HS_API int hs_screen_flush(hs_screen *s)
 HS_API int hs_screen_counts_devptr(hs_screen *s, void **d_counts, uint64_t *n)
 {
     if (!s || !d_counts || !n) return fail(HS_EINVAL, "null argument");
-    *d_counts = s->d_counts;
+    *d_counts = s->d_counts.get();
     *n = s->db->n_entries;
     // whoever asks for the raw vector may add to it (the dense all-reduce): the record of which
     // counts are non-zero no longer covers it, so reduction and reset take their dense forms
@@ -1734,10 +1692,10 @@ HS_API int hs_screen_counts_compact_async(hs_screen *s, void *d_pairs, uint32_t 
     ON_DEVICE(s->db->device);
     // no flush needed: counts[] is final, in stream order, as soon as the last feed has been enqueued
     // (the mixture finaliser never touches it), so the exchange can start underneath hs_screen_flush
-    CU(cudaMemsetAsync(d_n_out, 0, sizeof(uint32_t), s->stream));
+    CU(cudaMemsetAsync(d_n_out, 0, sizeof(uint32_t), s->stream.get()));
     SparseView sp = sparse_view(s);
     if (!s->touched_valid) sp.touched = nullptr;
-    CU(launch_counts_compact(sp, s->d_counts, s->db->n_entries, (unsigned long long *)d_pairs, cap, (uint32_t *)d_n_out, s->stream));
+    CU(launch_counts_compact(sp, s->d_counts.get(), s->db->n_entries, (unsigned long long *)d_pairs, cap, (uint32_t *)d_n_out, s->stream.get()));
     s->st.n_launches += sp.touched ? 2 : 1;
     return HS_OK;
 }
@@ -1748,8 +1706,8 @@ HS_API int hs_screen_counts_absorb(hs_screen *s, const void *d_rows, uint32_t n_
     ON_DEVICE(s->db->device);
     SparseView sp = sparse_view(s);
     if (!s->touched_valid) sp.touched = nullptr;
-    CU(launch_counts_absorb(sp, s->d_counts, s->db->n_entries, (const unsigned long long *)d_rows, n_rows, cap, skip_row,
-                            s->db->sm, s->stream));
+    CU(launch_counts_absorb(sp, s->d_counts.get(), s->db->n_entries, (const unsigned long long *)d_rows, n_rows, cap, skip_row,
+                            s->db->sm, s->stream.get()));
     s->st.n_launches++;
     return HS_OK;
 }
@@ -1768,10 +1726,10 @@ void mixture_row(const hs_screen *s, uint64_t *row)
 // what hs_screen_mixture_merge_device left in h_sparse / h_mixture becomes the screen's mixture
 void adopt_merged_mixture(hs_screen *s)
 {
-    const uint32_t nm = std::min<uint32_t>(s->h_sparse->n_mix, s->db->s);
-    s->mixture.assign(s->h_mixture, s->h_mixture + nm);
+    const uint32_t nm = std::min<uint32_t>(s->h_sparse.get()->n_mix, s->db->s);
+    s->mixture.assign(s->h_mixture.get(), s->h_mixture.get() + nm);
     s->st.n_mixture = nm;
-    s->st.set_size = s->h_sparse->set_size[0];
+    s->st.set_size = s->h_sparse.get()->set_size[0];
 }
 
 }  // namespace
@@ -1799,61 +1757,56 @@ HS_API int hs_screen_absorb_screens(hs_screen *dst, hs_screen *const *src, uint3
     // [n | (entry id << 32 | count) ...] is built on its own device, copied into row 1 + i of a buffer on
     // dst's device (row 0, dst's own, is empty and skipped), and hs_screen_counts_absorb and
     // hs_screen_mixture_merge_device take it from there.
-    std::vector<unsigned long long *> rec(n_src, nullptr);
-    unsigned long long *rows = nullptr;
-    const int rc = [&]() -> int {
-        std::vector<uint32_t> n(n_src);
-        uint32_t cap = 1;
-        for (uint32_t i = 0; i < n_src; i++) {
-            hs_screen *s = src[i];
-            ON_DEVICE(s->db->device);
-            CU(cudaMemcpyAsync(s->h_sparse, s->d_sparse, sizeof(SparseState), cudaMemcpyDeviceToHost, s->stream));
-            CU(cudaStreamSynchronize(s->stream));
-            const bool listed = s->sparse_enabled && s->touched_valid && s->h_sparse->n_touched <= s->touched_cap;
-            const uint64_t rcap = listed ? s->h_sparse->n_touched : db->n_entries;
-            CU(cudaMalloc((void **)&rec[i], (rcap + 1) * 8));
-            CU(cudaMemsetAsync(rec[i], 0, 8, s->stream));
-            int r = hs_screen_counts_compact_async(s, rec[i] + 1, (uint32_t)rcap, rec[i]);
-            if (r) return r;
-            CU(cudaMemcpyAsync(&n[i], rec[i], sizeof(uint32_t), cudaMemcpyDeviceToHost, s->stream));
-            CU(cudaStreamSynchronize(s->stream));
-            cap = std::max(cap, n[i]);
-        }
-        ON_DEVICE(db->device);
-        const size_t R = (size_t)n_src + 1, stride = (size_t)cap + 1, mstride = (size_t)db->s + 1;
-        CU(cudaMalloc((void **)&rows, R * (stride + mstride) * 8));
-        unsigned long long *mix = rows + R * stride;
-        CU(cudaMemsetAsync(rows, 0, 8, dst->stream));
-        for (uint32_t i = 0; i < n_src; i++)
-            CU(cudaMemcpyPeerAsync(rows + (i + 1) * stride, db->device, rec[i], src[i]->db->device, ((size_t)n[i] + 1) * 8,
-                                   dst->stream));
-        std::vector<uint64_t> h_mix(R * mstride);
-        mixture_row(dst, h_mix.data());
-        for (uint32_t i = 0; i < n_src; i++) mixture_row(src[i], h_mix.data() + (i + 1) * mstride);
-        CU(cudaMemcpyAsync(mix, h_mix.data(), h_mix.size() * 8, cudaMemcpyHostToDevice, dst->stream));
-        int r = hs_screen_counts_absorb(dst, rows, (uint32_t)R, cap, 0);
-        if (!r) r = hs_screen_mixture_merge_device(dst, mix, (uint32_t)R);
+    // temporaries on several devices: each is released on its own when the call returns
+    std::vector<DevBuf<unsigned long long>> rec(n_src);
+    DevBuf<unsigned long long> rows_buf;
+    std::vector<uint32_t> n(n_src);
+    uint32_t cap = 1;
+    for (uint32_t i = 0; i < n_src; i++) {
+        hs_screen *s = src[i];
+        ON_DEVICE(s->db->device);
+        CU(cudaMemcpyAsync(s->h_sparse.get(), s->d_sparse.get(), sizeof(SparseState), cudaMemcpyDeviceToHost, s->stream.get()));
+        CU(cudaStreamSynchronize(s->stream.get()));
+        const bool listed = s->sparse_enabled && s->touched_valid && s->h_sparse.get()->n_touched <= s->touched_cap;
+        const uint64_t rcap = listed ? s->h_sparse.get()->n_touched : db->n_entries;
+        CU(rec[i].grow(rcap + 1));
+        CU(cudaMemsetAsync(rec[i].get(), 0, 8, s->stream.get()));
+        int r = hs_screen_counts_compact_async(s, rec[i].get() + 1, (uint32_t)rcap, rec[i].get());
         if (r) return r;
-        // the merged mixture and its set size now, as for a single screen after flush (stats read before finish)
-        CU(cudaMemcpyAsync(dst->h_sparse, dst->d_sparse, sizeof(SparseState), cudaMemcpyDeviceToHost, dst->stream));
-        if (db->s) CU(cudaMemcpyAsync(dst->h_mixture, dst->d_mixture, (size_t)db->s * 8, cudaMemcpyDeviceToHost, dst->stream));
-        CU(cudaStreamSynchronize(dst->stream));
-        adopt_merged_mixture(dst);
-        for (uint32_t i = 0; i < n_src; i++) {
-            const hs_stats_t &t = src[i]->st;
-            dst->st.n_bases += t.n_bases; dst->st.n_records += t.n_records; dst->st.n_positions += t.n_positions;
-            dst->st.n_valid_kmers += t.n_valid_kmers; dst->st.n_probes += t.n_probes;
-            dst->st.n_bucket_reads += t.n_bucket_reads; dst->st.n_hits += t.n_hits;
-            dst->st.n_mix_inserts += t.n_mix_inserts; dst->st.h2d_bytes += t.h2d_bytes;
-            dst->st.n_launches += t.n_launches;
-            dst->st.ms_stream = std::max(dst->st.ms_stream, t.ms_stream);
-        }
-        return HS_OK;
-    }();
-    if (rows && cudaSetDevice(db->device) == cudaSuccess) cudaFree(rows);
+        CU(cudaMemcpyAsync(&n[i], rec[i].get(), sizeof(uint32_t), cudaMemcpyDeviceToHost, s->stream.get()));
+        CU(cudaStreamSynchronize(s->stream.get()));
+        cap = std::max(cap, n[i]);
+    }
+    ON_DEVICE(db->device);
+    const size_t R = (size_t)n_src + 1, stride = (size_t)cap + 1, mstride = (size_t)db->s + 1;
+    CU(rows_buf.grow(R * (stride + mstride)));
+    unsigned long long *rows = rows_buf.get(), *mix = rows + R * stride;
+    CU(cudaMemsetAsync(rows, 0, 8, dst->stream.get()));
     for (uint32_t i = 0; i < n_src; i++)
-        if (rec[i] && cudaSetDevice(src[i]->db->device) == cudaSuccess) cudaFree(rec[i]);
-    return rc;
+        CU(cudaMemcpyPeerAsync(rows + (i + 1) * stride, db->device, rec[i].get(), src[i]->db->device, ((size_t)n[i] + 1) * 8,
+                               dst->stream.get()));
+    std::vector<uint64_t> h_mix(R * mstride);
+    mixture_row(dst, h_mix.data());
+    for (uint32_t i = 0; i < n_src; i++) mixture_row(src[i], h_mix.data() + (i + 1) * mstride);
+    CU(cudaMemcpyAsync(mix, h_mix.data(), h_mix.size() * 8, cudaMemcpyHostToDevice, dst->stream.get()));
+    int r = hs_screen_counts_absorb(dst, rows, (uint32_t)R, cap, 0);
+    if (!r) r = hs_screen_mixture_merge_device(dst, mix, (uint32_t)R);
+    if (r) return r;
+    // the merged mixture and its set size now, as for a single screen after flush (stats read before finish)
+    CU(cudaMemcpyAsync(dst->h_sparse.get(), dst->d_sparse.get(), sizeof(SparseState), cudaMemcpyDeviceToHost, dst->stream.get()));
+    if (db->s) CU(cudaMemcpyAsync(dst->h_mixture.get(), dst->d_mixture.get(), (size_t)db->s * 8, cudaMemcpyDeviceToHost, dst->stream.get()));
+    CU(cudaStreamSynchronize(dst->stream.get()));
+    adopt_merged_mixture(dst);
+    for (uint32_t i = 0; i < n_src; i++) {
+        const hs_stats_t &t = src[i]->st;
+        dst->st.n_bases += t.n_bases; dst->st.n_records += t.n_records; dst->st.n_positions += t.n_positions;
+        dst->st.n_valid_kmers += t.n_valid_kmers; dst->st.n_probes += t.n_probes;
+        dst->st.n_bucket_reads += t.n_bucket_reads; dst->st.n_hits += t.n_hits;
+        dst->st.n_mix_inserts += t.n_mix_inserts; dst->st.h2d_bytes += t.h2d_bytes;
+        dst->st.n_launches += t.n_launches;
+        dst->st.ms_stream = std::max(dst->st.ms_stream, t.ms_stream);
+    }
+    return HS_OK;
 }
 
 HS_API int hs_screen_mixture_get(hs_screen *s, uint64_t *hashes, uint32_t *n)
@@ -1871,8 +1824,8 @@ HS_API int hs_screen_mixture_record(hs_screen *s, void *d_record)
     ON_DEVICE(s->db->device);
     if (s->flush_pending) {
         // the selection is still on its way: the record is cut out of it on the device, verdict included
-        CU(launch_mix_record(s->mix.view(~0ull), s->db->s, s->mix.sel_pad, s->mix.d_cand, (unsigned long long *)d_record,
-                             s->force_unsettled, s->stream));
+        CU(launch_mix_record(s->mix.view(~0ull), s->db->s, s->mix.sel_pad, s->mix.d_cand.get(), (unsigned long long *)d_record,
+                             s->force_unsettled, s->stream.get()));
         s->force_unsettled = 0;
         s->st.n_launches++;
         return HS_OK;
@@ -1880,8 +1833,8 @@ HS_API int hs_screen_mixture_record(hs_screen *s, void *d_record)
     if (!s->flushed) return fail(HS_ESTATE, "call hs_screen_flush first");
     // what every rank contributes to the mixture all-gather: it goes up from pinned memory on the
     // screen's stream and the record stays on the device for the collective
-    mixture_row(s, s->h_mixture);
-    CU(cudaMemcpyAsync(d_record, s->h_mixture, ((size_t)s->db->s + 1) * 8, cudaMemcpyHostToDevice, s->stream));
+    mixture_row(s, s->h_mixture.get());
+    CU(cudaMemcpyAsync(d_record, s->h_mixture.get(), ((size_t)s->db->s + 1) * 8, cudaMemcpyHostToDevice, s->stream.get()));
     return HS_OK;
 }
 
@@ -1893,16 +1846,15 @@ HS_API int hs_screen_mixture_merge_device(hs_screen *s, const void *d_rows, uint
     const uint32_t sc = s->db->s;
     uint32_t need = 2;
     while (need < (uint64_t)n_rows * sc) need <<= 1;
-    if (s->merge_cap < need) {
-        cudaFree(s->d_merge_work); cudaFree(s->d_merge_scratch); cudaFree(s->d_mixture);
-        s->d_merge_work = s->d_merge_scratch = s->d_mixture = nullptr;
-        CU(cudaMalloc((void **)&s->d_merge_work, (size_t)need * 8));
-        CU(cudaMalloc((void **)&s->d_merge_scratch, (size_t)need * 8));
-        CU(cudaMalloc((void **)&s->d_mixture, (size_t)std::max<uint32_t>(sc, 1) * 8));
-        s->merge_cap = need;
+    if (s->d_merge_work.cap() < need || s->d_merge_scratch.cap() < need) {
+        s->d_merge_work.reset(); s->d_merge_scratch.reset();   // both go before either grows
+        CU(s->d_merge_work.grow(need));
+        CU(s->d_merge_scratch.grow(need));
     }
-    CU(launch_mixture_merge((const unsigned long long *)d_rows, n_rows, sc, sc, s->db->d_seg_s, (uint32_t)s->db->seg_s.size(),
-                            s->db->use64, s->d_merge_work, need, s->d_merge_scratch, s->d_mixture, s->d_sparse, s->stream));
+    CU(s->d_mixture.grow(std::max<uint32_t>(sc, 1)));
+    CU(launch_mixture_merge((const unsigned long long *)d_rows, n_rows, sc, sc, s->db->d_seg_s.get(), (uint32_t)s->db->seg_s.size(),
+                            s->db->use64, s->d_merge_work.get(), need, s->d_merge_scratch.get(), s->d_mixture.get(),
+                            s->d_sparse.get(), s->stream.get()));
     s->st.n_launches += 3;
     s->mixture_on_device = true;   // finish reads the set sizes from the device and brings the mixture back with the results
     return HS_OK;
@@ -1927,36 +1879,34 @@ int enqueue_reduce(hs_screen *s, bool wta, bool dense)
     const size_t n_seg = db->seg_s.size();
     if (!N) return HS_OK;
     if (!dense) {
-        CU(cudaMemsetAsync(s->d_shared, 0, N * 8, s->stream));   // shared | median are adjacent
+        CU(cudaMemsetAsync(s->d_shared, 0, N * 8, s->stream.get()));   // shared | median are adjacent
         static_assert(offsetof(SparseState, overflow) == offsetof(SparseState, n_hit) + 8, "n_hit, n_pairs, overflow are cleared together");
-        CU(cudaMemsetAsync(&s->d_sparse->n_hit, 0, 3 * sizeof(uint32_t), s->stream));
+        CU(cudaMemsetAsync(&s->d_sparse.get()->n_hit, 0, 3 * sizeof(uint32_t), s->stream.get()));
         SparseReduceArgs a;
         memset(&a, 0, sizeof a);
         a.sp = sparse_view(s);
-        a.counts = s->d_counts; a.next = db->d_next; a.offsets = db->d_offsets; a.n_refs = (uint32_t)N;
-        a.lengths = db->d_lengths; a.seg_begin = db->d_seg_begin; a.n_seg = (uint32_t)n_seg;
+        a.counts = s->d_counts.get(); a.next = db->d_next.get(); a.offsets = db->d_offsets.get(); a.n_refs = (uint32_t)N;
+        a.lengths = db->d_lengths.get(); a.seg_begin = db->d_seg_begin.get(); a.n_seg = (uint32_t)n_seg;
         a.shared = s->d_shared; a.median = s->d_median; a.plain = s->d_plain; a.hit = s->d_hit;
-        a.seg_start = s->d_seg_start; a.seg_fill = s->d_seg_fill; a.depths = s->d_depths; a.pair_cap = s->pair_cap;
+        a.seg_start = s->d_seg_start; a.seg_fill = s->d_seg_fill; a.depths = s->d_depths.get(); a.pair_cap = s->pair_cap;
         a.ref_scale = (E && N <= E) ? (uint64_t)((((unsigned __int128)N) << 64) / ((unsigned __int128)E + 1)) : 0;
-        CU(launch_sparse_reduce(a, wta, db->sm, s->stream));
+        CU(launch_sparse_reduce(a, wta, db->sm, s->stream.get()));
         s->st.n_launches += wta ? 7 : 4;
         return HS_OK;
     }
-    CU(launch_sketch_reduce(db->d_offsets, N, db->d_canon, s->d_counts, nullptr, s->d_shared, s->d_median, db->sm, s->stream));
+    CU(launch_sketch_reduce(db->d_offsets.get(), N, db->d_canon.get(), s->d_counts.get(), nullptr, s->d_shared, s->d_median, db->sm, s->stream.get()));
     s->st.n_launches++;
     if (wta && E) {
-        if (!s->d_winner) {
-            CU(cudaMalloc((void **)&s->d_best_score, E * 8));
-            CU(cudaMalloc((void **)&s->d_best_len, E * 8));
-            CU(cudaMalloc((void **)&s->d_winner, E * 4));
-        }
+        CU(s->d_win.grow(E * 20));
+        auto *best_score = reinterpret_cast<unsigned long long *>(s->d_win.get()), *best_len = best_score + E;
+        auto *winner = reinterpret_cast<uint32_t *>(best_len + E);
         for (size_t j = 0; j < n_seg; j++) {   // -w is a competition among the references of one .msh (S12)
             const uint64_t b = db->seg_begin[j], n = db->seg_begin[j + 1] - b;
             if (!n) continue;
-            CU(launch_winner(db->d_offsets + b, n, db->d_canon, s->d_counts, s->d_shared + b, db->d_lengths + b,
-                             s->d_best_score, s->d_best_len, s->d_winner, E, db->sm, s->stream));
-            CU(launch_sketch_reduce(db->d_offsets + b, n, db->d_canon, s->d_counts, s->d_winner, s->d_shared + b,
-                                    s->d_median + b, db->sm, s->stream));
+            CU(launch_winner(db->d_offsets.get() + b, n, db->d_canon.get(), s->d_counts.get(), s->d_shared + b, db->d_lengths.get() + b,
+                             best_score, best_len, winner, E, db->sm, s->stream.get()));
+            CU(launch_sketch_reduce(db->d_offsets.get() + b, n, db->d_canon.get(), s->d_counts.get(), winner, s->d_shared + b,
+                                    s->d_median + b, db->sm, s->stream.get()));
             s->st.n_launches += 5;   // k_winner x4 (clear, score, length, index) + the reduction
         }
     }
@@ -1972,15 +1922,15 @@ int enqueue_stats_and_copy(hs_screen *s)
         const uint64_t b = db->seg_begin[j], n = db->seg_begin[j + 1] - b;
         if (!n) continue;
         CU(launch_stats(db->k, set_size_of(s->mixture, db->use64, db->seg_s[j]),
-                        s->mixture_on_device ? &s->d_sparse->set_size[j] : nullptr, n, s->d_shared + b, nullptr,
-                        db->d_offsets + b, nullptr, s->d_identity + b, s->d_pvalue + b, s->stream));
+                        s->mixture_on_device ? &s->d_sparse.get()->set_size[j] : nullptr, n, s->d_shared + b, nullptr,
+                        db->d_offsets.get() + b, nullptr, s->d_identity + b, s->d_pvalue + b, s->stream.get()));
         s->st.n_launches++;
     }
     const uint64_t NA = std::max<uint64_t>(N, 1);   // layout of the allocation (hs_screen_new)
-    if (N) CU(cudaMemcpyAsync(s->h_result, s->d_identity, NA * 24, cudaMemcpyDeviceToHost, s->stream));
-    CU(cudaMemcpyAsync(s->h_sparse, s->d_sparse, sizeof(SparseState), cudaMemcpyDeviceToHost, s->stream));
+    if (N) CU(cudaMemcpyAsync(s->h_result.get(), s->d_identity, NA * 24, cudaMemcpyDeviceToHost, s->stream.get()));
+    CU(cudaMemcpyAsync(s->h_sparse.get(), s->d_sparse.get(), sizeof(SparseState), cudaMemcpyDeviceToHost, s->stream.get()));
     if (s->mixture_on_device && db->s)
-        CU(cudaMemcpyAsync(s->h_mixture, s->d_mixture, (size_t)db->s * 8, cudaMemcpyDeviceToHost, s->stream));
+        CU(cudaMemcpyAsync(s->h_mixture.get(), s->d_mixture.get(), (size_t)db->s * 8, cudaMemcpyDeviceToHost, s->stream.get()));
     return HS_OK;
 }
 
@@ -1993,11 +1943,11 @@ int enqueue_hits(hs_screen *s, bool dense)
 {
     hs_db *db = s->db;
     const uint64_t N = db->n_refs;
-    if (N && !s->h_rows) {
+    if (N && !s->rows_host.ref) {   // (laid out once the pinned rows and their device address both exist)
         const size_t n3 = (N * 12 + 7) & ~(size_t)7;
-        CU(cudaHostAlloc((void **)&s->h_rows, n3 + N * 16, cudaHostAllocMapped));
+        CU(s->h_rows.grow(n3 + N * 16, cudaHostAllocMapped));
         char *d = nullptr;
-        CU(cudaHostGetDevicePointer((void **)&d, s->h_rows, 0));
+        CU(cudaHostGetDevicePointer((void **)&d, s->h_rows.get(), 0));
         auto lay = [&](char *base) {
             HitRows r;
             r.ref = reinterpret_cast<uint32_t *>(base); r.shared = r.ref + N; r.median = r.shared + N;
@@ -2005,7 +1955,7 @@ int enqueue_hits(hs_screen *s, bool dense)
             r.cap = (uint32_t)N;
             return r;
         };
-        s->rows_host = lay(s->h_rows);
+        s->rows_host = lay(s->h_rows.get());
         s->rows_dev = lay(d);
     }
     if (N) {
@@ -2013,15 +1963,15 @@ int enqueue_hits(hs_screen *s, bool dense)
         memset(&a, 0, sizeof a);
         a.k = db->k; a.n_seg = (uint32_t)db->seg_s.size();
         for (size_t j = 0; j < db->seg_s.size(); j++) a.set_size[j] = set_size_of(s->mixture, db->use64, db->seg_s[j]);
-        a.set_size_dev = s->mixture_on_device ? s->d_sparse->set_size : nullptr;
-        a.seg_begin = db->d_seg_begin; a.hit = s->d_hit; a.n_hit = &s->d_sparse->n_hit;
-        a.shared = s->d_shared; a.median = s->d_median; a.offsets = db->d_offsets; a.rows = s->rows_dev;
-        CU(launch_stats_hits(a, dense, (uint32_t)N, s->d_hit, &s->d_sparse->n_hit, db->sm, s->stream));
+        a.set_size_dev = s->mixture_on_device ? s->d_sparse.get()->set_size : nullptr;
+        a.seg_begin = db->d_seg_begin.get(); a.hit = s->d_hit; a.n_hit = &s->d_sparse.get()->n_hit;
+        a.shared = s->d_shared; a.median = s->d_median; a.offsets = db->d_offsets.get(); a.rows = s->rows_dev;
+        CU(launch_stats_hits(a, dense, (uint32_t)N, s->d_hit, &s->d_sparse.get()->n_hit, db->sm, s->stream.get()));
         s->st.n_launches += dense ? 2 : 1;
     }
-    CU(cudaMemcpyAsync(s->h_sparse, s->d_sparse, sizeof(SparseState), cudaMemcpyDeviceToHost, s->stream));
+    CU(cudaMemcpyAsync(s->h_sparse.get(), s->d_sparse.get(), sizeof(SparseState), cudaMemcpyDeviceToHost, s->stream.get()));
     if (s->mixture_on_device && db->s)
-        CU(cudaMemcpyAsync(s->h_mixture, s->d_mixture, (size_t)db->s * 8, cudaMemcpyDeviceToHost, s->stream));
+        CU(cudaMemcpyAsync(s->h_mixture.get(), s->d_mixture.get(), (size_t)db->s * 8, cudaMemcpyDeviceToHost, s->stream.get()));
     return HS_OK;
 }
 
@@ -2037,49 +1987,49 @@ int finish_core(hs_screen *s, bool wta, bool hits)
     bool dense = !(s->sparse_enabled && s->touched_valid);
     int rc;
     if (early) {
-        CU(cudaEventRecord(s->red2, s->stream));
+        CU(cudaEventRecord(s->red2.get(), s->stream.get()));
         if ((rc = enqueue_reduce(s, wta, dense)) != HS_OK) return rc;
-        CU(cudaEventRecord(s->red3, s->stream));
+        CU(cudaEventRecord(s->red3.get(), s->stream.get()));
     }
     if (!pending) {
         rc = hs_screen_flush(s);
         if (rc) return rc;
-        CU(cudaEventRecord(s->red0, s->stream));
+        CU(cudaEventRecord(s->red0.get(), s->stream.get()));
     }   // (pending: red0 was recorded by hs_screen_flush_async -- the exchange in between is part of the figure)
     if (early) {
         float ems = 0;
-        CU(cudaEventElapsedTime(&ems, s->red2, s->red3));   // flush synchronised the stream
+        CU(cudaEventElapsedTime(&ems, s->red2.get(), s->red3.get()));   // flush synchronised the stream
         s->st.ms_reduce += ems;
     }
     if (!early && (rc = enqueue_reduce(s, wta, dense)) != HS_OK) return rc;
     if ((rc = hits ? enqueue_hits(s, dense) : enqueue_stats_and_copy(s)) != HS_OK) return rc;
-    CU(cudaEventRecord(s->red1, s->stream));
-    CU(cudaStreamSynchronize(s->stream));
+    CU(cudaEventRecord(s->red1.get(), s->stream.get()));
+    CU(cudaStreamSynchronize(s->stream.get()));
     float ms = 0;
-    CU(cudaEventElapsedTime(&ms, s->red0, s->red1));
+    CU(cudaEventElapsedTime(&ms, s->red0.get(), s->red1.get()));
     s->st.ms_reduce = pending ? ms : s->st.ms_reduce + ms;
     s->st.mix_unsettled = 0;
     if (pending) {
         // the one synchronisation of this screen has happened: complete the flush from what came back with it
-        const MixState &hs_ = *s->mix.h_state;
+        const MixState &hs_ = *s->mix.h_state.get();
         const bool held = !s->force_unsettled && !hs_.overflow && !hs_.sel_too_many && hs_.n_out <= s->mix.sel_pad &&
                           (hs_.n_unique >= s->mix.s || hs_.tau == ~0ull);
         s->force_unsettled = 0;   // (tests; the multi-GPU path has already spent it in its mixture record)
-        const bool all_held = s->mixture_on_device ? !s->h_sparse->mix_unsettled : held;
+        const bool all_held = s->mixture_on_device ? !s->h_sparse.get()->mix_unsettled : held;
         if (!all_held) {
             if (s->mixture_on_device) {
                 // some rank's selection fell through: every rank knows (the gathered records say so) and the
                 // CALLER redoes flush + mixture exchange synchronously; the counts were absorbed and stay
                 s->st.mix_unsettled = 1;
-                s->st.exchange_overflow = s->h_sparse->xchg_overflow;
-                s->st.exchange_max_pairs = s->h_sparse->xchg_max;
+                s->st.exchange_overflow = s->h_sparse.get()->xchg_overflow;
+                s->st.exchange_max_pairs = s->h_sparse.get()->xchg_max;
                 return HS_OK;
             }
             rc = hs_screen_flush(s);              // single process: the iterative finaliser, then everything again
             if (rc) return rc;
             return finish_core(s, wta, hits);
         }
-        s->mixture.assign(s->mix.h_cand, s->mix.h_cand + std::min(hs_.n_unique, s->mix.s));
+        s->mixture.assign(s->mix.h_cand.get(), s->mix.h_cand.get() + std::min(hs_.n_unique, s->mix.s));
         if (hs_.has_max && s->mixture.size() < s->mix.s) s->mixture.push_back(~0ull);
         s->flush_pending = false;
         rc = flush_epilogue(s, s->flush_parsed);
@@ -2087,26 +2037,26 @@ int finish_core(hs_screen *s, bool wta, bool hits)
         s->flushed = true;
     }
     if (s->mixture_on_device) adopt_merged_mixture(s);   // the merged mixture and its set size arrive with the results
-    s->st.exchange_overflow = s->h_sparse->xchg_overflow;
-    s->st.exchange_max_pairs = s->h_sparse->xchg_max;
-    if (!dense && (s->h_sparse->n_touched > s->touched_cap || s->h_sparse->wrapped || s->h_sparse->overflow)) {
+    s->st.exchange_overflow = s->h_sparse.get()->xchg_overflow;
+    s->st.exchange_max_pairs = s->h_sparse.get()->xchg_max;
+    if (!dense && (s->h_sparse.get()->n_touched > s->touched_cap || s->h_sparse.get()->wrapped || s->h_sparse.get()->overflow)) {
         // the O(present) bookkeeping did not hold this query (more present hashes than its buffers, or a
         // count that wrapped): the dense kernels give the answer, and the next reset clears every count
         dense = true;
-        const uint32_t n_touched = s->h_sparse->n_touched;
-        CU(cudaEventRecord(s->red0, s->stream));
+        const uint32_t n_touched = s->h_sparse.get()->n_touched;
+        CU(cudaEventRecord(s->red0.get(), s->stream.get()));
         if ((rc = enqueue_reduce(s, wta, true)) != HS_OK) return rc;
         if ((rc = hits ? enqueue_hits(s, true) : enqueue_stats_and_copy(s)) != HS_OK) return rc;
-        CU(cudaEventRecord(s->red1, s->stream));
-        CU(cudaStreamSynchronize(s->stream));
-        CU(cudaEventElapsedTime(&ms, s->red0, s->red1));
+        CU(cudaEventRecord(s->red1.get(), s->stream.get()));
+        CU(cudaStreamSynchronize(s->stream.get()));
+        CU(cudaEventElapsedTime(&ms, s->red0.get(), s->red1.get()));
         s->st.ms_reduce += ms;
-        s->h_sparse->n_touched = n_touched;
+        s->h_sparse.get()->n_touched = n_touched;
     }
     s->st.reduce_path = dense ? 1u : 0u;
-    s->st.n_touched = s->h_sparse->n_touched;
-    s->st.n_hit_refs = (dense && !hits) ? 0u : s->h_sparse->n_hit;
-    s->st.n_pairs = dense ? 0u : s->h_sparse->n_pairs;
+    s->st.n_touched = s->h_sparse.get()->n_touched;
+    s->st.n_hit_refs = (dense && !hits) ? 0u : s->h_sparse.get()->n_hit;
+    s->st.n_pairs = dense ? 0u : s->h_sparse.get()->n_pairs;
     return HS_OK;
 }
 
@@ -2120,7 +2070,7 @@ HS_API int hs_screen_finish(hs_screen *s, int wta, uint64_t *shared, uint32_t *m
     int rc = finish_core(s, wta != 0, false);
     if (rc) return rc;
     const uint64_t N = s->db->n_refs, NA = std::max<uint64_t>(N, 1);   // layout of the allocation (hs_screen_new)
-    double *h_id = reinterpret_cast<double *>(s->h_result), *h_pv = h_id + NA;
+    double *h_id = reinterpret_cast<double *>(s->h_result.get()), *h_pv = h_id + NA;
     uint32_t *h_sh = reinterpret_cast<uint32_t *>(h_pv + NA), *h_md = h_sh + NA;
     if (shared) for (uint64_t i = 0; i < N; i++) shared[i] = h_sh[i];
     if (median && N) memcpy(median, h_md, N * 4);
@@ -2137,7 +2087,7 @@ HS_API int hs_screen_finish_hits(hs_screen *s, int wta, uint32_t *n_hits, hs_sta
     ON_DEVICE(s->db->device);
     int rc = finish_core(s, wta != 0, true);
     if (rc) return rc;
-    const uint32_t n = (uint32_t)std::min<uint64_t>(s->h_sparse->n_hit, s->db->n_refs);
+    const uint32_t n = (uint32_t)std::min<uint64_t>(s->h_sparse.get()->n_hit, s->db->n_refs);
     s->hit_order.clear();
     for (uint32_t q = 0; q < n; q++)
         if (s->rows_host.shared[q]) s->hit_order.push_back(q);   // -w leaves references that lost every hash: not reported
@@ -2169,7 +2119,7 @@ HS_API int hs_screen_reset(hs_screen *s)
 {
     if (!s) return fail(HS_EINVAL, "null handle");
     ON_DEVICE(s->db->device);
-    CU(cudaStreamSynchronize(s->stream));
+    CU(cudaStreamSynchronize(s->stream.get()));
     return screen_zero(s);
 }
 
@@ -2180,42 +2130,7 @@ HS_API int hs_screen_stats(hs_screen *s, hs_stats_t *stats)
     return HS_OK;
 }
 
-HS_API void hs_screen_free(hs_screen *s)
-{
-    if (!s) return;
-    if (s->db) cudaSetDevice(s->db->device);
-    if (s->stream) cudaStreamSynchronize(s->stream);
-    cudaFree(s->d_counts); cudaFree(s->d_stats);
-    cudaFree(s->d_sparse); cudaFree(s->d_touched); cudaFree(s->d_depths); cudaFree(s->d_hit);
-    cudaFree(s->d_mixture); cudaFree(s->d_merge_work); cudaFree(s->d_merge_scratch);
-    if (s->h_sparse) cudaFreeHost(s->h_sparse);
-    if (s->h_mixture) cudaFreeHost(s->h_mixture);
-    if (s->h_rows) cudaFreeHost(s->h_rows);
-    if (s->rst0) cudaEventDestroy(s->rst0);
-    if (s->rst1) cudaEventDestroy(s->rst1);
-    cudaFree(s->d_identity);   // one block: identity | p-value | shared | median
-    cudaFree(s->d_best_score); cudaFree(s->d_best_len); cudaFree(s->d_winner);
-    s->mix.destroy();
-    s->arena.release();
-    s->ingest.release();
-    s->ring.release();
-    for (auto &g : s->staging) {
-        if (g.seq) cudaFreeHost(g.seq);
-        if (g.inv) cudaFreeHost(g.inv);
-        if (g.free_ev) cudaEventDestroy(g.free_ev);
-    }
-    for (auto &e : s->ev_pool) { cudaEventDestroy(e.first); cudaEventDestroy(e.second); }
-    if (s->red0) cudaEventDestroy(s->red0);
-    if (s->red1) cudaEventDestroy(s->red1);
-    if (s->red2) cudaEventDestroy(s->red2);
-    if (s->red3) cudaEventDestroy(s->red3);
-    if (s->h_result) cudaFreeHost(s->h_result);
-    if (s->h_stats) cudaFreeHost(s->h_stats);
-    if (s->own_stream && s->stream) cudaStreamDestroy(s->stream);
-    if (s->copy_stream) { cudaStreamSynchronize(s->copy_stream); cudaStreamDestroy(s->copy_stream); }
-    for (auto &e : s->copy_evs) cudaEventDestroy(e);
-    delete s;
-}
+HS_API void hs_screen_free(hs_screen *s) { if (s) delete s; }
 
 // =============================================================================
 // single stages
@@ -2228,29 +2143,28 @@ HS_API int hs_hash_packed(uint32_t k, uint32_t seed, const uint64_t *seq2, const
     NEED_DEVICE();
     if (!n_bases) return HS_OK;
     const uint64_t words = (n_bases + 31) / 32, alloc = hs_packed_words(n_bases);
-    uint64_t *dseq = nullptr, *dh = nullptr;
-    uint32_t *dinv = nullptr;
-    uint8_t *dv = nullptr;
-    unsigned long long *dst = nullptr;
-    CU(cudaMalloc((void **)&dseq, alloc * 8));
-    CU(cudaMalloc((void **)&dinv, alloc * 4));
-    CU(cudaMalloc((void **)&dh, n_bases * 8));
-    CU(cudaMalloc((void **)&dv, n_bases));
-    CU(cudaMalloc((void **)&dst, ST_COUNT * sizeof(unsigned long long)));
-    CU(cudaMemset(dseq, 0, alloc * 8));
-    CU(cudaMemset(dinv, 0xFF, alloc * 4));
-    CU(cudaMemset(dh, 0, n_bases * 8));
-    CU(cudaMemset(dv, 0, n_bases));
-    CU(cudaMemset(dst, 0, ST_COUNT * sizeof(unsigned long long)));
-    CU(cudaMemcpy(dseq, seq2, words * 8, cudaMemcpyHostToDevice));
-    CU(cudaMemcpy(dinv, inv, words * 4, cudaMemcpyHostToDevice));
-    Chunk c{dseq, dinv, n_bases};
+    DevBuf<uint64_t> dseq, dh;
+    DevBuf<uint32_t> dinv;
+    DevBuf<uint8_t> dv;
+    DevBuf<unsigned long long> dst;
+    CU(dseq.grow(alloc));
+    CU(dinv.grow(alloc));
+    CU(dh.grow(n_bases));
+    CU(dv.grow(n_bases));
+    CU(dst.grow(ST_COUNT));
+    CU(cudaMemset(dseq.get(), 0, alloc * 8));
+    CU(cudaMemset(dinv.get(), 0xFF, alloc * 4));
+    CU(cudaMemset(dh.get(), 0, n_bases * 8));
+    CU(cudaMemset(dv.get(), 0, n_bases));
+    CU(cudaMemset(dst.get(), 0, ST_COUNT * sizeof(unsigned long long)));
+    CU(cudaMemcpy(dseq.get(), seq2, words * 8, cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(dinv.get(), inv, words * 4, cudaMemcpyHostToDevice));
+    Chunk c{dseq.get(), dinv.get(), n_bases};
     StreamArgs a = base_args(c, k, seed, pow(4.0, (double)k) > pow(2.0, 32.0));
-    a.emit_hash = dh; a.emit_valid = dv; a.stats = dst;
+    a.emit_hash = dh.get(); a.emit_valid = dv.get(); a.stats = dst.get();
     CU(launch_stream(a, g_sm, 0));
-    CU(cudaMemcpy(out_hash, dh, n_bases * 8, cudaMemcpyDeviceToHost));
-    CU(cudaMemcpy(out_valid, dv, n_bases, cudaMemcpyDeviceToHost));
-    cudaFree(dseq); cudaFree(dinv); cudaFree(dh); cudaFree(dv); cudaFree(dst);
+    CU(cudaMemcpy(out_hash, dh.get(), n_bases * 8, cudaMemcpyDeviceToHost));
+    CU(cudaMemcpy(out_valid, dv.get(), n_bases, cudaMemcpyDeviceToHost));
     return HS_OK;
 }
 
@@ -2267,29 +2181,28 @@ HS_API int hs_pack_text_device(const char *text, size_t n, uint64_t *seq2, uint3
     Ingest in;
     int rc = in.ensure(n, 0);
     if (rc) return rc;
-    uint8_t *raw = nullptr, *codes = nullptr;
-    uint64_t *dseq = nullptr;
-    uint32_t *dinv = nullptr;
-    unsigned long long *d_npos = nullptr, tot[4] = {0, 0, 0, 0};
-    CU(cudaMalloc((void **)&raw, n + 64)); CU(cudaMalloc((void **)&codes, n + 64));
-    CU(cudaMalloc((void **)&dseq, alloc * 8)); CU(cudaMalloc((void **)&dinv, alloc * 4));
-    CU(cudaMalloc((void **)&d_npos, sizeof(unsigned long long)));
-    CU(cudaMemcpy(raw, text, n, cudaMemcpyHostToDevice));
+    DevBuf<uint8_t> raw, codes;
+    DevBuf<uint64_t> dseq;
+    DevBuf<uint32_t> dinv;
+    DevBuf<unsigned long long> d_npos;
+    unsigned long long tot[4] = {0, 0, 0, 0};
+    CU(raw.grow(n + 64)); CU(codes.grow(n + 64));
+    CU(dseq.grow(alloc)); CU(dinv.grow(alloc));
+    CU(d_npos.grow(1));
+    CU(cudaMemcpy(raw.get(), text, n, cudaMemcpyHostToDevice));
     FaScratch sc = in.sc;
-    sc.chunk_positions = d_npos;
-    CU(launch_fasta_to_codes(raw, (uint32_t)n, codes, sc, 0));
-    CU(launch_pack_codes_dyn(codes, d_npos, dseq, dinv, alloc, 0));
-    CU(cudaMemcpy(tot, in.d_totals, sizeof tot, cudaMemcpyDeviceToHost));
+    sc.chunk_positions = d_npos.get();
+    CU(launch_fasta_to_codes(raw.get(), (uint32_t)n, codes.get(), sc, 0));
+    CU(launch_pack_codes_dyn(codes.get(), d_npos.get(), dseq.get(), dinv.get(), alloc, 0));
+    CU(cudaMemcpy(tot, in.d_totals.get(), sizeof tot, cudaMemcpyDeviceToHost));
     const uint64_t words = (tot[0] + 31) / 32;
     if (words > cap_words) rc = fail(HS_EINVAL, "output capacity too small");
     if (rc == HS_OK && words) {
-        CU(cudaMemcpy(seq2, dseq, words * 8, cudaMemcpyDeviceToHost));
-        CU(cudaMemcpy(inv, dinv, words * 4, cudaMemcpyDeviceToHost));
+        CU(cudaMemcpy(seq2, dseq.get(), words * 8, cudaMemcpyDeviceToHost));
+        CU(cudaMemcpy(inv, dinv.get(), words * 4, cudaMemcpyDeviceToHost));
     }
     *n_bases = tot[0];
     if (stats) { stats->n_positions = tot[0]; stats->n_bases = tot[1]; stats->n_records = tot[2]; }
-    cudaFree(raw); cudaFree(codes); cudaFree(dseq); cudaFree(dinv); cudaFree(d_npos);
-    in.release();
     return rc;
 }
 
@@ -2298,17 +2211,16 @@ HS_API int hs_db_probe(hs_db *db, const uint64_t *hashes, uint64_t n, uint32_t *
     if (!db || (!hashes && n) || (!out_entry && n)) return fail(HS_EINVAL, "null argument");
     ON_DEVICE(db->device);
     if (!n) return HS_OK;
-    uint64_t *dh = nullptr;
-    uint32_t *de = nullptr;
-    unsigned long long *dst = nullptr;
-    CU(cudaMalloc((void **)&dh, n * 8));
-    CU(cudaMalloc((void **)&de, n * 4));
-    CU(cudaMalloc((void **)&dst, 2 * sizeof(unsigned long long)));
-    CU(cudaMemset(dst, 0, 2 * sizeof(unsigned long long)));
-    CU(cudaMemcpy(dh, hashes, n * 8, cudaMemcpyHostToDevice));
-    CU(launch_probe(db->view(), dh, n, de, dst, db->sm, 0));
-    CU(cudaMemcpy(out_entry, de, n * 4, cudaMemcpyDeviceToHost));
-    cudaFree(dh); cudaFree(de); cudaFree(dst);
+    DevBuf<uint64_t> dh;
+    DevBuf<uint32_t> de;
+    DevBuf<unsigned long long> dst;
+    CU(dh.grow(n));
+    CU(de.grow(n));
+    CU(dst.grow(2));
+    CU(cudaMemset(dst.get(), 0, 2 * sizeof(unsigned long long)));
+    CU(cudaMemcpy(dh.get(), hashes, n * 8, cudaMemcpyHostToDevice));
+    CU(launch_probe(db->view(), dh.get(), n, de.get(), dst.get(), db->sm, 0));
+    CU(cudaMemcpy(out_entry, de.get(), n * 4, cudaMemcpyDeviceToHost));
     return HS_OK;
 }
 
@@ -2317,22 +2229,22 @@ HS_API int hs_db_probe_device(hs_db *db, const void *d_hashes, uint64_t n, uint6
 {
     if (!db || (!d_hashes && n)) return fail(HS_EINVAL, "null argument");
     ON_DEVICE(db->device);
-    unsigned long long *dst = nullptr, h[2] = {0, 0};
-    cudaEvent_t e0, e1;
-    CU(cudaMalloc((void **)&dst, 2 * sizeof(unsigned long long)));
-    CU(cudaMemset(dst, 0, 2 * sizeof(unsigned long long)));
-    CU(cudaEventCreate(&e0)); CU(cudaEventCreate(&e1));
-    CU(cudaEventRecord(e0, 0));
-    CU(launch_probe(db->view(), (const uint64_t *)d_hashes, n, nullptr, dst, db->sm, 0));
-    CU(cudaEventRecord(e1, 0));
-    CU(cudaEventSynchronize(e1));
+    unsigned long long h[2] = {0, 0};
+    DevBuf<unsigned long long> dst;
+    Event e0, e1;
+    CU(dst.grow(2));
+    CU(cudaMemset(dst.get(), 0, 2 * sizeof(unsigned long long)));
+    CU(e0.create()); CU(e1.create());
+    CU(cudaEventRecord(e0.get(), 0));
+    CU(launch_probe(db->view(), (const uint64_t *)d_hashes, n, nullptr, dst.get(), db->sm, 0));
+    CU(cudaEventRecord(e1.get(), 0));
+    CU(cudaEventSynchronize(e1.get()));
     float t = 0;
-    CU(cudaEventElapsedTime(&t, e0, e1));
-    CU(cudaMemcpy(h, dst, sizeof h, cudaMemcpyDeviceToHost));
+    CU(cudaEventElapsedTime(&t, e0.get(), e1.get()));
+    CU(cudaMemcpy(h, dst.get(), sizeof h, cudaMemcpyDeviceToHost));
     if (n_hits) *n_hits = h[0];
     if (n_bucket_reads) *n_bucket_reads = h[1];
     if (ms) *ms = t;
-    cudaFree(dst); cudaEventDestroy(e0); cudaEventDestroy(e1);
     return HS_OK;
 }
 
@@ -2340,15 +2252,14 @@ HS_API int hs_gather_bench(const void *d_buf, uint64_t bytes, uint64_t n_reads, 
 {
     if (!d_buf || bytes < 64 || !ms) return fail(HS_EINVAL, "bad argument");
     NEED_DEVICE();
-    cudaEvent_t e0, e1;
-    CU(cudaEventCreate(&e0)); CU(cudaEventCreate(&e1));
+    Event e0, e1;
+    CU(e0.create()); CU(e1.create());
     CU(launch_gather_bench(d_buf, bytes, n_reads, g_sm, 0));  // warm-up
-    CU(cudaEventRecord(e0, 0));
+    CU(cudaEventRecord(e0.get(), 0));
     CU(launch_gather_bench(d_buf, bytes, n_reads, g_sm, 0));
-    CU(cudaEventRecord(e1, 0));
-    CU(cudaEventSynchronize(e1));
-    CU(cudaEventElapsedTime(ms, e0, e1));
-    cudaEventDestroy(e0); cudaEventDestroy(e1);
+    CU(cudaEventRecord(e1.get(), 0));
+    CU(cudaEventSynchronize(e1.get()));
+    CU(cudaEventElapsedTime(ms, e0.get(), e1.get()));
     return HS_OK;
 }
 
@@ -2356,7 +2267,7 @@ HS_API int hs_db_entry_ids(hs_db *db, uint32_t *out)
 {
     if (!db || !out) return fail(HS_EINVAL, "null argument");
     ON_DEVICE(db->device);
-    if (db->n_entries) CU(cudaMemcpy(out, db->d_canon, db->n_entries * 4, cudaMemcpyDeviceToHost));
+    if (db->n_entries) CU(cudaMemcpy(out, db->d_canon.get(), db->n_entries * 4, cudaMemcpyDeviceToHost));
     return HS_OK;
 }
 
@@ -2366,16 +2277,15 @@ HS_API int hs_stat_batch(uint32_t k, uint64_t set_size, uint64_t n, const uint64
     if ((!shared || !size || !identity || !pvalue) && n) return fail(HS_EINVAL, "null argument");
     NEED_DEVICE();
     if (!n) return HS_OK;
-    uint64_t *dx = nullptr, *dn = nullptr;
-    double *di = nullptr, *dp = nullptr;
-    CU(cudaMalloc((void **)&dx, n * 8)); CU(cudaMalloc((void **)&dn, n * 8));
-    CU(cudaMalloc((void **)&di, n * 8)); CU(cudaMalloc((void **)&dp, n * 8));
-    CU(cudaMemcpy(dx, shared, n * 8, cudaMemcpyHostToDevice));
-    CU(cudaMemcpy(dn, size, n * 8, cudaMemcpyHostToDevice));
-    CU(launch_stats(k, set_size, nullptr, n, nullptr, dx, nullptr, dn, di, dp, 0));
-    CU(cudaMemcpy(identity, di, n * 8, cudaMemcpyDeviceToHost));
-    CU(cudaMemcpy(pvalue, dp, n * 8, cudaMemcpyDeviceToHost));
-    cudaFree(dx); cudaFree(dn); cudaFree(di); cudaFree(dp);
+    DevBuf<uint64_t> dx, dn;
+    DevBuf<double> di, dp;
+    CU(dx.grow(n)); CU(dn.grow(n));
+    CU(di.grow(n)); CU(dp.grow(n));
+    CU(cudaMemcpy(dx.get(), shared, n * 8, cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(dn.get(), size, n * 8, cudaMemcpyHostToDevice));
+    CU(launch_stats(k, set_size, nullptr, n, nullptr, dx.get(), nullptr, dn.get(), di.get(), dp.get(), 0));
+    CU(cudaMemcpy(identity, di.get(), n * 8, cudaMemcpyDeviceToHost));
+    CU(cudaMemcpy(pvalue, dp.get(), n * 8, cudaMemcpyDeviceToHost));
     return HS_OK;
 }
 
@@ -2407,61 +2317,35 @@ constexpr uint64_t kSketchSetWords = (uint64_t)8 << 20;   // 64 MB of sets per b
 constexpr uint32_t kSketchMaxCap = 1u << 24;              // mixset_slot spreads a set over at most 2^24 slots
 constexpr uint64_t kTilePositions = (uint64_t)kTileWords * kBasesPerWord;
 
-// a buffer with a single owner that grows on demand (device memory, or pinned host memory)
-template <class T, bool HOST>
-struct Grow {
-    T *p = nullptr;
-    size_t cap = 0;
-    cudaError_t need(size_t n)
-    {
-        if (n <= cap) return cudaSuccess;
-        release();
-        n = std::max<size_t>(n + n / 2, 64);
-        const cudaError_t e = HOST ? cudaHostAlloc((void **)&p, n * sizeof(T), cudaHostAllocDefault)
-                                   : cudaMalloc((void **)&p, n * sizeof(T));
-        if (e == cudaSuccess) cap = n; else p = nullptr;
-        return e;
-    }
-    void release()
-    {
-        if (p) { if (HOST) cudaFreeHost(p); else cudaFree(p); }
-        p = nullptr; cap = 0;
-    }
-};
+// room for n elements in a buffer that grows on demand: half as much again when it has to (at least 64)
+template <class B>
+cudaError_t need(B &b, size_t n)
+{
+    return n <= b.cap() ? cudaSuccess : b.grow(std::max<size_t>(n + n / 2, 64));
+}
 
-// every CUDA resource of a sketcher, released in one place
+// every CUDA resource of a sketcher; the stream (declared first) is released last
 struct SketchDev {
-    bool ready = false;
-    cudaStream_t stream = nullptr;
-    cudaEvent_t ev[4] = {};
-    unsigned long long *stats = nullptr;
-    Grow<uint64_t, false> seq, sets, out, out_off;
-    Grow<uint32_t, false> inv, tile_genome, n_out;
-    Grow<SketchSlot, false> slots;
-    Grow<uint64_t, true> h_seq, h_out, h_out_off;
-    Grow<uint32_t, true> h_inv, h_tile_genome, h_n_out;
-    Grow<SketchSlot, true> h_slots;
+    Stream stream;
+    Event ev[4];
+    DevBuf<unsigned long long> stats;
+    DevBuf<uint64_t> seq, sets, out, out_off;
+    DevBuf<uint32_t> inv, tile_genome, n_out;
+    DevBuf<SketchSlot> slots;
+    PinnedBuf<uint64_t> h_seq, h_out, h_out_off;
+    PinnedBuf<uint32_t> h_inv, h_tile_genome, h_n_out;
+    PinnedBuf<SketchSlot> h_slots;
     int init()
     {
-        if (ready) return HS_OK;
-        ready = true;   // from here on release() owns whatever was created
-        CU(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
-        for (auto &e : ev) CU(cudaEventCreate(&e));
-        CU(cudaMalloc((void **)&stats, ST_COUNT * sizeof(unsigned long long)));
-        CU(cudaMemsetAsync(stats, 0, ST_COUNT * sizeof(unsigned long long), stream));
+        CU(stream.create());
+        for (auto &e : ev) CU(e.create());
+        CU(stats.grow(ST_COUNT));
+        CU(cudaMemsetAsync(stats.get(), 0, ST_COUNT * sizeof(unsigned long long), stream.get()));
         return HS_OK;
     }
-    void release()
-    {
-        if (stream) cudaStreamSynchronize(stream);
-        seq.release(); sets.release(); out.release(); out_off.release(); inv.release(); tile_genome.release();
-        n_out.release(); slots.release(); h_seq.release(); h_out.release(); h_out_off.release(); h_inv.release();
-        h_tile_genome.release(); h_n_out.release(); h_slots.release();
-        cudaFree(stats); stats = nullptr;
-        for (auto &e : ev) { if (e) cudaEventDestroy(e); e = nullptr; }
-        if (stream) cudaStreamDestroy(stream);
-        stream = nullptr;
-        ready = false;
+    ~SketchDev()
+    {   // nothing is released while the stream may still use it
+        if (stream.get()) cudaStreamSynchronize(stream.get());
     }
 };
 
@@ -2563,14 +2447,14 @@ int sketch_plan(hs_sketcher *sk, SkGenome &g)
 // the genome's words [w0, w1) into the staging at tile t0, padded with invalid positions to `tiles` tiles
 uint32_t sketch_stage(SketchDev &d, const SkGenome &g, uint64_t w0, uint64_t w1, uint32_t tiles, uint32_t t0, uint32_t slot)
 {
-    uint64_t *sq = d.h_seq.p + (size_t)t0 * kTileWords;
-    uint32_t *iv = d.h_inv.p + (size_t)t0 * kTileWords;
+    uint64_t *sq = d.h_seq.get() + (size_t)t0 * kTileWords;
+    uint32_t *iv = d.h_inv.get() + (size_t)t0 * kTileWords;
     memcpy(sq, g.seq.data() + w0, (w1 - w0) * 8);
     memcpy(iv, g.inv.data() + w0, (w1 - w0) * 4);
     const size_t pad = (size_t)tiles * kTileWords - (w1 - w0);
     memset(sq + (w1 - w0), 0, pad * 8);
     memset(iv + (w1 - w0), 0xFF, pad * 4);
-    for (uint32_t t = 0; t < tiles; t++) d.h_tile_genome.p[t0 + t] = slot;
+    for (uint32_t t = 0; t < tiles; t++) d.h_tile_genome.get()[t0 + t] = slot;
     return tiles;
 }
 
@@ -2579,22 +2463,22 @@ int sketch_launch(hs_sketcher *sk, uint32_t tiles)
 {
     SketchDev &d = sk->dev;
     const size_t words = (size_t)tiles * kTileWords;
-    CU(d.seq.need(words)); CU(d.inv.need(words)); CU(d.tile_genome.need(tiles));
-    CU(cudaMemcpyAsync(d.seq.p, d.h_seq.p, words * 8, cudaMemcpyHostToDevice, d.stream));
-    CU(cudaMemcpyAsync(d.inv.p, d.h_inv.p, words * 4, cudaMemcpyHostToDevice, d.stream));
-    CU(cudaMemcpyAsync(d.tile_genome.p, d.h_tile_genome.p, (size_t)tiles * 4, cudaMemcpyHostToDevice, d.stream));
+    CU(need(d.seq, words)); CU(need(d.inv, words)); CU(need(d.tile_genome, tiles));
+    CU(cudaMemcpyAsync(d.seq.get(), d.h_seq.get(), words * 8, cudaMemcpyHostToDevice, d.stream.get()));
+    CU(cudaMemcpyAsync(d.inv.get(), d.h_inv.get(), words * 4, cudaMemcpyHostToDevice, d.stream.get()));
+    CU(cudaMemcpyAsync(d.tile_genome.get(), d.h_tile_genome.get(), (size_t)tiles * 4, cudaMemcpyHostToDevice, d.stream.get()));
     StreamArgs a;
     memset(&a, 0, sizeof a);
-    a.seq = d.seq.p; a.inv = d.inv.p; a.n_bases = tiles * kTilePositions; a.n_tiles = tiles;
-    a.k = (int)sk->k; a.seed = sk->seed; a.use64 = sk->use64; a.stats = d.stats;
-    a.sk = SketchView{d.tile_genome.p, d.slots.p, d.sets.p};
-    CU(cudaEventRecord(d.ev[0], d.stream));
-    CU(launch_stream(a, g_sm, d.stream));
-    CU(cudaEventRecord(d.ev[1], d.stream));
+    a.seq = d.seq.get(); a.inv = d.inv.get(); a.n_bases = tiles * kTilePositions; a.n_tiles = tiles;
+    a.k = (int)sk->k; a.seed = sk->seed; a.use64 = sk->use64; a.stats = d.stats.get();
+    a.sk = SketchView{d.tile_genome.get(), d.slots.get(), d.sets.get()};
+    CU(cudaEventRecord(d.ev[0].get(), d.stream.get()));
+    CU(launch_stream(a, g_sm, d.stream.get()));
+    CU(cudaEventRecord(d.ev[1].get(), d.stream.get()));
     // the staging is refilled next: wait for the copies (and take the kernel time with them)
-    CU(cudaEventSynchronize(d.ev[1]));
+    CU(cudaEventSynchronize(d.ev[1].get()));
     float ms = 0;
-    CU(cudaEventElapsedTime(&ms, d.ev[0], d.ev[1]));
+    CU(cudaEventElapsedTime(&ms, d.ev[0].get(), d.ev[1].get()));
     sk->st.ms_stream += ms;
     sk->st.n_launches++;
     return HS_OK;
@@ -2605,29 +2489,29 @@ int sketch_batch(hs_sketcher *sk, const std::vector<uint32_t> &ids)
 {
     SketchDev &d = sk->dev;
     const uint32_t n = (uint32_t)ids.size();
-    CU(d.h_slots.need(n)); CU(d.slots.need(n)); CU(d.h_out_off.need(n)); CU(d.out_off.need(n));
-    CU(d.h_n_out.need(n)); CU(d.n_out.need(n));
+    CU(need(d.h_slots, n)); CU(need(d.slots, n)); CU(need(d.h_out_off, n)); CU(need(d.out_off, n));
+    CU(need(d.h_n_out, n)); CU(need(d.n_out, n));
     uint64_t set_words = 0, out_words = 0, tiles = 0;
     uint32_t max_cap = 0;
     for (uint32_t j = 0; j < n; j++) {
         const SkGenome &g = sk->gen[ids[j]];
-        SketchSlot &sl = d.h_slots.p[j];
+        SketchSlot &sl = d.h_slots.get()[j];
         memset(&sl, 0, sizeof sl);
         sl.st.tau = g.tau;
         sl.set_off = set_words;
         sl.mask = g.cap - 1; sl.limit = g.cap / 2;
-        d.h_out_off.p[j] = out_words;
+        d.h_out_off.get()[j] = out_words;
         set_words += g.cap;
         out_words += std::min<uint64_t>(sk->s, g.cap);
         max_cap = std::max(max_cap, g.cap);
         tiles += g.tiles();
     }
-    CU(d.sets.need(set_words)); CU(d.out.need(out_words)); CU(d.h_out.need(out_words));
+    CU(need(d.sets, set_words)); CU(need(d.out, out_words)); CU(need(d.h_out, out_words));
     const uint64_t stage_tiles = std::min<uint64_t>(tiles, kSketchBatchTiles);
-    CU(d.h_seq.need(stage_tiles * kTileWords)); CU(d.h_inv.need(stage_tiles * kTileWords)); CU(d.h_tile_genome.need(stage_tiles));
-    CU(cudaMemcpyAsync(d.slots.p, d.h_slots.p, n * sizeof(SketchSlot), cudaMemcpyHostToDevice, d.stream));
-    CU(cudaMemcpyAsync(d.out_off.p, d.h_out_off.p, n * 8, cudaMemcpyHostToDevice, d.stream));
-    CU(cudaMemsetAsync(d.sets.p, 0xFF, set_words * 8, d.stream));
+    CU(need(d.h_seq, stage_tiles * kTileWords)); CU(need(d.h_inv, stage_tiles * kTileWords)); CU(need(d.h_tile_genome, stage_tiles));
+    CU(cudaMemcpyAsync(d.slots.get(), d.h_slots.get(), n * sizeof(SketchSlot), cudaMemcpyHostToDevice, d.stream.get()));
+    CU(cudaMemcpyAsync(d.out_off.get(), d.h_out_off.get(), n * 8, cudaMemcpyHostToDevice, d.stream.get()));
+    CU(cudaMemsetAsync(d.sets.get(), 0xFF, set_words * 8, d.stream.get()));
     sk->st.n_batches++;
     if (tiles <= kSketchBatchTiles) {
         uint32_t t = 0;
@@ -2651,26 +2535,26 @@ int sketch_batch(hs_sketcher *sk, const std::vector<uint32_t> &ids)
             w0 = w1 - 1;
         }
     }
-    CU(cudaEventRecord(d.ev[2], d.stream));
-    CU(launch_sketch_select(d.slots.p, n, max_cap, d.sets.p, sk->s, d.out_off.p, d.out.p, d.n_out.p, d.stream));
-    CU(cudaEventRecord(d.ev[3], d.stream));
+    CU(cudaEventRecord(d.ev[2].get(), d.stream.get()));
+    CU(launch_sketch_select(d.slots.get(), n, max_cap, d.sets.get(), sk->s, d.out_off.get(), d.out.get(), d.n_out.get(), d.stream.get()));
+    CU(cudaEventRecord(d.ev[3].get(), d.stream.get()));
     sk->st.n_launches++;
-    CU(cudaMemcpyAsync(d.h_slots.p, d.slots.p, n * sizeof(SketchSlot), cudaMemcpyDeviceToHost, d.stream));
-    CU(cudaMemcpyAsync(d.h_n_out.p, d.n_out.p, n * 4, cudaMemcpyDeviceToHost, d.stream));
-    CU(cudaMemcpyAsync(d.h_out.p, d.out.p, out_words * 8, cudaMemcpyDeviceToHost, d.stream));
-    CU(cudaStreamSynchronize(d.stream));
+    CU(cudaMemcpyAsync(d.h_slots.get(), d.slots.get(), n * sizeof(SketchSlot), cudaMemcpyDeviceToHost, d.stream.get()));
+    CU(cudaMemcpyAsync(d.h_n_out.get(), d.n_out.get(), n * 4, cudaMemcpyDeviceToHost, d.stream.get()));
+    CU(cudaMemcpyAsync(d.h_out.get(), d.out.get(), out_words * 8, cudaMemcpyDeviceToHost, d.stream.get()));
+    CU(cudaStreamSynchronize(d.stream.get()));
     float ms = 0;
-    CU(cudaEventElapsedTime(&ms, d.ev[2], d.ev[3]));
+    CU(cudaEventElapsedTime(&ms, d.ev[2].get(), d.ev[3].get()));
     sk->st.ms_select += ms;
     // settle or re-stream each genome (see the argument at the top of this section)
     const uint64_t top = sk->top();
     for (uint32_t j = 0; j < n; j++) {
         SkGenome &g = sk->gen[ids[j]];
-        const MixState &r = d.h_slots.p[j].st;
+        const MixState &r = d.h_slots.get()[j].st;
         const uint64_t have = (uint64_t)r.count + (r.has_max ? 1 : 0);
         if (!r.overflow && (have >= sk->s || g.tau == top)) {
-            const uint64_t *h = d.h_out.p + d.h_out_off.p[j];
-            g.hashes.assign(h, h + d.h_n_out.p[j]);
+            const uint64_t *h = d.h_out.get() + d.h_out_off.get()[j];
+            g.hashes.assign(h, h + d.h_n_out.get()[j]);
             if (r.has_max && g.hashes.size() < sk->s) g.hashes.push_back(~0ull);   // hash 2^64-1 (kEmptyKey) is never stored in a set
             std::vector<uint64_t>().swap(g.seq);
             std::vector<uint32_t>().swap(g.inv);
@@ -2887,15 +2771,7 @@ HS_API int hs_sketcher_stats(const hs_sketcher *sk, hs_sketch_stats_t *stats)
     return HS_OK;
 }
 
-HS_API void hs_sketcher_free(hs_sketcher *sk)
-{
-    if (!sk) return;
-    if (sk->dev.ready) {
-        cudaSetDevice(sk->device);
-        sk->dev.release();
-    }
-    delete sk;
-}
+HS_API void hs_sketcher_free(hs_sketcher *sk) { if (sk) delete sk; }
 
 HS_API int hs_sketch_packed_device(uint32_t k, uint32_t s_, uint32_t seed, const void *d_seq2, const void *d_inv,
                                    uint64_t n_bases, uint64_t *out_hashes, uint32_t *n_out)
@@ -2964,23 +2840,26 @@ HS_API int hs_lca_weighted(uint64_t n_q, const uint64_t *q_off, const int32_t *t
     if (n_tax && !names) return fail(HS_EINVAL, "null argument");
     for (uint64_t j = 0; j < n_a; j++)
         if (tax[j] >= 0 && (uint64_t)tax[j] >= n_tax) return fail(HS_EINVAL, "taxid row out of range");
-    DevBufs d;
+    // every array has at least one element: no kernel argument is a null pointer
+    const uint64_t na1 = std::max<uint64_t>(n_a, 1), nt1 = std::max<uint64_t>(n_tax, 1);
+    DevBuf<uint64_t> d_off;
+    DevBuf<int32_t> d_tax, s_tax;
+    DevBuf<double> d_w, s_w, s_nw, o_conf;
+    DevBuf<uint32_t> d_names, s_name, o_names, o_depth;
+    DevBuf<uint8_t> o_any;
+    CU(d_off.grow(n_q + 1));
+    CU(d_tax.grow(na1)); CU(d_w.grow(na1)); CU(d_names.grow(nt1 * kLcaRanks));
+    CU(s_tax.grow(na1)); CU(s_w.grow(na1)); CU(s_name.grow(na1)); CU(s_nw.grow(na1));
+    CU(o_names.grow(n_q * kLcaRanks)); CU(o_depth.grow(n_q)); CU(o_conf.grow(n_q)); CU(o_any.grow(n_q));
     LcaArgs a;
     memset(&a, 0, sizeof a);
-    uint64_t *d_off = nullptr;
-    int32_t *d_tax = nullptr;
-    double *d_w = nullptr;
-    uint32_t *d_names = nullptr;
-    CU(d.alloc(&d_off, (n_q + 1) * 8));
-    CU(d.alloc(&d_tax, n_a * 4)); CU(d.alloc(&d_w, n_a * 8)); CU(d.alloc(&d_names, n_tax * kLcaRanks * 4));
-    CU(d.alloc(&a.s_tax, n_a * 4)); CU(d.alloc(&a.s_w, n_a * 8)); CU(d.alloc(&a.s_name, n_a * 4)); CU(d.alloc(&a.s_nw, n_a * 8));
-    CU(d.alloc(&a.out_names, n_q * kLcaRanks * 4)); CU(d.alloc(&a.out_depth, n_q * 4));
-    CU(d.alloc(&a.out_conf, n_q * 8)); CU(d.alloc(&a.out_any, n_q));
-    CU(cudaMemcpy(d_off, q_off, (n_q + 1) * 8, cudaMemcpyHostToDevice));
-    if (n_a) { CU(cudaMemcpy(d_tax, tax, n_a * 4, cudaMemcpyHostToDevice)); CU(cudaMemcpy(d_w, w, n_a * 8, cudaMemcpyHostToDevice)); }
-    if (n_tax) CU(cudaMemcpy(d_names, names, n_tax * kLcaRanks * 4, cudaMemcpyHostToDevice));
+    a.s_tax = s_tax.get(); a.s_w = s_w.get(); a.s_name = s_name.get(); a.s_nw = s_nw.get();
+    a.out_names = o_names.get(); a.out_depth = o_depth.get(); a.out_conf = o_conf.get(); a.out_any = o_any.get();
+    CU(cudaMemcpy(d_off.get(), q_off, (n_q + 1) * 8, cudaMemcpyHostToDevice));
+    if (n_a) { CU(cudaMemcpy(d_tax.get(), tax, n_a * 4, cudaMemcpyHostToDevice)); CU(cudaMemcpy(d_w.get(), w, n_a * 8, cudaMemcpyHostToDevice)); }
+    if (n_tax) CU(cudaMemcpy(d_names.get(), names, n_tax * kLcaRanks * 4, cudaMemcpyHostToDevice));
     CU(cudaMemset(a.out_names, 0, n_q * kLcaRanks * 4));
-    a.n_q = n_q; a.q_off = d_off; a.tax = d_tax; a.w = d_w; a.names = d_names;
+    a.n_q = n_q; a.q_off = d_off.get(); a.tax = d_tax.get(); a.w = d_w.get(); a.names = d_names.get();
     CU(launch_weighted_lca(a, g_sm, 0));
     CU(cudaMemcpy(out_names, a.out_names, n_q * kLcaRanks * 4, cudaMemcpyDeviceToHost));
     CU(cudaMemcpy(out_depth, a.out_depth, n_q * 4, cudaMemcpyDeviceToHost));
