@@ -62,6 +62,17 @@ class SketchStats(C.Structure):
         return {f: getattr(self, f) for f, _ in self._fields_}
 
 
+class DistanceStats(C.Structure):
+    _fields_ = [("n_queries", C.c_uint64), ("n_refs", C.c_uint64), ("n_candidates", C.c_uint64),
+                ("n_lines", C.c_uint64), ("n_blocks", C.c_uint32), ("n_splits", C.c_uint32),
+                ("block_queries", C.c_uint32), ("result_cap", C.c_uint32),
+                ("ms_mark", C.c_float), ("ms_compact", C.c_float), ("ms_merge", C.c_float),
+                ("t_write_s", C.c_double), ("t_total_s", C.c_double)]
+
+    def asdict(self):
+        return {f: getattr(self, f) for f, _ in self._fields_}
+
+
 # name -> (restype, argtypes).  Must list every symbol include/hymet_screen.h declares
 # (tests/test_abi.py checks the header against this table and against the .so).
 SIGNATURES = {
@@ -130,6 +141,14 @@ SIGNATURES = {
     "hs_sketch_packed_device": (C.c_int, [C.c_uint32, C.c_uint32, C.c_uint32, C.c_void_p, C.c_void_p, C.c_uint64,
                                           u64p, u32p]),
     "hs_pack_codes_device": (C.c_int, [C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "hs_distance_new": (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p)]),
+    "hs_distance_add_msh": (C.c_int, [C.c_void_p, C.c_void_p]),
+    "hs_distance_add_sketch": (C.c_int, [C.c_void_p, C.c_char_p, C.c_char_p, C.c_uint64, C.c_uint32, u64p, C.c_uint64]),
+    "hs_distance_run": (C.c_int, [C.c_void_p, C.c_int, C.c_double, C.c_double, C.c_int, C.c_int, C.c_int]),
+    "hs_distance_run_rows": (C.c_int, [C.c_void_p, C.c_double, u64p]),
+    "hs_distance_rows_copy": (C.c_int, [C.c_void_p, C.c_uint64, u32p, u32p, u32p, u32p, f64p]),
+    "hs_distance_stats": (C.c_int, [C.c_void_p, C.POINTER(DistanceStats)]),
+    "hs_distance_free": (None, [C.c_void_p]),
     "hs_lca_weighted": (C.c_int, [C.c_uint64, u64p, C.POINTER(C.c_int32), f64p, C.c_uint64, u32p, u32p, u32p, f64p, u8p]),
 }
 

@@ -8,8 +8,8 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libhymet_screen.so")
-SOURCES = ["abi.cu", "screen_kernels.cu", "lca_kernels.cu", "msh_capnp.cpp", "fasta_pack.cpp"]
-HEADERS = ["kmer_core.cuh", "cuda_owned.h", "screen_kernels.h", "lca_kernels.h", "msh_capnp.h", "fasta_pack.h",
+SOURCES = ["abi.cu", "screen_kernels.cu", "distance_kernels.cu", "lca_kernels.cu", "msh_capnp.cpp", "fasta_pack.cpp"]
+HEADERS = ["kmer_core.cuh", "table_device.cuh", "cuda_owned.h", "screen_kernels.h", "distance_kernels.h", "lca_kernels.h", "msh_capnp.h", "fasta_pack.h",
            os.path.join("..", "..", "include", "hymet_screen.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC,-fvisibility=hidden,-pthread", "--shared", "-cudart", "shared"]

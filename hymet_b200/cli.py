@@ -275,12 +275,8 @@ def sketch_main(args: List[str], stdout=None) -> int:
     except hs.HsError as e:
         _err(e.msg)
         return 1
-    comments = []
-    for g in sketches:
-        first = g.header.decode("utf-8", "replace").strip()
-        if g.n_records > 1:  # Mash's comment convention for multi-record genomes
-            first = "[%d seqs] %s [...]" % (g.n_records, first)
-        comments.append(first)
+    from .distance import sketch_comment
+    comments = [sketch_comment(g.header, g.n_records) for g in sketches]
     offsets = np.concatenate([[0], np.cumsum([len(g.hashes) for g in sketches])]).astype(np.uint64)
     db = mshfmt.SketchDB(k=k, s=s, seed=seed, names=list(paths), comments=comments,
                          lengths=np.array([g.length for g in sketches], np.uint64), offsets=offsets,
@@ -290,6 +286,147 @@ def sketch_main(args: List[str], stdout=None) -> int:
         out += ".msh"
     sys.stderr.write("Writing to %s...\n" % out)
     mshfmt.write_msh(out, db)
+    return 0
+
+
+DIST_USAGE = """
+Usage:
+
+  mash dist [options] <reference>.msh <query> [<query>] ...
+
+Description:
+
+  Estimate the distance of each query sequence to each reference sketch.  The
+  reference is one sketch file (.msh); queries are sketch files (.msh) or
+  FASTA/FASTQ files, gzipped or not, which are sketched with the reference's
+  k-mer size, sketch size and seed (one sketch per file).  The output fields are
+  [reference-ID, query-ID, distance, p-value, shared-hashes].  Computed on the
+  GPU, exactly as Mash 2.3 computes it.
+
+Options:
+
+  -h          Help
+  -p <int>    Host threads sketching sequence queries and formatting output [1]
+  -l          List input. Each query is a file that lists one input path per
+              line (empty lines are ignored).
+  -t          Table output (one row per query, distances only).
+  -C          Show comments for sequences (name:comment).
+  -v <num>    Maximum p-value to report. (0-1) [1.0]
+  -d <num>    Maximum distance to report. (0-1) [1.0]
+"""
+
+# sketching options of `mash dist`: Mash refuses them when the reference is a sketch (its parameters win)
+_DIST_SKETCH_OPTS = {"-k", "-s", "-S", "-w", "-a", "-z", "-n", "-Z", "-r", "-b", "-c", "-m", "-g", "-i"}
+_DIST_VALUE_OPTS = {"-p", "-v", "-d", "-k", "-s", "-S", "-w", "-z", "-b", "-c", "-m", "-g"}
+
+
+def _dist_first_positional(args: List[str]) -> Optional[str]:
+    i = 0
+    while i < len(args):
+        a = args[i]
+        if a.startswith("-") and len(a) > 1:
+            i += 2 if a in _DIST_VALUE_OPTS else 1
+            continue
+        return a
+    return None
+
+
+def distance_main(args: List[str], stdout=None, stderr=None) -> int:
+    """`mash dist` against a reference sketch file (DESIGN.md §5 "mash dist"): exact Mash 2.3 distances on the GPU."""
+    stdout = stdout or sys.stdout
+    stderr = stderr or sys.stderr
+    _e = lambda msg: _err(msg, stderr)
+    threads, lists, table, comments, pmax, dmax = 1, False, False, False, 1.0, 1.0
+    pos: List[str] = []
+    i = 0
+    try:
+        while i < len(args):
+            a = args[i]
+            if a == "-h":
+                stdout.write(DIST_USAGE)
+                return 0
+            if a == "-l":
+                lists = True
+            elif a == "-t":
+                table = True
+            elif a == "-C":
+                comments = True
+            elif a in ("-p", "-v", "-d"):
+                if i + 1 >= len(args):
+                    _e("-%s requires an argument" % a[1])
+                    return 1
+                v = args[i + 1]
+                i += 1
+                if a == "-p":
+                    threads = int(v)
+                elif a == "-v":
+                    pmax = float(v)
+                else:
+                    dmax = float(v)
+            elif a in _DIST_SKETCH_OPTS:
+                _e("Sketching option %s cannot be used when the reference is a sketch (.msh): its parameters are used" % a)
+                return 1
+            elif a.startswith("-") and a != "-":
+                _e("Unrecognized option: %s" % a)
+                return 1
+            else:
+                pos.append(a)
+            i += 1
+    except ValueError:
+        _e("malformed numeric option value")
+        return 1
+    if len(pos) < 2:
+        stdout.write(DIST_USAGE)
+        return 0
+    if threads < 1 or not (0.0 <= pmax <= 1.0) or not (0.0 <= dmax <= 1.0):
+        _e("option value out of range")
+        return 1
+    ref_path, queries = pos[0], pos[1:]
+    if not ref_path.endswith(".msh"):
+        _e("%s does not look like a sketch (.msh)" % ref_path)
+        return 1
+    if lists:
+        listed: List[str] = []
+        for lf in queries:
+            try:
+                with open(lf, "rb") as fh:
+                    listed += [os.fsdecode(ln) for ln in fh.read().split(b"\n") if ln]
+            except OSError:
+                _e("could not open %s for reading." % lf)
+                return 1
+        if not listed:
+            _e("no input files listed in %s" % " ".join(queries))
+            return 1
+        queries = listed
+    for p in [ref_path] + queries:
+        if not os.path.isfile(p):
+            _e("could not open %s for reading." % p)
+            return 1
+
+    from . import distance as dist
+    from ._abi import HsError
+    try:
+        ref = dist.HostMsh(ref_path)
+        for p in queries:                      # every query sketch file is checked before the GPU is touched
+            if dist.is_msh(p):
+                m = dist.HostMsh(p)
+                why = dist.mismatch(ref.header, m.header)
+                m.close()
+                if why:
+                    _e("%s: %s" % (p, why))
+                    return 1
+        d = dist.Distance(ref, int(os.environ.get("HYMET_SCREEN_DEVICE", "0")))
+        try:
+            dist.add_queries(d, queries, threads, int(os.environ.get("HYMET_SCREEN_DEVICE", "0")),
+                             warn=lambda msg: stderr.write("WARNING: %s\n" % msg))
+            stdout.flush()
+            d.run(stdout.fileno(), dmax, pmax, table, comments, threads)
+        finally:
+            d.close()
+            ref.close()
+    except HsError as e:
+        _e(e.msg)
+        return 1
     return 0
 
 
@@ -319,13 +456,18 @@ def _via_server(args: List[str]) -> Optional[int]:
 def main(argv: Optional[List[str]] = None) -> int:
     argv = sys.argv[1:] if argv is None else argv
     if not argv or argv[0] in ("-h", "--help", "help"):
-        sys.stdout.write("mash (hymet-screen-b200): commands `screen` and `sketch` are provided.\n" + USAGE)
+        sys.stdout.write("mash (hymet-screen-b200): commands `screen`, `sketch` and `dist` (against a .msh reference) "
+                         "are provided.\n" + USAGE)
         return 0
     if argv[0] == "--version":
         sys.stdout.write("2.3-hymet-screen-b200\n")
         return 0
     if argv[0] == "sketch":
         return sketch_main(argv[1:])
+    if argv[0] == "dist":
+        first = _dist_first_positional(argv[1:])
+        if (first is None and "-h" in argv[1:]) or (first is not None and first.endswith(".msh")):
+            return distance_main(argv[1:])
     if argv[0] == "screen" and os.environ.get("HYMET_SCREEN_SERVER", "0") not in ("", "0"):
         rc = _via_server(argv[1:])
         if rc is not None:

@@ -16,6 +16,7 @@
 #include <sys/stat.h>
 #include <unistd.h>
 #include <zlib.h>
+#include <errno.h>
 
 #include <algorithm>
 #include <atomic>
@@ -30,6 +31,7 @@
 
 #include "../../include/hymet_screen.h"
 #include "cuda_owned.h"
+#include "distance_kernels.h"
 #include "fasta_pack.h"
 #include "kmer_core.cuh"
 #include "lca_kernels.h"
@@ -2866,4 +2868,455 @@ HS_API int hs_lca_weighted(uint64_t n_q, const uint64_t *q_off, const int32_t *t
     CU(cudaMemcpy(out_conf, a.out_conf, n_q * 8, cudaMemcpyDeviceToHost));
     CU(cudaMemcpy(out_any, a.out_any, n_q, cudaMemcpyDeviceToHost));
     return HS_OK;
+}
+
+// =============================================================================
+// `mash dist` (DESIGN.md §5 "mash dist"): one reference .msh against query sketches, exactly
+// =============================================================================
+namespace {
+
+constexpr uint64_t kDistBlockBytes = 48ull << 20;   // bitmap rows + query hashes of one block: stays in L2 (126 MB)
+constexpr uint32_t kDistMaxBlock = 1u << 16;        // queries per block at most
+constexpr uint32_t kDistResultRows = 1u << 19;      // candidate rows one block holds (at least one query's worth)
+
+struct DistQuery {
+    std::string name, comment;
+    uint64_t length = 0;
+    uint32_t sp = 0;        // min(reference file's s, this query file's s)
+};
+
+struct DistSlot {
+    DevBuf<DistRow> d_rows;
+    PinnedBuf<DistRow> h_rows;
+    PinnedBuf<unsigned long long> h_total;
+    Event ev_t0, ev_t1, ev_t2, ev_done, ev_copied;   // t0 mark t1 count + scan + compact t2 merge done
+    uint32_t q0 = 0, n_q = 0;
+};
+
+}  // namespace
+
+struct hs_distance {
+    int device = 0, sm = 0;
+    std::unique_ptr<hs_db, void (*)(hs_db *)> db{nullptr, hs_db_free};
+    DevBuf<uint64_t> d_ref_hashes;           // the references' sorted hashes, flat (hs_db keeps only its table)
+    std::vector<uint64_t> ref_sizes;
+    uint64_t ref_scale = 0;
+    std::vector<DistQuery> q;
+    std::vector<uint64_t> q_off{0}, q_hashes;
+    bool uploaded = false;
+    DevBuf<uint64_t> d_q_off, d_q_hashes, d_q_len;
+    DevBuf<uint32_t> d_q_sp, d_bitmap;
+    DevBuf<unsigned long long> d_row_start;
+    DistSlot slot[2];
+    Stream st, st_copy;
+    std::vector<DistRow> rows;               // hs_distance_run_rows
+    hs_distance_stats_t stats{};
+};
+
+namespace {
+
+int dist_add(hs_distance *d, const char *name, const char *comment, uint64_t length, uint32_t s_q, const uint64_t *h, uint64_t n)
+{
+    for (uint64_t i = 1; i < n; i++)
+        if (h[i] <= h[i - 1]) return fail(HS_EFORMAT, "sketch hashes are not strictly ascending");
+    if (d->q.size() >= 0xFFFFFFF0ull) return fail(HS_EUNSUPPORTED, "more than 2^32 query sketches");
+    DistQuery x;
+    x.name = name ? name : "";
+    x.comment = comment ? comment : "";
+    x.length = length;
+    x.sp = std::min(d->db->s, s_q);
+    d->q.push_back(std::move(x));
+    d->q_hashes.insert(d->q_hashes.end(), h, h + n);
+    d->q_off.push_back(d->q_hashes.size());
+    d->uploaded = false;
+    return HS_OK;
+}
+
+int dist_upload(hs_distance *d)
+{
+    if (d->uploaded) return HS_OK;
+    const uint64_t nq = d->q.size();
+    std::vector<uint64_t> len(std::max<uint64_t>(nq, 1), 0);
+    std::vector<uint32_t> sp(std::max<uint64_t>(nq, 1), 0);
+    for (uint64_t i = 0; i < nq; i++) { len[i] = d->q[i].length; sp[i] = d->q[i].sp; }
+    d->d_q_off.reset(); d->d_q_hashes.reset(); d->d_q_len.reset(); d->d_q_sp.reset();
+    CU(d->d_q_off.grow(nq + 1));
+    CU(d->d_q_hashes.grow(std::max<uint64_t>(d->q_hashes.size(), 1)));
+    CU(d->d_q_len.grow(len.size()));
+    CU(d->d_q_sp.grow(sp.size()));
+    CU(cudaMemcpy(d->d_q_off.get(), d->q_off.data(), (nq + 1) * 8, cudaMemcpyHostToDevice));
+    if (!d->q_hashes.empty())
+        CU(cudaMemcpy(d->d_q_hashes.get(), d->q_hashes.data(), d->q_hashes.size() * 8, cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(d->d_q_len.get(), len.data(), len.size() * 8, cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(d->d_q_sp.get(), sp.data(), sp.size() * 4, cudaMemcpyHostToDevice));
+    d->uploaded = true;
+    return HS_OK;
+}
+
+// D2 from the exact integers, with the double expression of Mash's CommandDistance
+double dist_value(uint64_t common, uint64_t denom, uint32_t k)
+{
+    if (common == denom) return 0.0;
+    if (common == 0) return 1.0;
+    const double jaccard = double(common) / denom;
+    const double distance = -log(2 * jaccard / (1. + jaccard)) / k;
+    return distance > 1 ? 1 : distance;
+}
+
+// The block pipeline.  Blocks of queries go through the kernels on `st`; while the device computes
+// block b + 1, the candidate rows of block b are copied (on `st_copy`) into that slot's pinned buffer
+// and handed to `sink` on the calling thread, in query order.  A block whose candidates overflow the
+// result buffer is redone as blocks half its size, and so are the blocks after it (the one already in
+// flight is dropped).
+template <class Sink>
+int dist_pipeline(hs_distance *d, double max_d, Sink &&sink)
+{
+    ON_DEVICE(d->device);
+    int rc = dist_upload(d);
+    if (rc) return rc;
+    const hs_db *db = d->db.get();
+    const uint64_t nq = d->q.size(), nr = db->n_refs;
+    const uint32_t words = (uint32_t)((nr + 31) / 32);
+    const double avg_q = nq ? (double)d->q_hashes.size() / (double)nq : 0.0;
+    const double per_q = (double)words * 4 + avg_q * 8 + 8;
+    uint64_t block = (uint64_t)((double)kDistBlockBytes / per_q);
+    block = std::max<uint64_t>(1, std::min<uint64_t>({block, (uint64_t)kDistMaxBlock, std::max<uint64_t>(nq, 1)}));
+    const uint32_t cap = (uint32_t)std::max<uint64_t>(kDistResultRows, nr);
+    d->stats.block_queries = (uint32_t)block;
+    d->stats.result_cap = cap;
+    if (!nq) return HS_OK;
+
+    if (!d->st.get()) { CU(d->st.create()); CU(d->st_copy.create()); }
+    if (d->d_bitmap.cap() < block * words) {
+        CU(d->d_bitmap.grow(std::max<uint64_t>(block * words, 1)));
+        CU(cudaMemset(d->d_bitmap.get(), 0, d->d_bitmap.cap() * 4));   // k_dist_compact leaves it zero again
+    }
+    CU(d->d_row_start.grow(block + 1));
+    for (DistSlot &s : d->slot) {
+        CU(s.d_rows.grow(cap));
+        CU(s.h_total.grow(1));
+        if (!s.ev_done.get()) {
+            CU(s.ev_t0.create()); CU(s.ev_t1.create()); CU(s.ev_t2.create()); CU(s.ev_done.create());
+            CU(s.ev_copied.create(cudaEventDisableTiming));
+            CU(cudaEventRecord(s.ev_copied.get(), d->st_copy.get()));
+        }
+    }
+    const cudaStream_t st = d->st.get(), stc = d->st_copy.get();
+    DistArgs a;
+    memset(&a, 0, sizeof a);
+    a.tab = db->view(); a.next = db->d_next.get();
+    a.ref_off = db->d_offsets.get(); a.ref_hashes = d->d_ref_hashes.get(); a.ref_len = db->d_lengths.get();
+    a.n_refs = (uint32_t)nr; a.ref_scale = d->ref_scale;
+    a.q_off = d->d_q_off.get(); a.q_hashes = d->d_q_hashes.get(); a.q_len = d->d_q_len.get(); a.q_sp = d->d_q_sp.get();
+    a.bitmap = d->d_bitmap.get(); a.words = words; a.row_start = d->d_row_start.get();
+    a.cap = cap; a.k = db->k; a.max_d = max_d;
+
+    uint64_t q_next = 0, blk = block;   // next block: [q_next, q_next + blk)
+    int prev = -1, next_slot = 0;
+    while (q_next < nq || prev >= 0) {
+        int cur = -1;
+        if (q_next < nq) {
+            DistSlot &s = d->slot[next_slot];
+            s.q0 = (uint32_t)q_next; s.n_q = (uint32_t)std::min<uint64_t>(blk, nq - q_next);
+            q_next += s.n_q;
+            a.q0 = s.q0; a.n_q = s.n_q; a.rows = s.d_rows.get();
+            CU(cudaStreamWaitEvent(st, s.ev_copied.get(), 0));   // this slot's previous rows are home
+            CU(cudaEventRecord(s.ev_t0.get(), st));
+            CU(launch_dist_candidates(a, d->sm, s.ev_t1.get(), st));
+            CU(cudaEventRecord(s.ev_t2.get(), st));
+            CU(launch_dist_merge(a, d->sm, st));
+            CU(cudaMemcpyAsync(s.h_total.get(), d->d_row_start.get() + s.n_q, sizeof(unsigned long long),
+                               cudaMemcpyDeviceToHost, st));
+            CU(cudaEventRecord(s.ev_done.get(), st));
+            d->stats.n_blocks++;
+            cur = next_slot;
+            next_slot ^= 1;
+        }
+        if (prev >= 0) {
+            DistSlot &s = d->slot[prev];
+            CU(cudaEventSynchronize(s.ev_done.get()));
+            float ms[3] = {0, 0, 0};
+            CU(cudaEventElapsedTime(ms, s.ev_t0.get(), s.ev_t1.get()));
+            CU(cudaEventElapsedTime(ms + 1, s.ev_t1.get(), s.ev_t2.get()));
+            CU(cudaEventElapsedTime(ms + 2, s.ev_t2.get(), s.ev_done.get()));
+            d->stats.ms_mark += ms[0]; d->stats.ms_compact += ms[1]; d->stats.ms_merge += ms[2];
+            const unsigned long long n = *s.h_total.get();
+            if (n > cap) {
+                // redo from this block on (the one in flight behind it is dropped) with blocks half its size;
+                // a block of one query always fits (cap >= references)
+                CU(cudaStreamSynchronize(st));
+                q_next = s.q0;
+                blk = std::max<uint64_t>(1, s.n_q / 2);
+                d->stats.n_splits++;
+                prev = -1;
+                next_slot = 0;
+                continue;
+            }
+            uint64_t want = 1;
+            while (want < n) want <<= 1;
+            CU(s.h_rows.grow(want));
+            CU(cudaStreamWaitEvent(stc, s.ev_done.get(), 0));
+            if (n) CU(cudaMemcpyAsync(s.h_rows.get(), s.d_rows.get(), n * sizeof(DistRow), cudaMemcpyDeviceToHost, stc));
+            CU(cudaEventRecord(s.ev_copied.get(), stc));
+            CU(cudaEventSynchronize(s.ev_copied.get()));
+            d->stats.n_candidates += n;
+            if ((rc = sink(s.q0, s.n_q, s.h_rows.get(), (uint64_t)n))) return rc;
+        }
+        prev = cur;
+    }
+    return HS_OK;
+}
+
+void put_g(std::string &o, double x)
+{
+    char b[32];
+    o.append(b, (size_t)snprintf(b, sizeof b, "%g", x));
+}
+void put_u(std::string &o, uint64_t x)
+{
+    char b[24];
+    o.append(b, (size_t)snprintf(b, sizeof b, "%llu", (unsigned long long)x));
+}
+
+int write_all(int fd, const std::string &s)
+{
+    size_t off = 0;
+    while (off < s.size()) {
+        const ssize_t w = ::write(fd, s.data() + off, s.size() - off);
+        if (w < 0) {
+            if (errno == EINTR) continue;
+            return fail(HS_EIO, std::string("writing the output: ") + strerror(errno));
+        }
+        off += (size_t)w;
+    }
+    return HS_OK;
+}
+
+struct DistFormat {
+    const hs_distance *d;
+    double max_d, max_p;
+    bool table, comments;
+    std::vector<std::string> ref_names;      // name or name:comment
+    bool implicit_all;                        // non-candidate pairs pass D4 (-d >= 1 and -v >= 1)
+
+    std::string qname(uint64_t q) const
+    {
+        const DistQuery &x = d->q[q];
+        return comments ? x.name + ":" + x.comment : x.name;
+    }
+    // the lines of query q; its candidate rows are [r0, r1) in reference order.  Returns lines written.
+    uint64_t query(uint64_t q, const DistRow *r0, const DistRow *r1, std::string &o) const
+    {
+        const hs_db *db = d->db.get();
+        const uint32_t k = db->k;
+        const uint64_t nr = db->n_refs, qsize = d->q_off[q + 1] - d->q_off[q];
+        const uint32_t sp = d->q[q].sp;
+        const std::string qn = qname(q);
+        const bool empties = qsize == 0 && max_p >= 1;   // pairs of two empty sketches: distance 0, p-value 1
+        auto line = [&](uint64_t r, uint64_t common, uint64_t denom, double dist, double p) {
+            o += ref_names[r]; o += '\t'; o += qn; o += '\t';
+            put_g(o, dist); o += '\t'; put_g(o, p); o += '\t';
+            put_u(o, common); o += '/'; put_u(o, denom); o += '\n';
+        };
+        if (table) {
+            o += qn;
+            const DistRow *c = r0;
+            for (uint64_t r = 0; r < nr; r++) {
+                o += '\t';
+                uint64_t common = 0, denom;
+                double p = 1.0;
+                if (c < r1 && c->r == r) { common = c->common; denom = c->denom; p = c->p; c++; }
+                else denom = std::min<uint64_t>(sp, d->ref_sizes[r] + qsize);
+                const double dist = dist_value(common, denom, k);
+                if (dist > max_d || p > max_p) continue;
+                put_g(o, dist);
+            }
+            o += '\n';
+            return 1;
+        }
+        uint64_t n = 0;
+        if (implicit_all || empties) {
+            const DistRow *c = r0;
+            for (uint64_t r = 0; r < nr; r++) {
+                if (c < r1 && c->r == r) {
+                    const double dist = dist_value(c->common, c->denom, k);
+                    if (!(dist > max_d) && !(c->p > max_p)) { line(r, c->common, c->denom, dist, c->p); n++; }
+                    c++;
+                    continue;
+                }
+                const uint64_t denom = std::min<uint64_t>(sp, d->ref_sizes[r] + qsize);
+                if (denom == 0 ? max_p >= 1 : implicit_all) { line(r, 0, denom, denom == 0 ? 0.0 : 1.0, 1.0); n++; }
+            }
+            return n;
+        }
+        for (const DistRow *c = r0; c < r1; c++) {
+            const double dist = dist_value(c->common, c->denom, k);
+            if (dist > max_d || c->p > max_p) continue;
+            line(c->r, c->common, c->denom, dist, c->p);
+            n++;
+        }
+        return n;
+    }
+};
+
+}  // namespace
+
+HS_API int hs_distance_new(const hs_msh *ref, hs_distance **out)
+{
+    if (!ref || !out) return fail(HS_EINVAL, "null argument");
+    NEED_DEVICE();
+    std::unique_ptr<hs_distance> d(new hs_distance());
+    d->device = g_device; d->sm = g_sm;
+    hs_db *db = nullptr;
+    int rc = hs_db_from_msh(ref, &db);
+    if (rc) return rc;
+    d->db.reset(db);
+    const uint64_t N = db->n_refs, E = db->n_entries;
+    d->ref_sizes.resize(N);
+    for (uint64_t i = 0; i < N; i++) d->ref_sizes[i] = db->offsets[i + 1] - db->offsets[i];
+    d->ref_scale = (E && N <= E) ? (uint64_t)((((unsigned __int128)N) << 64) / ((unsigned __int128)E + 1)) : 0;
+    CU(d->d_ref_hashes.grow(std::max<uint64_t>(E, 1)));
+    if (E) CU(cudaMemcpy(d->d_ref_hashes.get(), ref->d.hashes.data(), E * 8, cudaMemcpyHostToDevice));
+    d->stats.n_refs = N;
+    *out = d.release();
+    return HS_OK;
+}
+
+HS_API int hs_distance_add_msh(hs_distance *d, const hs_msh *m)
+{
+    if (!d || !m) return fail(HS_EINVAL, "null argument");
+    const hs_db *db = d->db.get();
+    if (m->d.k != db->k || m->d.seed != db->seed || m->d.use64 != db->use64)
+        return fail(HS_EUNSUPPORTED, "query sketch file differs from the reference in k-mer size (" + std::to_string(m->d.k) +
+                                         " vs " + std::to_string(db->k) + "), seed (" + std::to_string(m->d.seed) + " vs " +
+                                         std::to_string(db->seed) + ") or hash width");
+    const uint64_t n = m->d.offsets.size() - 1;
+    for (uint64_t i = 0; i < n; i++) {
+        const uint64_t b = m->d.offsets[i], e = m->d.offsets[i + 1];
+        const int rc = dist_add(d, m->d.names[i].c_str(), m->d.comments[i].c_str(), m->d.lengths[i], m->d.s,
+                                m->d.hashes.data() + b, e - b);
+        if (rc) return rc;
+    }
+    return HS_OK;
+}
+
+HS_API int hs_distance_add_sketch(hs_distance *d, const char *name, const char *comment, uint64_t length, uint32_t s,
+                                  const uint64_t *hashes, uint64_t n)
+{
+    if (!d || (!hashes && n)) return fail(HS_EINVAL, "null argument");
+    if (s == 0) return fail(HS_EINVAL, "sketch size must be positive");
+    return dist_add(d, name, comment, length, s, hashes, n);
+}
+
+HS_API int hs_distance_run(hs_distance *d, int fd, double max_distance, double max_pvalue, int table, int comments,
+                           int host_threads)
+{
+    if (!d) return fail(HS_EINVAL, "null handle");
+    if (!(max_distance >= 0 && max_distance <= 1) || !(max_pvalue >= 0 && max_pvalue <= 1))
+        return fail(HS_EINVAL, "maximum distance and p-value must be in [0, 1]");
+    const double t0 = now_s();
+    const hs_db *db = d->db.get();
+    DistFormat f;
+    f.d = d; f.max_d = max_distance; f.max_p = max_pvalue; f.table = table != 0; f.comments = comments != 0;
+    f.implicit_all = max_distance >= 1 && max_pvalue >= 1;
+    f.ref_names.resize(db->n_refs);
+    for (uint64_t r = 0; r < db->n_refs; r++)
+        f.ref_names[r] = f.comments ? db->names[r] + ":" + db->comments[r] : db->names[r];
+    const int threads = std::max(1, host_threads);
+    double t_write = 0;
+    int rc = HS_OK;
+    if (table) {
+        std::string h = "#query";
+        for (const std::string &n : f.ref_names) { h += '\t'; h += n; }
+        h += '\n';
+        if ((rc = write_all(fd, h))) return rc;
+    }
+    std::vector<std::string> out(threads);
+    std::vector<uint64_t> lines(threads);
+    rc = dist_pipeline(d, max_distance, [&](uint32_t q0, uint32_t n_q, const DistRow *rows, uint64_t n) -> int {
+        const double tw = now_s();
+        // query q's rows start at the first row whose q is >= q
+        auto first_of = [&](uint64_t q) { return std::lower_bound(rows, rows + n, q, [](const DistRow &x, uint64_t v) { return x.q < v; }); };
+        const uint32_t nt = (uint32_t)std::min<uint64_t>((uint64_t)threads, n_q);
+        auto part = [&](uint32_t t) {
+            const uint64_t qa = q0 + (uint64_t)n_q * t / nt, qb = q0 + (uint64_t)n_q * (t + 1) / nt;
+            std::string &o = out[t];
+            o.clear();
+            lines[t] = 0;
+            const DistRow *c = first_of(qa);
+            for (uint64_t q = qa; q < qb; q++) {
+                const DistRow *e = first_of(q + 1);
+                lines[t] += f.query(q, c, e, o);
+                c = e;
+            }
+        };
+        if (nt <= 1) part(0);
+        else {
+            std::vector<std::thread> th;
+            for (uint32_t t = 1; t < nt; t++) th.emplace_back(part, t);
+            part(0);
+            for (auto &x : th) x.join();
+        }
+        for (uint32_t t = 0; t < nt; t++) {
+            const int r = write_all(fd, out[t]);
+            if (r) return r;
+            d->stats.n_lines += lines[t];
+        }
+        t_write += now_s() - tw;
+        return HS_OK;
+    });
+    d->stats.t_write_s += t_write;
+    d->stats.t_total_s += now_s() - t0;
+    return rc;
+}
+
+HS_API int hs_distance_run_rows(hs_distance *d, double max_distance, uint64_t *n_rows)
+{
+    if (!d || !n_rows) return fail(HS_EINVAL, "null argument");
+    if (!(max_distance >= 0 && max_distance <= 1)) return fail(HS_EINVAL, "maximum distance must be in [0, 1]");
+    const double t0 = now_s();
+    d->rows.clear();
+    const int rc = dist_pipeline(d, max_distance, [&](uint32_t, uint32_t, const DistRow *rows, uint64_t n) -> int {
+        d->rows.insert(d->rows.end(), rows, rows + n);
+        return HS_OK;
+    });
+    d->stats.t_total_s += now_s() - t0;
+    *n_rows = d->rows.size();
+    return rc;
+}
+
+HS_API int hs_distance_rows_copy(const hs_distance *d, uint64_t cap, uint32_t *q, uint32_t *r, uint32_t *common,
+                                 uint32_t *denom, double *pvalue)
+{
+    if (!d) return fail(HS_EINVAL, "null handle");
+    const uint64_t n = std::min<uint64_t>(cap, d->rows.size());
+    for (uint64_t i = 0; i < n; i++) {
+        const DistRow &x = d->rows[i];
+        if (q) q[i] = x.q;
+        if (r) r[i] = x.r;
+        if (common) common[i] = x.common;
+        if (denom) denom[i] = x.denom;
+        if (pvalue) pvalue[i] = x.p;
+    }
+    return HS_OK;
+}
+
+HS_API int hs_distance_stats(const hs_distance *d, hs_distance_stats_t *stats)
+{
+    if (!d || !stats) return fail(HS_EINVAL, "null argument");
+    *stats = d->stats;
+    stats->n_queries = d->q.size();
+    return HS_OK;
+}
+
+HS_API void hs_distance_free(hs_distance *d)
+{
+    if (!d) return;
+    int cur = -1;
+    const bool other = cudaGetDevice(&cur) == cudaSuccess && cur != d->device;
+    if (other) cudaSetDevice(d->device);
+    if (d->st.get()) cudaStreamSynchronize(d->st.get());
+    if (d->st_copy.get()) cudaStreamSynchronize(d->st_copy.get());
+    if (other) cudaSetDevice(cur);
+    delete d;
 }

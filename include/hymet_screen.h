@@ -316,6 +316,51 @@ int hs_sketch_packed_device(uint32_t k, uint32_t s, uint32_t seed, const void *d
  * invalid).  Runs on `cuda_stream` (NULL = default stream) and returns without syncing. */
 int hs_pack_codes_device(const void *d_codes, uint64_t n, void *d_seq2, void *d_inv, void *cuda_stream);
 
+/* ---- `mash dist`: one reference sketch file against query sketches (DESIGN.md §5 "mash dist") ------------------
+ * Every (query, reference) pair gets Mash 2.3's exact (common, denom) -- its merge of the two sorted
+ * sketches truncated at s_p, the smaller of the two files' sketch sizes -- its distance and its p-value.
+ * On the device: the pairs that share a hash (found through the reference key table, one query block at
+ * a time), the merge and the p-value.  On the host: the distance and both filters, from the exact
+ * integers with libm, and the TSV.  Pairs that share no hash are written without device work. */
+typedef struct hs_distance hs_distance;
+typedef struct {
+    uint64_t n_queries, n_refs;
+    uint64_t n_candidates;   /* pairs that share a hash (computed blocks, redone ones excluded) */
+    uint64_t n_lines;        /* lines written (-t: query rows) */
+    uint32_t n_blocks;       /* query blocks sent to the device, redone ones included */
+    uint32_t n_splits;       /* blocks whose candidates overflowed the result buffer: redone at half the size */
+    uint32_t block_queries;  /* queries per block (chosen so that the block's bitmap and sketches stay in L2) */
+    uint32_t result_cap;     /* candidate pairs one block's result buffer holds */
+    float ms_mark;           /* device time: probes + chain walks marking candidate pairs (CUDA events) */
+    float ms_compact;        /* device time: popcount, scan, compaction into (q, r) rows */
+    float ms_merge;          /* device time: truncated merges + p-values */
+    double t_write_s;        /* host seconds formatting and writing lines */
+    double t_total_s;        /* wall clock of the runs */
+} hs_distance_stats_t;
+
+/* The reference side: a key table over the sketches of `ref` on the bound device. */
+int hs_distance_new(const hs_msh *ref, hs_distance **out);
+/* Queue every sketch of one query file, in file order.  HS_EUNSUPPORTED if its k-mer size, seed or hash
+ * width differs from the reference's.  Its sketch size sets s_p for its pairs. */
+int hs_distance_add_msh(hs_distance *d, const hs_msh *m);
+/* Queue one sketch (a sketcher result): n ascending hashes, sketch size s of the file it stands for. */
+int hs_distance_add_sketch(hs_distance *d, const char *name, const char *comment, uint64_t length, uint32_t s,
+                           const uint64_t *hashes, uint64_t n);
+/* Write `mash dist` output for every queued query (queries outer, references inner) to fd.  Pairs with
+ * distance > max_distance or p-value > max_pvalue (both in [0, 1]) are left out; table = -t (one row
+ * per query, distances only), comments = -C (name:comment); host_threads format disjoint query ranges. */
+int hs_distance_run(hs_distance *d, int fd, double max_distance, double max_pvalue, int table, int comments,
+                    int host_threads);
+/* The same pipeline without output: keeps the candidate pairs (those that share a hash) in (query,
+ * reference) order; *n_rows = how many.  p-value < 0: not computed, the pair is farther than max_distance.
+ * hs_distance_rows_copy fills the caller's arrays (cap elements each, NULL to skip a column). */
+int hs_distance_run_rows(hs_distance *d, double max_distance, uint64_t *n_rows);
+int hs_distance_rows_copy(const hs_distance *d, uint64_t cap, uint32_t *q, uint32_t *r, uint32_t *common,
+                          uint32_t *denom, double *pvalue);
+/* Counters accumulated over the handle's runs. */
+int hs_distance_stats(const hs_distance *d, hs_distance_stats_t *stats);
+void hs_distance_free(hs_distance *d);
+
 /* ---- SURVEY.md 8f rank 4: the classifier's weighted-LCA vote ----------------------------------------
  * /root/reference/scripts/classification_cami.py:251-308 (_weighted_lca, _process_one) for n_q queries
  * at once, one GPU thread per query, bit-exact with the reference's double arithmetic (sums in dict
